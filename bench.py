@@ -2,6 +2,7 @@
 """bench.py — QPS & effective index GB/s of the 4b x 1b BBQ score+top-k path (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c3q1|c4|c5] [--impl reference]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic queries: validate + quantise the query batch (K4),
@@ -20,6 +21,8 @@ cpu_baseline   the CPU oracle (restatement of the reference's TypeScript path; "
 parity     the lists the TIMED configuration returned, checked against the oracle (re-score of the returned rows,
            and no row of a 1M-row sample may beat the k-th returned row)
 secondary  (N=1, default run only) the other BASELINE configs, each measured the same way in a few seconds
+--dump-outputs DIR   the top-k lists the timed path returned in its last step, as .npy files (inputs are seeded, so
+                     two builds run with the same arguments can be compared list for list; bench_outputs/ is ignored by git)
 --impl reference   times the CPU path as the main line (the TypeScript reference itself cannot run here:
                    no node / tsc / cargo in the image; see DESIGN.md)
 """
@@ -343,6 +346,23 @@ def _stage(rank, what):
         print(f"[bench r{rank} {time.time() % 1000:.1f}] {what}", file=sys.stderr, flush=True)
 
 
+DUMP_LIMIT = 64 << 20    # bytes --dump-outputs may write
+
+
+def dump_outputs(path, idx, sc):
+    """--dump-outputs: the top-k lists the timed path returned in its last step, as a caller receives them (global row
+    ids as float64, exact below 2**53; f32 scores), one row per query.  Above DUMP_LIMIT a fixed seeded sample of the
+    query rows is written; query_rows.npy names the rows either way."""
+    os.makedirs(path, exist_ok=True)
+    rows = np.arange(idx.shape[0])
+    per_row = idx.shape[1] * (8 + 4) + 8
+    if rows.size * per_row > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(0).choice(rows.size, DUMP_LIMIT // per_row, replace=False))
+    np.save(os.path.join(path, "query_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(path, "topk_indices.npy"), idx[rows].astype(np.float64))
+    np.save(os.path.join(path, "topk_scores.npy"), sc[rows].astype(np.float32))
+
+
 def measure(args, torch, dist, bbq, w, rank, world, local_rank, steps, warmup, flush, sample_clocks):
     """Builds this rank's shard of workload w and times it.  -> dict of raw measurements (every rank), or None."""
     n, dim, k, nq = w["n"], w["dim"], w["k"], w["nq"]
@@ -370,7 +390,13 @@ def measure(args, torch, dist, bbq, w, rank, world, local_rank, steps, warmup, f
     sampler = ClockSampler(local_rank) if (rank == 0 and sample_clocks) else None
     if sampler:
         sampler.start()
-    ms_total = tm.device(lambda: searcher.search_device(dq, k), steps, 0)
+    last = []
+
+    def step():
+        last[:] = searcher.search_device(dq, k)
+
+    ms_total = tm.device(step, steps, 0)
+    outputs = (last[0].cpu().numpy(), last[1].cpu().numpy())     # the last timed step's lists (its stream is synchronised)
     _stage(rank, "device-timed steps done")
     st = fmt.stats()
     launches = st["kernel_launches"] - l0
@@ -389,7 +415,7 @@ def measure(args, torch, dist, bbq, w, rank, world, local_rank, steps, warmup, f
                 "note": "same device-resident search, L2 not flushed between steps (index is L2-resident)"}
     return dict(fmt=fmt, shard=shard, searcher=searcher, hq=hq, st=st, launches=launches, ms_step=ms_total / steps,
                 e2e_ms_step=e2e_ms / steps, clocks=clocks, warm=warm, build_s=build_s, device_gen=device_gen,
-                rows_local=r1 - r0, r0=r0)
+                rows_local=r1 - r0, r0=r0, outputs=outputs)
 
 
 def roofline_of(w, m, world, steps, peaks, probe, workload_key):
@@ -519,6 +545,8 @@ def run_gpu(args, w, rank, world, local_rank):
             dist.barrier()
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *m["outputs"])
     peaks = load_peaks()
     st = m["st"]
     roofline, index_gbps = roofline_of(w, m, world, args.steps, peaks, probe, args.workload)
@@ -707,7 +735,7 @@ def main():
     ap.add_argument("--rows", type=int, default=0, help="override the corpus rows of the workload (experiments)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / parity legs")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary workloads of the default run")
-    ap.add_argument("--secondary-steps", type=int, default=10)
+    ap.add_argument("--secondary-steps", type=int, default=0, help="timed steps of each secondary workload (0 = --steps)")
     ap.add_argument("--parity-multi", action="store_true")
     ap.add_argument("--parity-queries", type=int, default=64, help="queries of the timed batch whose lists are verified")
     ap.add_argument("--cpu-budget", type=float, default=15.0, help="seconds of CPU work for cpu_baseline")
@@ -716,7 +744,12 @@ def main():
     ap.add_argument("--ref-rows", type=int, default=1_000_000, help="--impl reference: rows of the corpus sampled")
     ap.add_argument("--ref-queries-per-step", type=int, default=1, help="--impl reference: queries per thread and step")
     ap.add_argument("--ref-threads", type=int, default=0, help="--impl reference: host threads (0 = all cores)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the top-k lists of the last one as DIR/*.npy (GPU arm)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU arm computed: use it with --impl b200")
+    args.secondary_steps = args.secondary_steps or args.steps
     if os.environ.get("BBQ_BENCH_WATCHDOG"):   # diagnostics: dump every Python stack and exit if the run blocks this long
         import faulthandler
         faulthandler.dump_traceback_later(float(os.environ["BBQ_BENCH_WATCHDOG"]), exit=True)

@@ -19,7 +19,7 @@ Nothing of the reference is copied into the repository: the sources are read whe
 SHA-256 so that it is clear which text produced it.  `tests/test_golden_from_ts.py` compares the oracle with the
 fixtures bit for bit; `tests/test_tsinterp.py` tests the interpreter itself.
 
-    python tests/golden/from_ts/make_golden_with_interp.py [--reference /root/reference] [case ...]
+    python tests/golden/from_ts/make_golden_with_interp.py [--reference <reference checkout>] [case ...]
 """
 import argparse
 import hashlib
@@ -222,7 +222,7 @@ def run_errors(ref_root):
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("--reference", default="/root/reference")
+    ap.add_argument("--reference", default=os.environ.get("BBQ_REFERENCE_DIR"), required="BBQ_REFERENCE_DIR" not in os.environ)
     ap.add_argument("cases", nargs="*", default=list(CASES) + ["index_bits_2", "errors"])
     a = ap.parse_args()
     for nm in a.cases:

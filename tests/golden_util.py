@@ -6,6 +6,10 @@ import numpy as np
 from tests.fixtures import gaussian, sincos_dataset
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# A checkout of the reference project (leolee9086/better-binary-quantization), the source golden/from_ts was generated
+# from.  Only the tests that execute the reference's own files read it; they skip when BBQ_REFERENCE_DIR is not set.
+REFERENCE_DIR = os.environ.get("BBQ_REFERENCE_DIR", "")
+HAVE_REFERENCE = bool(REFERENCE_DIR) and os.path.isdir(os.path.join(REFERENCE_DIR, "src"))
 
 
 def golden_cases():

@@ -5,6 +5,8 @@ import os
 import re
 import subprocess
 
+from tests.golden_util import REFERENCE_DIR
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 NAPI = os.path.join(ROOT, "better-binary-quantization_b200", "bindings", "napi")
 TS = os.path.join(ROOT, "better-binary-quantization_b200", "bindings", "ts")
@@ -40,7 +42,7 @@ def test_typescript_class_uses_registered_addon_functions():
         assert name in ts, name      # src/types.ts:32-49
 
 
-REFERENCE_CLASS = "/root/reference/src/binaryQuantizationFormat.ts"
+REFERENCE_CLASS = os.path.join(REFERENCE_DIR, "src", "binaryQuantizationFormat.ts") if REFERENCE_DIR else ""
 # the ten public members of the reference class, src/binaryQuantizationFormat.ts:141-601
 PUBLIC_MEMBERS = ["constructor", "quantizeVectors", "quantizeQueryVector", "searchNearestNeighbors",
                   "computeQuantizationAccuracy", "serializeVectorData", "deserializeVectorData", "getConfig",
@@ -60,7 +62,7 @@ def test_typescript_class_keeps_every_public_member_of_the_reference():
     assert "constructor(config: BinaryQuantizationConfig)" in ts and "super(config)" in ts
     inherited = set(PUBLIC_MEMBERS) - overridden - {"constructor"}
     assert inherited == {"getConfig", "getQuantizer", "getScorer"}
-    if os.path.exists(REFERENCE_CLASS):   # (this container only; the GPU box has no /root/reference)
+    if REFERENCE_CLASS and os.path.exists(REFERENCE_CLASS):   # with a reference checkout (BBQ_REFERENCE_DIR)
         ref = open(REFERENCE_CLASS, encoding="utf-8").read()
         body = ref[ref.index("export class BinaryQuantizationFormat"):]
         ref_public = set(re.findall(r"^  public (\w+)\(", body, flags=re.M)) | {"constructor"}

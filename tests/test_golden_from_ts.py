@@ -1,6 +1,6 @@
 """Oracle vs fixtures generated FROM THE REFERENCE'S OWN SOURCE TEXT.
 
-`tests/golden/from_ts/*.ts.json` were produced by executing the unmodified `/root/reference/src/index.ts` (and every
+`tests/golden/from_ts/*.ts.json` were produced by executing the unmodified `src/index.ts` of the reference (and every
 module it imports) with `tests/golden/from_ts/tsinterp.py` — a TypeScript-subset interpreter written for this purpose,
 because no JavaScript runtime exists in the image or on the GPU box (profiles/r02_js_runtime_probe.txt) — through
 `tests/golden/from_ts/make_golden_with_interp.py`.  Each fixture records the SHA-256 of the reference files that produced
@@ -21,6 +21,8 @@ import pytest
 from oracle import oracle as O
 from tests.fixtures import gaussian
 from tests.golden.make_golden import CASES, case_inputs
+from tests.golden.from_ts import live_cases as L
+from tests.golden_util import HAVE_REFERENCE, REFERENCE_DIR
 
 HERE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "from_ts")
 FIXTURES = sorted(glob.glob(os.path.join(HERE, "*.ts.json")))
@@ -35,7 +37,7 @@ def _u64(a):
 
 
 def test_fixtures_from_the_reference_source_exist():
-    assert len(FIXTURES) >= 11, "run tests/golden/from_ts/make_golden_with_interp.py (needs /root/reference)"
+    assert len(FIXTURES) >= 11, "run tests/golden/from_ts/make_golden_with_interp.py (needs the reference)"
     sims = {json.load(open(p))["sim"] for p in FIXTURES}
     assert sims == {"EUCLIDEAN", "COSINE", "MAXIMUM_INNER_PRODUCT"}
 
@@ -85,32 +87,33 @@ def test_oracle_equals_the_typescript_reference(path):
             assert np.float64(stats[f]).view(np.uint64) == np.float64(want).view(np.uint64), f
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="the reference sources are not on this box")
+def _oracle_equals_stored(cases, stored):
+    """The oracle against the reference's stored answers for `cases` (live_cases.py): correctives (f64 bit patterns), packed
+    codes, the heap-ordered top-k list of every query and its f32 scores."""
+    for name, sim, qb, lam, iters, k, base, queries in cases:
+        idx = O.quantize_vectors(base, sim=sim, index_bits=1, lam=lam, iters=iters)
+        res = [O.search_nearest_neighbors(q, idx, k, query_bits=qb, lam=lam, iters=iters, mode="heap") for q in queries]
+        assert L.encode(idx.corr, idx.packed, [(i.tolist(), s) for i, s in res]) == stored[name], name
+
+
+def _reference_equals_stored(cases, stored):
+    """With a reference checkout: the reference source, interpreted now, gives the stored answers (guards them, and the
+    interpreter, against going stale)."""
+    if HAVE_REFERENCE:
+        live = L.run_reference(REFERENCE_DIR, cases)
+        for name, *_ in cases:
+            assert live[name] == stored[name], name
+
+
 @pytest.mark.parametrize("sim,qb,n,dim", [("COSINE", 4, 40, 24), ("EUCLIDEAN", 1, 30, 20), ("MAXIMUM_INNER_PRODUCT", 4, 36, 36)])
 def test_reference_source_interpreted_live_equals_oracle(sim, qb, n, dim):
-    """Where /root/reference exists (the build container), run the reference source through the interpreter NOW on a
-    tiny seeded case and compare with the oracle — guards the committed fixtures against a stale interpreter."""
-    import sys
-    sys.path.insert(0, HERE)
-    import tsinterp as T
-    console = []
-    interp = T.Interp(log=lambda *a: console.append(a), stub_modules=["/src/wasm/index.ts"])
-    ex = interp.load("/root/reference/src/index.ts")
-    base, queries = gaussian(n, dim, 4242 + n), gaussian(2, dim, 4343 + n)
-    fmt = interp.call(ex["createBinaryQuantizationFormat"], args=[
-        {"queryBits": float(qb), "indexBits": 1.0, "quantizer": {"similarityFunction": sim, "lambda": 0.1, "iters": 5.0}}])
-    rows = [interp.float32(r.tolist()) for r in base]
-    qv = interp.call(interp.get(fmt, "quantizeVectors"), fmt, [rows])["quantizedVectors"]
-    idx = O.quantize_vectors(base, sim=sim, index_bits=1)
-    corr = np.array([[interp.call(interp.get(qv, "getCorrectiveTerms"), qv, [float(i)])[f] for f in
-                      ("lowerInterval", "upperInterval", "additionalCorrection", "quantizedComponentSum")] for i in range(n)], np.float64)
-    assert np.array_equal(_u64(corr), _u64(idx.corr))
-    for q in queries:
-        res = interp.call(interp.get(fmt, "searchNearestNeighbors"), fmt, [interp.float32(q.tolist()), qv, 5.0])
-        hi, hs = O.search_nearest_neighbors(q, idx, 5, query_bits=qb, mode="heap")
-        assert [int(r["index"]) for r in res] == hi.tolist()
-        assert np.array([r["score"] for r in res], np.float32).view(np.uint32).tolist() == hs.view(np.uint32).tolist()
-    assert not console
+    """A tiny seeded case, two queries: the oracle gives the reference's answers (stored in live_cases.json; run through
+    the reference source again when BBQ_REFERENCE_DIR names a checkout)."""
+    cases = [c for c in L.fixed_cases() if c[0] == f"fixed_{sim}_{qb}_{n}x{dim}"]
+    assert len(cases) == 1
+    stored = L.load_stored()
+    _oracle_equals_stored(cases, stored)
+    _reference_equals_stored(cases, stored)
 
 
 class _OracleBackedFormat:
@@ -205,54 +208,15 @@ def test_host_messages_equal_the_executed_reference():
     assert str(e.value) == by[("COSINE", "ragged rows (row 1 has 10 of 64 dims)")]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="the reference sources are not on this box")
 def test_fuzz_reference_source_interpreted_live_equals_oracle():
-    """150 random small configurations, reference source (interpreted, now) vs oracle: every similarity function, query
-    bits 1..8, dims 1..70 (below and across the 8-dim packing boundary), 1..40 rows, lambda in {0, 0.001, 0.1, 0.5, 1},
-    0 / 1 / 5 / 20 iterations, component scales 1e-3..1e3, duplicated and all-zero rows; every sixth case each made of
-    signed zeros only, of integers, or of values near the top of the f32 range.  Correctives (f64 bit patterns),
-    packed codes, the heap-ordered top-k list and its f32 scores must be identical in every case.  (Four other seeds x
-    150 cases were run by hand when this was written: no mismatch.)"""
-    import sys
-    sys.path.insert(0, HERE)
-    import tsinterp as T
-    console = []
-    interp = T.Interp(log=lambda *a: console.append(a), stub_modules=["/src/wasm/index.ts"])
-    ex = interp.load("/root/reference/src/index.ts")
-    rng = np.random.default_rng(7)
-    sims = ["EUCLIDEAN", "COSINE", "MAXIMUM_INNER_PRODUCT"]
-    for case in range(150):
-        sim, qb = sims[rng.integers(3)], int(rng.integers(1, 9))
-        dim, n = int(rng.choice([1, 2, 3, 5, 7, 8, 9, 15, 16, 17, 31, 33, 64, 70])), int(rng.integers(1, 40))
-        lam, iters, k = float(rng.choice([0.1, 0.001, 0.5, 0.0, 1.0])), int(rng.choice([0, 1, 5, 20])), int(rng.integers(1, 12))
-        scale = float(rng.choice([1.0, 1e-3, 1e3]))
-        base = (rng.standard_normal((n, dim)) * scale).astype(np.float32)
-        q = (rng.standard_normal(dim) * scale).astype(np.float32)
-        if rng.random() < 0.3:
-            base[rng.integers(n)] = base[0]
-        if rng.random() < 0.2:
-            base[rng.integers(n)] = 0
-        kind = case % 6                                  # every sixth case each: an extreme shape
-        if kind == 1:                                    # signed zeros only (Math.min(+0, -0) = -0 decides the interval's sign)
-            base[:, ::2] = 0
-            base[:, 1::2] = np.float32(-0.0) * base[:, 1::2]
-        elif kind == 2:                                  # integers: exact ties and .5 roundings
-            base, q = np.round(base).astype(np.float32), np.round(q).astype(np.float32)
-        elif kind == 3:                                  # near the top of the f32 range
-            base = (rng.standard_normal((n, dim)) * 1e30).astype(np.float32)
-            q[0] = np.float32(3e38)
-        tag = (case, kind, sim, qb, dim, n, lam, iters, k, scale)
-        fmt = interp.call(ex["createBinaryQuantizationFormat"], args=[
-            {"queryBits": float(qb), "indexBits": 1.0, "quantizer": {"similarityFunction": sim, "lambda": lam, "iters": float(iters)}}])
-        qv = interp.call(interp.get(fmt, "quantizeVectors"), fmt, [[interp.float32(r.tolist()) for r in base]])["quantizedVectors"]
-        corr = np.array([[interp.call(interp.get(qv, "getCorrectiveTerms"), qv, [float(i)])[f] for f in
-                          ("lowerInterval", "upperInterval", "additionalCorrection", "quantizedComponentSum")] for i in range(n)], np.float64)
-        packed = np.array([list(interp.call(interp.get(qv, "vectorValue"), qv, [float(i)]).a) for i in range(n)], np.uint8)
-        res = interp.call(interp.get(fmt, "searchNearestNeighbors"), fmt, [interp.float32(q.tolist()), qv, float(k)])
-        idx = O.quantize_vectors(base, sim=sim, index_bits=1, lam=lam, iters=iters)
-        hi, hs = O.search_nearest_neighbors(q, idx, k, query_bits=qb, lam=lam, iters=iters, mode="heap")
-        assert np.array_equal(_u64(corr), _u64(idx.corr)), tag
-        assert np.array_equal(packed, idx.packed), tag
-        assert [int(r["index"]) for r in res] == hi.tolist(), tag
-        assert np.array([r["score"] for r in res], np.float32).view(np.uint32).tolist() == hs.view(np.uint32).tolist(), tag
-    assert not console
+    """150 random small configurations (live_cases.fuzz_cases: every similarity function, query bits 1..8, dims 1..70,
+    1..40 rows, lambda 0..1, 0..20 iterations, scales 1e-3..1e3, duplicated and all-zero rows, signed zeros, integers,
+    values near the f32 limit): correctives (f64 bit patterns), packed codes, the heap-ordered top-k list and its f32
+    scores of the oracle are the reference's in every case (stored in live_cases.json; run through the reference source
+    again when BBQ_REFERENCE_DIR names a checkout).  This is the comparison that found the signed-zero rule of
+    Math.min / Math.max."""
+    cases = L.fuzz_cases()
+    assert len(cases) == 150
+    stored = L.load_stored()
+    _oracle_equals_stored(cases, stored)
+    _reference_equals_stored(cases, stored)

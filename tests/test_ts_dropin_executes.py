@@ -5,7 +5,8 @@ is the CPU oracle (tests/ts_dropin/oracle_addon.py: same function names, argumen
 bindings/napi/bbq_napi.c).  What this checks is the TypeScript layer itself, which nothing had ever run: that it loads in
 place of the reference's file with `src/index.ts` unchanged, marshals arguments and results correctly, keeps every public
 member, and is indistinguishable from the reference's class to a caller — same values bit for bit, same Error messages —
-including to the reference's own vitest file.  Needs /root/reference (skipped elsewhere)."""
+including to the reference's own vitest file.  Needs a checkout of the reference in BBQ_REFERENCE_DIR (skipped
+without one)."""
 import json
 import os
 import struct
@@ -15,11 +16,11 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden", "from_ts"))
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="the reference sources are not on this box")
-
 from tests.fixtures import edge_dataset, gaussian  # noqa: E402
+from tests.golden_util import HAVE_REFERENCE, REFERENCE_DIR as REF  # noqa: E402
+
+pytestmark = pytest.mark.skipif(not HAVE_REFERENCE, reason="needs a checkout of the reference project in BBQ_REFERENCE_DIR")
 
 SIMS = ["EUCLIDEAN", "COSINE", "MAXIMUM_INNER_PRODUCT"]
 

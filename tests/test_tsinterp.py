@@ -12,6 +12,8 @@ import pytest
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "from_ts"))
 import tsinterp as T  # noqa: E402
 
+from tests.golden_util import HAVE_REFERENCE, REFERENCE_DIR  # noqa: E402
+
 
 def run(tmp_path, src, extra=None, fn="main", args=()):
     for name, text in (extra or {}).items():
@@ -179,7 +181,7 @@ def test_modules_and_errors(tmp_path):
             run(tmp_path, bad)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tests"), reason="the reference is not on this box")
+@pytest.mark.skipif(not HAVE_REFERENCE, reason="needs a checkout of the reference project in BBQ_REFERENCE_DIR")
 @pytest.mark.parametrize("name,tests", [("utils.test.ts", 27), ("computeCentroid-correctness.test.ts", 2), ("recall.test.ts", 8)])
 def test_reference_own_test_files_pass_under_the_interpreter(name, tests):
     """The reference's OWN vitest files, executed against the reference's own sources by the interpreter (a minimal
@@ -187,6 +189,6 @@ def test_reference_own_test_files_pass_under_the_interpreter(name, tests):
     files — batch-*.test.ts, simple-quantized-query.test.ts, recall-all-dimensions.test.ts: thousands of 1024-d vectors —
     are not run: an interpreter in Python is the wrong tool for those.)"""
     import vitest_shim as V
-    passed, failed, assertions, console = V.run_test_file(os.path.join("/root/reference/tests", name))
+    passed, failed, assertions, console = V.run_test_file(os.path.join(REFERENCE_DIR, "tests", name))
     assert not failed, failed[:3]
     assert len(passed) == tests and assertions > 0
