@@ -73,6 +73,9 @@ SYMBOLS = {
     "bbq_index_attach_rows": (C.c_int, [_vp, _vp]),
     "bbq_index_attach_rows_device": (C.c_int, [_vp, _vp]),
     "bbq_search_rerank": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp, _vp, C.POINTER(C.c_uint32)]),
+    "bbq_search_rerank_sharded": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp, _vp,
+                                            C.POINTER(C.c_uint32)]),
+    "bbq_rerank_owned_device": (C.c_int, [_vp, _vp, C.c_uint32, _vp, C.c_uint32, _vp, _vp]),
     "bbq_merge_topk_device": (C.c_int, [_vp, _vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp, _vp]),
     "bbq_debug_quantize_query": (C.c_int, [_vp, _vp, _vp, _vp]),
     "bbq_debug_qcdist": (C.c_int, [_vp, _vp, _vp]),

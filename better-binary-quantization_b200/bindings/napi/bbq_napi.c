@@ -217,7 +217,7 @@ static napi_value n_attach_rows(napi_env env, napi_callback_info info) {
 
 /* searchRerank(index, queriesFlat, nq, k, oversampleFactor) -> {indices, quantizedScores, trueScores, count}
  * replaces getOversampledTopKWithSort / getOversampledTopKWithHeap, src/topKSelector.ts:29-114 */
-static napi_value n_search_rerank(napi_env env, napi_callback_info info) {
+static napi_value rerank_common(napi_env env, napi_callback_info info, int sharded) {
   ARGS(5);
   void* ix;
   const float* q;
@@ -236,7 +236,8 @@ static napi_value n_search_rerank(napi_env env, napi_callback_info info) {
   void* p2 = p1 ? new_buffer(env, slots * sizeof(float), &a2) : NULL;
   void* p3 = p2 ? new_buffer(env, slots * sizeof(double), &a3) : NULL;
   if (!p1 || !p2 || !p3) return NULL;
-  const int st = bbq_search_rerank((bbq_index*)ix, q, nq, k, factor, (int32_t*)p1, (float*)p2, (double*)p3, &count);
+  const int st = sharded ? bbq_search_rerank_sharded((bbq_index*)ix, q, nq, k, factor, (int32_t*)p1, (float*)p2, (double*)p3, &count)
+                         : bbq_search_rerank((bbq_index*)ix, q, nq, k, factor, (int32_t*)p1, (float*)p2, (double*)p3, &count);
   if (st != BBQ_OK) return throw_status(env, st);
   napi_create_typedarray(env, napi_int32_array, slots, a1, 0, &t1);
   napi_create_typedarray(env, napi_float32_array, slots, a2, 0, &t2);
@@ -249,6 +250,10 @@ static napi_value n_search_rerank(napi_env env, napi_callback_info info) {
   napi_set_named_property(env, out, "count", v);
   return out;
 }
+static napi_value n_search_rerank(napi_env env, napi_callback_info info) { return rerank_common(env, info, 0); }
+/* searchRerankSharded(index, queriesFlat, nq, k, oversampleFactor): the same over ALL row shards of the box
+ * (collective; bbq_search_rerank_sharded), same result object */
+static napi_value n_search_rerank_sharded(napi_env env, napi_callback_info info) { return rerank_common(env, info, 1); }
 
 static int get_path(napi_env env, napi_value v, char* buf, size_t cap) {
   size_t n = 0;
@@ -409,6 +414,7 @@ NAPI_MODULE_INIT() {
       {"rows", NULL, n_rows, NULL, NULL, NULL, 0, NULL},
       {"attachRows", NULL, n_attach_rows, NULL, NULL, NULL, 0, NULL},
       {"searchRerank", NULL, n_search_rerank, NULL, NULL, NULL, 0, NULL},
+      {"searchRerankSharded", NULL, n_search_rerank_sharded, NULL, NULL, NULL, 0, NULL},
       {"saveIndex", NULL, n_save_index, NULL, NULL, NULL, 0, NULL},
       {"loadIndex", NULL, n_load_index, NULL, NULL, NULL, 0, NULL},
       {"quantizeQuery", NULL, n_quantize_query, NULL, NULL, NULL, 0, NULL},

@@ -39,6 +39,8 @@ const addon = require('./bbq_b200.node') as {
   attachRows(index: Handle, rows: Float32Array): void;
   searchRerank(index: Handle, queries: Float32Array, nq: number, k: number, factor: number):
     { indices: Int32Array; quantizedScores: Float32Array; trueScores: Float64Array; count: number };
+  searchRerankSharded(index: Handle, queries: Float32Array, nq: number, k: number, factor: number):
+    { indices: Int32Array; quantizedScores: Float32Array; trueScores: Float64Array; count: number };
   saveIndex(index: Handle, veb: string, vemb: string): void;
   loadIndex(ctx: Handle, veb: string, vemb: string): Handle;
   quantizeQuery(ctx: Handle, query: Float32Array, centroid: Float32Array): { codes: Uint8Array; corrections: Float64Array };
@@ -240,10 +242,14 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
     try { addon.attachRows(deviceHandle(targetVectors), flat); }
     catch (e) { throw toReferenceError(e, 'build'); }
   }
+  /** With sharded = true (after joinShardGroup, each rank's own rows attached) the re-rank runs over ALL row shards
+   *  of the box and returns, on every rank, what the unsharded call returns on the whole corpus. */
   public searchOversampled(queryVector: Float32Array, targetVectors: BinarizedByteVectorValues, k: number,
-      oversampleFactor: number): Array<{ index: number; quantizedScore: number; trueScore: number }> {
+      oversampleFactor: number, sharded = false): Array<{ index: number; quantizedScore: number; trueScore: number }> {
     try {
-      const r = addon.searchRerank(deviceHandle(targetVectors), queryVector, 1, k, oversampleFactor);
+      const h = deviceHandle(targetVectors);
+      const r = sharded ? addon.searchRerankSharded(h, queryVector, 1, k, oversampleFactor)
+                        : addon.searchRerank(h, queryVector, 1, k, oversampleFactor);
       return Array.from({ length: r.count }, (_u, i) =>
         ({ index: r.indices[i]!, quantizedScore: r.quantizedScores[i]!, trueScore: r.trueScores[i]! }));
     } catch (e) { throw toReferenceError(e, 'search'); }

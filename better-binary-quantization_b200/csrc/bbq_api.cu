@@ -202,7 +202,8 @@ struct bbq_index {
   double cdp = 0.0;
   uint64_t base = 0;
   IndexBounds* bounds = nullptr;  // device; valid for bounds_n rows (tensor-core screen margins)
-  float* rows = nullptr;          // device [n][dim]: original rows for the exact re-rank (bbq_index_attach_rows)
+  float* rows = nullptr;          // device [rows_n][dim]: original rows for the exact re-rank (bbq_index_attach_rows)
+  uint64_t rows_n = 0;            // rows attached: the re-rank refuses an index that has grown (appended) since
   float4* rscreen = nullptr;      // device [capacity]: per-row screen constants, same validity
   uint64_t bounds_n = 0;
   uint64_t capacity = 0;  // rows allocated (== n except while a streaming build is in progress)
@@ -1474,9 +1475,35 @@ static int attach_rows(bbq_index* ix, const float* rows, cudaMemcpyKind kind) {
   const size_t bytes = (size_t)ix->n * ix->dim * sizeof(float);
   if (ix->rows) CU(cudaFree(ix->rows));
   ix->rows = nullptr;
+  ix->rows_n = 0;
   CU(cudaMalloc(&ix->rows, bytes));
   CU(cudaMemcpyAsync(ix->rows, rows, bytes, kind, c->stream));
   CU(cudaStreamSynchronize(c->stream));
+  ix->rows_n = ix->n;
+  return BBQ_OK;
+}
+
+// the rows the exact re-rank reads must cover the whole index (not an index appended to after bbq_index_attach_rows)
+static int check_attached_rows(const bbq_index* ix) {
+  if (!ix->rows) return fail(BBQ_ERR_INVALID_ARG, "no original rows attached (bbq_index_attach_rows)");
+  if (ix->rows_n != ix->n)
+    return fail(BBQ_ERR_INVALID_ARG, "rows attached for " + std::to_string(ix->rows_n) + " rows, index has " +
+                                         std::to_string(ix->n));
+  return BBQ_OK;
+}
+
+static int launch_rerank_scores(bbq_index* ix, bool owned_only, const float* d_queries, uint32_t nq, uint32_t m,
+                                const int32_t* d_cand_idx, double* d_true, cudaStream_t st) {
+  bbq_ctx* c = ix->ctx;
+  const int64_t pairs = (int64_t)nq * m;
+  const unsigned grid = (unsigned)((pairs + RERANK_WARPS - 1) / RERANK_WARPS);
+  if (owned_only) {
+    LAUNCH(c, k_rerank_scores<true>, grid, RERANK_WARPS * 32, 0, st, ix->rows, (int)ix->dim, d_queries, (int)nq, (int)m,
+           d_cand_idx, (uint32_t)ix->base, (uint32_t)ix->rows_n, d_true);
+  } else {
+    LAUNCH(c, k_rerank_scores<false>, grid, RERANK_WARPS * 32, 0, st, ix->rows, (int)ix->dim, d_queries, (int)nq, (int)m,
+           d_cand_idx, (uint32_t)ix->base, (uint32_t)ix->rows_n, d_true);
+  }
   return BBQ_OK;
 }
 extern "C" int bbq_index_attach_rows(bbq_index* ix, const float* rows) { return attach_rows(ix, rows, cudaMemcpyHostToDevice); }
@@ -1484,38 +1511,24 @@ extern "C" int bbq_index_attach_rows_device(bbq_index* ix, const float* d_rows) 
   return attach_rows(ix, d_rows, cudaMemcpyDeviceToDevice);
 }
 
-extern "C" int bbq_search_rerank(bbq_index* ix, const float* queries, uint32_t nq, uint32_t k, uint32_t factor,
-                                 int32_t* out_idx, float* out_qscore, double* out_true, uint32_t* out_count) {
-  if (out_count) *out_count = 0;
-  if (!ix) return fail(BBQ_ERR_NULL, "target vector set must not be null");
-  if (!queries) return fail(BBQ_ERR_NULL, "query vector must not be null");
-  if (!ix->rows) return fail(BBQ_ERR_INVALID_ARG, "no original rows attached (bbq_index_attach_rows)");
-  if (nq == 0 || k == 0) return BBQ_OK;
-  if (!out_idx || !out_qscore || !out_true) return fail(BBQ_ERR_NULL, "output buffers must not be null");
-  if (factor == 0 || (uint64_t)k * factor > K_MAX) return fail(BBQ_ERR_UNSUPPORTED, "k * oversampleFactor must be in 1..4096");
-  bbq_ctx* c = ix->ctx;
-  const uint32_t m = (uint32_t)std::min<uint64_t>((uint64_t)k * factor, ix->n);  // candidates per query
-  const uint32_t kk = std::min(k, m);
-  CU(cudaSetDevice(c->device));
-  cudaStream_t st = c->stream;
-  TRY(c->qrows.reserve((size_t)nq * ix->dim * sizeof(float)));
+// scratch of a re-rank call: m candidates and kk results per query
+static int reserve_rerank(bbq_ctx* c, uint32_t dim, uint32_t nq, uint32_t m, uint32_t kk) {
+  TRY(c->qrows.reserve((size_t)nq * dim * sizeof(float)));
   TRY(c->out_idx.reserve((size_t)nq * m * sizeof(int32_t)));
   TRY(c->out_score.reserve((size_t)nq * m * sizeof(float)));
   TRY(c->rr_true.reserve((size_t)nq * m * sizeof(double)));
   TRY(c->rr_idx.reserve((size_t)nq * kk * sizeof(int32_t)));
   TRY(c->rr_q.reserve((size_t)nq * kk * sizeof(float)));
   TRY(c->rr_t.reserve((size_t)nq * kk * sizeof(double)));
-  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * ix->dim * sizeof(float), cudaMemcpyHostToDevice, st));
-  ValidationScope vscope(c);
-  TRY(enqueue_query_validation(c, c->qrows.as<float>(), st));
-  TRY(bbq_search_device(ix, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(), c->out_score.as<float>(), st));
-  TRY(finish_query_validation(c, st, /*sync=*/false));
+  return BBQ_OK;
+}
+
+// the tail of a re-rank call, once rr_true holds the exact score of every candidate in out_idx / out_score: the kk
+// best per query into the caller's rows of stride k, one synchronisation, then the verdict of the query screening
+static int rerank_select_and_copy(bbq_ctx* c, cudaStream_t st, uint32_t nq, uint32_t m, uint32_t k, uint32_t kk,
+                                  int32_t* out_idx, float* out_qscore, double* out_true) {
   {
     ProfScope prof(c, st, PROF_SELECT);
-    const int64_t pairs = (int64_t)nq * m;
-    LAUNCH(c, k_rerank_scores, (unsigned)((pairs + RERANK_WARPS - 1) / RERANK_WARPS), RERANK_WARPS * 32, 0, st, ix->rows,
-           (int)ix->dim, c->qrows.as<float>(), (int)nq, (int)m, c->out_idx.as<int32_t>(), (uint32_t)ix->base,
-           c->rr_true.as<double>());
     LAUNCH(c, k_rerank_select, nq, 256, 0, st, c->rr_true.as<double>(), c->out_idx.as<int32_t>(), c->out_score.as<float>(),
            (int)m, kk, c->rr_idx.as<int32_t>(), c->rr_q.as<float>(), c->rr_t.as<double>());
   }
@@ -1531,7 +1544,35 @@ extern "C" int bbq_search_rerank(bbq_index* ix, const float* queries, uint32_t n
   TRY(copy_out(out_qscore, c->rr_q.p, sizeof(float)));
   TRY(copy_out(out_true, c->rr_t.p, sizeof(double)));
   CU(cudaStreamSynchronize(st));
-  TRY(report_query_validation(c));
+  return report_query_validation(c);
+}
+
+extern "C" int bbq_search_rerank(bbq_index* ix, const float* queries, uint32_t nq, uint32_t k, uint32_t factor,
+                                 int32_t* out_idx, float* out_qscore, double* out_true, uint32_t* out_count) {
+  if (out_count) *out_count = 0;
+  if (!ix) return fail(BBQ_ERR_NULL, "target vector set must not be null");
+  if (!queries) return fail(BBQ_ERR_NULL, "query vector must not be null");
+  TRY(check_attached_rows(ix));
+  if (nq == 0 || k == 0) return BBQ_OK;
+  if (!out_idx || !out_qscore || !out_true) return fail(BBQ_ERR_NULL, "output buffers must not be null");
+  if (factor == 0 || (uint64_t)k * factor > K_MAX) return fail(BBQ_ERR_UNSUPPORTED, "k * oversampleFactor must be in 1..4096");
+  bbq_ctx* c = ix->ctx;
+  const uint32_t m = (uint32_t)std::min<uint64_t>((uint64_t)k * factor, ix->n);  // candidates per query
+  const uint32_t kk = std::min(k, m);
+  CU(cudaSetDevice(c->device));
+  cudaStream_t st = c->stream;
+  TRY(reserve_rerank(c, ix->dim, nq, m, kk));
+  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * ix->dim * sizeof(float), cudaMemcpyHostToDevice, st));
+  ValidationScope vscope(c);
+  TRY(enqueue_query_validation(c, c->qrows.as<float>(), st));
+  TRY(bbq_search_device(ix, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(), c->out_score.as<float>(), st));
+  TRY(finish_query_validation(c, st, /*sync=*/false));
+  {
+    ProfScope prof(c, st, PROF_SELECT);
+    TRY(launch_rerank_scores(ix, /*owned_only=*/false, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(),
+                             c->rr_true.as<double>(), st));
+  }
+  TRY(rerank_select_and_copy(c, st, nq, m, k, kk, out_idx, out_qscore, out_true));
   if (out_count) *out_count = kk;
   return BBQ_OK;
 }
@@ -1802,6 +1843,110 @@ extern "C" int bbq_search_sharded(bbq_index* ix, const float* queries, uint32_t 
   }
   CU(cudaStreamSynchronize(c->stream));
   TRY(report_query_validation(c));
+  if (out_count) *out_count = kk;
+  return BBQ_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// oversampled search + exact re-rank across row shards: the sharded search's global top-m candidates on every rank,
+// each candidate scored exactly by the one rank that holds its row (bbq_rerank_owned_device), the f64 bits summed as
+// integers in one ncclAllReduce (every other rank contributes 0), and the same k_rerank_select on every rank.
+// ------------------------------------------------------------------------------------------------
+extern "C" int bbq_rerank_owned_device(bbq_index* ix, const float* d_queries, uint32_t nq, const int32_t* d_cand_idx,
+                                       uint32_t m, uint64_t* d_true_bits, void* stream) {
+  if (!ix) return fail(BBQ_ERR_NULL, "target vector set must not be null");
+  if (!d_queries || !d_cand_idx || !d_true_bits) return fail(BBQ_ERR_NULL, "null");
+  TRY(check_attached_rows(ix));
+  if (nq == 0 || m == 0) return BBQ_OK;
+  bbq_ctx* c = ix->ctx;
+  CU(cudaSetDevice(c->device));
+  cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
+  StreamBridge bridge(c, st);
+  return launch_rerank_scores(ix, /*owned_only=*/true, d_queries, nq, m, d_cand_idx, reinterpret_cast<double*>(d_true_bits), st);
+}
+
+// One all-gather of every rank's {base, rows, rows attached, status of its local preparation}, before any collective
+// that depends on per-rank state: every rank derives the same verdict from the same words, so either all ranks go on
+// or all return the same status and message.  Attached rows must cover each shard (an empty shard needs none), and
+// the shards' id ranges must be disjoint: two owners of one id would add their bits together.
+static int agree_on_shards(bbq_index* ix, int local_status, cudaStream_t st, uint64_t* n_global) {
+  bbq_ctx* c = ix->ctx;
+  const int world = c->world;
+  TRY(c->nglob.reserve((size_t)(4 + 4 * world) * sizeof(unsigned long long)));
+  unsigned long long* d = c->nglob.as<unsigned long long>();
+  const unsigned long long mine[4] = {ix->base, ix->n, ix->rows_n, (unsigned long long)local_status};
+  std::vector<unsigned long long> all((size_t)4 * world);
+  CU(cudaMemcpyAsync(d, mine, sizeof mine, cudaMemcpyHostToDevice, st));
+  NC(nccl_api()->AllGather(d, d + 4, 4, ncclUint64, c->comm, st));
+  CU(cudaMemcpyAsync(all.data(), d + 4, all.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  auto word = [&](int r, int f) { return all[(size_t)4 * r + f]; };
+  for (int r = 0; r < world; r++)
+    if (word(r, 3) != BBQ_OK)
+      return fail((int)word(r, 3), "sharded re-rank: rank " + std::to_string(r) + " could not reserve its scratch (status " +
+                                       std::to_string(word(r, 3)) + ")");
+  uint64_t total = 0;
+  std::vector<int> order;
+  for (int r = 0; r < world; r++) {
+    const uint64_t n = word(r, 1), rows_n = word(r, 2);
+    if (n > 0 && rows_n == 0)
+      return fail(BBQ_ERR_INVALID_ARG, "sharded re-rank: rank " + std::to_string(r) +
+                                           " has no original rows attached (bbq_index_attach_rows)");
+    if (n > 0 && rows_n != n)
+      return fail(BBQ_ERR_INVALID_ARG, "sharded re-rank: rank " + std::to_string(r) + " has rows attached for " +
+                                           std::to_string(rows_n) + " rows, index has " + std::to_string(n));
+    if (n > 0) order.push_back(r);
+    total += n;
+  }
+  std::sort(order.begin(), order.end(), [&](int a, int b) { return word(a, 0) < word(b, 0) || (word(a, 0) == word(b, 0) && a < b); });
+  for (size_t i = 1; i < order.size(); i++) {
+    const int a = order[i - 1], b = order[i];
+    if (word(a, 0) + word(a, 1) > word(b, 0))
+      return fail(BBQ_ERR_INVALID_ARG, "sharded re-rank: the row ids of rank " + std::to_string(a) + " [" +
+                                           std::to_string(word(a, 0)) + ", " + std::to_string(word(a, 0) + word(a, 1)) +
+                                           ") overlap those of rank " + std::to_string(b) + " [" + std::to_string(word(b, 0)) +
+                                           ", " + std::to_string(word(b, 0) + word(b, 1)) + ")");
+  }
+  *n_global = total;
+  return BBQ_OK;
+}
+
+extern "C" int bbq_search_rerank_sharded(bbq_index* ix, const float* queries, uint32_t nq, uint32_t k, uint32_t factor,
+                                         int32_t* out_idx, float* out_qscore, double* out_true, uint32_t* out_count) {
+  if (out_count) *out_count = 0;
+  if (!ix) return fail(BBQ_ERR_NULL, "target vector set must not be null");
+  if (!queries) return fail(BBQ_ERR_NULL, "query vector must not be null");
+  bbq_ctx* c = ix->ctx;
+  if (!c->comm || c->world == 1)  // one shard: the plain entry
+    return bbq_search_rerank(ix, queries, nq, k, factor, out_idx, out_qscore, out_true, out_count);
+  // the replicated arguments: every rank reaches the same verdict on them without communicating
+  const bool work = nq != 0 && k != 0;
+  if (work && (!out_idx || !out_qscore || !out_true)) return fail(BBQ_ERR_NULL, "output buffers must not be null");
+  if (work && (factor == 0 || (uint64_t)k * factor > K_MAX))
+    return fail(BBQ_ERR_UNSUPPORTED, "k * oversampleFactor must be in 1..4096");
+  CU(cudaSetDevice(c->device));
+  cudaStream_t st = c->stream;
+  const uint32_t mk = work ? k * factor : 0;  // candidates per query before the clamp to the rows of all shards
+  const int prep = work ? reserve_rerank(c, ix->dim, nq, mk, k) : BBQ_OK;
+  uint64_t n_global = 0;
+  TRY(agree_on_shards(ix, prep, st, &n_global));
+  const uint32_t m = (uint32_t)std::min<uint64_t>(mk, n_global);
+  const uint32_t kk = std::min(k, m);
+  if (m == 0) return BBQ_OK;
+  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * ix->dim * sizeof(float), cudaMemcpyHostToDevice, st));
+  ValidationScope vscope(c);
+  TRY(enqueue_query_validation(c, c->qrows.as<float>(), st));
+  TRY(bbq_search_sharded_device(ix, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(), c->out_score.as<float>(), st));
+  TRY(finish_query_validation(c, st, /*sync=*/false));
+  {
+    ProfScope prof(c, st, PROF_SELECT);
+    TRY(launch_rerank_scores(ix, /*owned_only=*/true, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(),
+                             c->rr_true.as<double>(), st));
+    // integer sum, never a floating-point one: exactly one rank owns each filled slot, so the owner's bits arrive
+    // unchanged (-0.0 and NaN payloads included)
+    NC(nccl_api()->AllReduce(c->rr_true.p, c->rr_true.p, (size_t)nq * m, ncclUint64, ncclSum, c->comm, st));
+  }
+  TRY(rerank_select_and_copy(c, st, nq, m, k, kk, out_idx, out_qscore, out_true));
   if (out_count) *out_count = kk;
   return BBQ_OK;
 }

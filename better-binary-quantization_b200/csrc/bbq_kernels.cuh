@@ -1059,20 +1059,27 @@ __global__ void __launch_bounds__(SELECT_THREADS) k_select(const SelectParams p,
 // f32 row with computeCosineSimilarity (src/vectorSimilarity.ts:75-102: three interleaved sequential f64 sums),
 // and the k best true scores are kept — (trueScore desc, quantised rank asc), i.e. the stable sort of
 // getOversampledTopKWithSort.
+// kOwnedOnly (a row shard, global candidate ids): only candidates with 0 <= idx - base < rows_n are scored; every other
+// slot, empty ones included, gets +0.0, whose bits are 0, so that an integer sum of all shards' outputs delivers each
+// owner's f64 bits unchanged.
 // ------------------------------------------------------------------------------------------------
 constexpr int RERANK_WARPS = 4;
+template <bool kOwnedOnly>
 __global__ void __launch_bounds__(RERANK_WARPS * 32) k_rerank_scores(const float* __restrict__ rows, int dim,
                                                                     const float* __restrict__ queries, int nq, int m,
                                                                     const int32_t* __restrict__ cand_idx,
-                                                                    uint32_t base, double* __restrict__ true_scores) {
+                                                                    uint32_t base, uint32_t rows_n,
+                                                                    double* __restrict__ true_scores) {
   __shared__ double terms_s[RERANK_WARPS][6][33];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t pair = (int64_t)blockIdx.x * RERANK_WARPS + warp;
   if (pair >= (int64_t)nq * m) return;
   const int q = (int)(pair / m);
   const int32_t idx = cand_idx[pair];
-  if (idx < 0) {
-    if (lane == 0) true_scores[pair] = -INFINITY;  // empty slot (fewer than k*factor rows)
+  // base + rows_n < 2^31 (bbq_index_set_base), so an id below base wraps to >= 2^31 and fails the unsigned test too
+  const bool skip = idx < 0 || (kOwnedOnly && (uint32_t)idx - base >= rows_n);
+  if (skip) {
+    if (lane == 0) true_scores[pair] = kOwnedOnly ? 0.0 : -INFINITY;  // empty slot (fewer than k*factor rows) / not ours
     return;
   }
   const float* a = queries + (int64_t)q * dim;

@@ -352,8 +352,10 @@ class BinaryQuantizationFormat:
         """Same, rows already in device memory ([size, dimension] f32, e.g. a torch tensor's data_ptr())."""
         _check(_native.load().bbq_index_attach_rows_device(targetVectors._h, d_rows_ptr), "build")
 
-    def searchOversampledBatch(self, queries, targetVectors: BinarizedByteVectorValues, k: int, oversampleFactor: int):
-        """-> (idx i32[nq, kk], quantizedScore f32[nq, kk], trueScore f64[nq, kk])"""
+    def searchOversampledBatch(self, queries, targetVectors: BinarizedByteVectorValues, k: int, oversampleFactor: int,
+                               sharded: bool = False):
+        """-> (idx i32[nq, kk], quantizedScore f32[nq, kk], trueScore f64[nq, kk]).  sharded=True: over all row shards
+        of the communicator (bbq_search_rerank_sharded, collective), the same lists on every rank."""
         qs = np.ascontiguousarray(queries, np.float32)
         if qs.ndim != 2 or qs.shape[1] != targetVectors.dimension():
             raise BbqError(4, "查询向量维度与目标向量维度不匹配")
@@ -362,10 +364,18 @@ class BinaryQuantizationFormat:
         qsc = np.empty((nq, max(k, 1)), np.float32)
         tsc = np.empty((nq, max(k, 1)), np.float64)
         cnt = C.c_uint32(0)
-        _check(_native.load().bbq_search_rerank(targetVectors._h, qs.ctypes.data, nq, k, oversampleFactor,
-                                                idx.ctypes.data, qsc.ctypes.data, tsc.ctypes.data, C.byref(cnt)), "search")
+        L = _native.load()
+        fn = L.bbq_search_rerank_sharded if sharded else L.bbq_search_rerank
+        _check(fn(targetVectors._h, qs.ctypes.data, nq, k, oversampleFactor, idx.ctypes.data, qsc.ctypes.data,
+                  tsc.ctypes.data, C.byref(cnt)), "search")
         n = cnt.value
         return idx[:, :n].copy(), qsc[:, :n].copy(), tsc[:, :n].copy()
+
+    def rerankOwnedDevice(self, targetVectors: BinarizedByteVectorValues, d_queries_ptr: int, nq: int,
+                          d_cand_idx_ptr: int, m: int, d_true_bits_ptr: int, stream: int = 0):
+        """bbq_rerank_owned_device: [nq][m] u64 = this shard's exact-score bits for the candidates it holds, else 0."""
+        _check(_native.load().bbq_rerank_owned_device(targetVectors._h, d_queries_ptr, nq, d_cand_idx_ptr, m,
+                                                      d_true_bits_ptr, stream or None), "search")
 
     # -- parity taps (tests) ------------------------------------------------------------------------------
     def debugQcDist(self, queryVector, targetVectors: BinarizedByteVectorValues) -> np.ndarray:

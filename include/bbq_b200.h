@@ -210,7 +210,9 @@ void bbq_host_free(void* p);
 /* -------- oversampled search + exact re-rank (SURVEY §8f rank 2) ---------------------------------------- */
 
 /* Keeps a copy of the ORIGINAL f32 rows next to the index (device memory, n*dim*4 bytes) for the exact re-rank.
- * rows: HOST (bbq_index_attach_rows) or DEVICE (bbq_index_attach_rows_device) memory, n = bbq_index_size rows. */
+ * rows: HOST (bbq_index_attach_rows) or DEVICE (bbq_index_attach_rows_device) memory, n = bbq_index_size rows.
+ * The copy covers the rows the index has at attach time: after a later bbq_index_append* the re-rank entries return
+ * BBQ_ERR_INVALID_ARG ("rows attached for N rows, index has M") until the rows are attached again. */
 int bbq_index_attach_rows(bbq_index* index, const float* rows);
 int bbq_index_attach_rows_device(bbq_index* index, const float* d_rows);
 
@@ -221,6 +223,28 @@ int bbq_index_attach_rows_device(bbq_index* index, const float* d_rows);
  * out_idx / out_qscore (the quantised f32 score) / out_true (f64): nq*k each; k*factor <= 4096. */
 int bbq_search_rerank(bbq_index* index, const float* queries, uint32_t nq, uint32_t k, uint32_t factor,
                       int32_t* out_idx, float* out_qscore, double* out_true, uint32_t* out_count);
+
+/* bbq_search_rerank over ALL row shards (the sharded search's setup: bbq_comm_init, bbq_index_set_base, and the
+ * original rows of its own shard attached on every rank).  Collective: every rank calls it with the same queries, nq,
+ * k and factor, and every rank gets, bit for bit, what bbq_search_rerank returns on one index holding the whole
+ * corpus: m = min(k*factor, rows over all ranks) candidates per query, *out_count = min(k, m), k*factor <= 4096.
+ * The candidates are the sharded search's global top m; the rank that holds a candidate's row scores it, and the f64
+ * bits reach every rank in one integer-sum ncclAllReduce of nq*m words.  Before that exchange the ranks share
+ * {base, rows, rows attached} in one small all-gather: a rank without rows attached for all its rows, or two ranks
+ * whose id ranges overlap, make EVERY rank return BBQ_ERR_INVALID_ARG with the same message.  Query screening and
+ * argument errors are those of bbq_search_rerank.  Without a communicator (or world == 1) it is bbq_search_rerank.
+ * HOST pointers. */
+int bbq_search_rerank_sharded(bbq_index* index, const float* queries, uint32_t nq, uint32_t k, uint32_t factor,
+                              int32_t* out_idx, float* out_qscore, double* out_true, uint32_t* out_count);
+
+/* The shard-local step of bbq_search_rerank_sharded on its own (not collective; a host with an exchange of its own
+ * uses it the way it uses bbq_merge_topk_device): for [nq][m] GLOBAL candidate ids d_cand_idx (-1 = empty slot),
+ * writes [nq][m] 64-bit words to d_true_bits: the bits of the f64 computeCosineSimilarity of query and row
+ * (src/vectorSimilarity.ts:75-102, the same arithmetic as bbq_search_rerank) when this shard holds the row
+ * (0 <= id - base < rows), else 0.  Summed as integers over all shards, the words are the exact scores' bits.
+ * d_queries: the raw nq*dim f32 queries.  DEVICE pointers, enqueued on `stream` (NULL = the context's stream). */
+int bbq_rerank_owned_device(bbq_index* index, const float* d_queries, uint32_t nq, const int32_t* d_cand_idx,
+                            uint32_t m, uint64_t* d_true_bits, void* stream);
 
 /* Deterministic merge of `lists` per-shard results (e.g. after an NCCL allgather, SURVEY §8e):
  * inputs [lists][nq][k] idx / score in DEVICE memory, output [nq][k].  Replaces nothing in the
