@@ -48,9 +48,15 @@ static int fail(int status, const std::string& msg, int64_t vec = -1, int64_t po
   } while (0)
 
 static std::atomic<uint64_t> g_scratch_gen{0};  // bumped whenever any scratch buffer moves: a captured launch sequence holds its address
-struct DevBuf {  // grow-only device scratch
+struct DevBuf {  // grow-only device scratch, freed with its owner (on the owner's device)
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
   int reserve(size_t bytes) {
     if (bytes <= cap) return BBQ_OK;
     g_scratch_gen++;
@@ -60,11 +66,6 @@ struct DevBuf {  // grow-only device scratch
     CU(cudaMalloc(&p, bytes));
     cap = bytes;
     return BBQ_OK;
-  }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
   }
   template <class T>
   T* as() const { return reinterpret_cast<T*>(p); }
@@ -83,7 +84,7 @@ struct bbq_ctx {
   // build scratch
   DevBuf T, stage, cacc;
   // query scratch
-  DevBuf qrows, qT, qcodes, qcorr, planes, qterms, tau, dump, cand, cand_cnt, flag, lists_a, lists_b,
+  DevBuf qrows, qT, qcodes, qcorr, planes, qterms, tau, dump, cand, cand_cnt, lists_a, lists_b,
       out_idx, out_score, dots, images, qscreen, tau_bits, trace, rr_true, rr_idx, rr_q, rr_t, cenv, qoff, qenv;
   int64_t sample_tiles_dyn = 128;  // BBQ_SAMPLE_TILES: sample size when the running threshold is on
   int k1s_ctas = 4;         // BBQ_K1S_CTAS: persistent CTAs per SM of the streaming scan (huge = one tile per CTA)
@@ -282,14 +283,8 @@ extern "C" int bbq_create(const bbq_config* config, bbq_ctx** out_ctx) {
 static void comm_release(bbq_ctx* c);
 static void ctx_release(bbq_ctx* c) {
   if (--c->refs > 0) return;
-  cudaSetDevice(c->device);
+  cudaSetDevice(c->device);  // also for the scratch buffers, which `delete c` frees
   cudaStreamSynchronize(c->stream);
-  for (DevBuf* b : {&c->T, &c->stage, &c->cacc, &c->qrows, &c->qT, &c->qcodes, &c->qcorr, &c->planes, &c->qterms,
-                    &c->tau, &c->dump, &c->cand, &c->cand_cnt, &c->flag, &c->lists_a, &c->lists_b, &c->out_idx,
-                    &c->out_score, &c->dots, &c->images, &c->qscreen, &c->tau_bits, &c->trace, &c->rr_true, &c->rr_idx,
-                    &c->rr_q, &c->rr_t, &c->cenv, &c->qoff, &c->qenv, &c->keys_local, &c->keys_all, &c->loc_idx, &c->loc_score, &c->bad,
-                    &c->nglob})
-    b->release();
   comm_release(c);
   if (c->h_flag) cudaFreeHost(c->h_flag);
   if (c->sgraph.exec) cudaGraphExecDestroy(c->sgraph.exec);
@@ -403,6 +398,20 @@ extern "C" void bbq_index_destroy(bbq_index* ix) {
   ctx_release(c);
 }
 
+// an index under construction: destroyed on every early return unless released to the caller
+struct IndexGuard {
+  bbq_index* ix = nullptr;
+  IndexGuard() = default;
+  IndexGuard(const IndexGuard&) = delete;
+  IndexGuard& operator=(const IndexGuard&) = delete;
+  ~IndexGuard() { bbq_index_destroy(ix); }
+  bbq_index* release() {
+    bbq_index* r = ix;
+    ix = nullptr;
+    return r;
+  }
+};
+
 static int finish_centroid(bbq_index* ix) {
   bbq_ctx* c = ix->ctx;
   TRY(c->cacc.reserve(sizeof(double)));
@@ -413,7 +422,54 @@ static int finish_centroid(bbq_index* ix) {
   return BBQ_OK;
 }
 
-// rows: host (is_host) or device pointer.  Processes chunk by chunk through the transposed scratch.
+// Rows [off, off + rows_here) of `rows` (host when is_host, else device; row-major) into the transposed scratch T
+// (leading dimension R), normalised for COSINE.  A host chunk goes through `stage`: the context's stream orders the
+// next chunk's copy behind this chunk's kernels.
+static int stage_chunk(bbq_ctx* c, const float* rows, bool is_host, uint32_t dim, int64_t R, int64_t off,
+                       int64_t rows_here) {
+  TRY(c->T.reserve((size_t)R * dim * sizeof(float)));
+  const float* src = rows + off * (int64_t)dim;
+  if (is_host) {
+    TRY(c->stage.reserve((size_t)R * dim * sizeof(float)));
+    CU(cudaMemcpyAsync(c->stage.p, src, (size_t)rows_here * dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    src = c->stage.as<float>();
+  }
+  dim3 grid((unsigned)((rows_here + 31) / 32), (dim + 31) / 32), block(32, 8);
+  LAUNCH(c, k_transpose, grid, block, 0, c->stream, src, rows_here, (int)dim, c->T.as<float>(), R);
+  if (c->cfg.similarity == BBQ_SIM_COSINE)
+    LAUNCH(c, k_normalize_T, (unsigned)((rows_here + 127) / 128), 128, 0, c->stream, c->T.as<float>(), R, rows_here,
+           (int)dim, 1);
+  return BBQ_OK;
+}
+
+// quantise rows [0, n) of `rows` into index rows [ix->n, ix->n + n) with the index's centroid
+static int append_impl(bbq_index* ix, const float* rows, bool is_host, uint64_t n) {
+  if (!ix) return fail(BBQ_ERR_NULL, "null index");
+  if (!rows) return fail(BBQ_ERR_NULL, "rows is null");
+  if (ix->n + n > ix->capacity) return fail(BBQ_ERR_INVALID_ARG, "append exceeds the reserved capacity");
+  bbq_ctx* c = ix->ctx;
+  CU(cudaSetDevice(c->device));
+  const int64_t R = (int64_t)std::min<uint64_t>(std::max<uint64_t>(n, 1), BUILD_CHUNK);
+  for (int64_t off = 0; off < (int64_t)n; off += R) {
+    const int64_t rows_here = std::min<int64_t>(R, (int64_t)n - off);
+    TRY(stage_chunk(c, rows, is_host, ix->dim, R, off, rows_here));
+    const unsigned grid = (unsigned)((rows_here + 127) / 128);
+    if (ix->ib == 1)
+      LAUNCH(c, k_osq_index<1>, grid, 128, 0, c->stream, c->T.as<float>(), R, rows_here, (int)ix->dim, ix->centroid,
+             (int)c->cfg.similarity, c->cfg.lambda, (int)c->cfg.iters, ix->codes, ix->row_bytes, (int64_t)ix->n + off,
+             ix->lower, ix->upper, ix->addc, ix->compsum);
+    else
+      LAUNCH(c, k_osq_index<2>, grid, 128, 0, c->stream, c->T.as<float>(), R, rows_here, (int)ix->dim, ix->centroid,
+             (int)c->cfg.similarity, c->cfg.lambda, (int)c->cfg.iters, ix->codes, ix->row_bytes, (int64_t)ix->n + off,
+             ix->lower, ix->upper, ix->addc, ix->compsum);
+  }
+  CU(cudaStreamSynchronize(c->stream));
+  ix->n += n;
+  return BBQ_OK;
+}
+
+// rows: host (is_host) or device pointer.  The centroid (unless given) from one pass over the rows, then the rows are
+// appended to an index reserved for all of them.
 static int build_impl(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, uint32_t dim, const float* centroid,
                       bbq_index** out_index) {
   if (!c || !out_index) return fail(BBQ_ERR_NULL, "null ctx/out_index");
@@ -427,81 +483,25 @@ static int build_impl(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, u
                 "indexBits > 2: the reference's search cannot run any indexBits != 1 (createDirectPackedBuffer throws); "
                 "this build searches 1-bit indexes (reference behaviour) and 2-bit ones (extension)");
   CU(cudaSetDevice(c->device));
-  bbq_index* ix = nullptr;
-  int st = index_alloc(c, n, dim, &ix);
-  if (st != BBQ_OK) {
-    bbq_index_destroy(ix);
-    return st;
-  }
-  auto bail = [&](int s) {
-    bbq_index_destroy(ix);
-    return s;
-  };
-  const int sim = (int)c->cfg.similarity;
-  const int64_t R = (int64_t)std::min<uint64_t>(n, BUILD_CHUNK);
-  st = c->T.reserve((size_t)R * dim * sizeof(float));
-  if (st != BBQ_OK) return bail(st);
-  if (is_host) {
-    st = c->stage.reserve((size_t)R * dim * sizeof(float));
-    if (st != BBQ_OK) return bail(st);
-  }
-  float* T = c->T.as<float>();
-  auto stage_chunk = [&](int64_t off, int64_t rows_here) -> int {
-    const float* src = rows + off * (int64_t)dim;
-    if (is_host) {
-      CU(cudaMemcpyAsync(c->stage.p, src, (size_t)rows_here * dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-      src = c->stage.as<float>();
-    }
-    dim3 grid((unsigned)((rows_here + 31) / 32), (dim + 31) / 32), block(32, 8);
-    LAUNCH(c, k_transpose, grid, block, 0, c->stream, src, rows_here, (int)dim, T, R);
-    if (sim == BBQ_SIM_COSINE)
-      LAUNCH(c, k_normalize_T, (unsigned)((rows_here + 127) / 128), 128, 0, c->stream, T, R, rows_here, (int)dim, 1);
-    return BBQ_OK;
-  };
+  IndexGuard g;
+  TRY(index_alloc(c, n, dim, &g.ix));
+  bbq_index* ix = g.ix;
+  ix->n = 0;
   if (centroid) {
-    st = [&]() -> int {
-      CU(cudaMemcpyAsync(ix->centroid, centroid, dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-      return BBQ_OK;
-    }();
-    if (st != BBQ_OK) return bail(st);
+    CU(cudaMemcpyAsync(ix->centroid, centroid, dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   } else {
+    const int64_t R = (int64_t)std::min<uint64_t>(n, BUILD_CHUNK);
     for (int64_t off = 0; off < (int64_t)n; off += R) {
       const int64_t rows_here = std::min<int64_t>(R, (int64_t)n - off);
-      st = stage_chunk(off, rows_here);
-      if (st != BBQ_OK) return bail(st);
-      st = [&]() -> int {
-        LAUNCH(c, k_centroid_accum, (dim + 63) / 64, 64, 0, c->stream, T, R, rows_here, (int)dim, ix->centroid,
-               off == 0 ? 1 : 0);
-        return BBQ_OK;
-      }();
-      if (st != BBQ_OK) return bail(st);
+      TRY(stage_chunk(c, rows, is_host, dim, R, off, rows_here));
+      LAUNCH(c, k_centroid_accum, (dim + 63) / 64, 64, 0, c->stream, c->T.as<float>(), R, rows_here, (int)dim,
+             ix->centroid, off == 0 ? 1 : 0);
     }
-    st = [&]() -> int {
-      LAUNCH(c, k_centroid_finish, (dim + 127) / 128, 128, 0, c->stream, ix->centroid, (int)dim, (double)n);
-      return BBQ_OK;
-    }();
-    if (st != BBQ_OK) return bail(st);
+    LAUNCH(c, k_centroid_finish, (dim + 127) / 128, 128, 0, c->stream, ix->centroid, (int)dim, (double)n);
   }
-  for (int64_t off = 0; off < (int64_t)n; off += R) {
-    const int64_t rows_here = std::min<int64_t>(R, (int64_t)n - off);
-    st = stage_chunk(off, rows_here);
-    if (st != BBQ_OK) return bail(st);
-    st = [&]() -> int {
-      if (ix->ib == 1)
-        LAUNCH(c, k_osq_index<1>, (unsigned)((rows_here + 127) / 128), 128, 0, c->stream, T, R, rows_here, (int)dim,
-               ix->centroid, sim, c->cfg.lambda, (int)c->cfg.iters, ix->codes, ix->row_bytes, off, ix->lower, ix->upper,
-               ix->addc, ix->compsum);
-      else
-        LAUNCH(c, k_osq_index<2>, (unsigned)((rows_here + 127) / 128), 128, 0, c->stream, T, R, rows_here, (int)dim,
-               ix->centroid, sim, c->cfg.lambda, (int)c->cfg.iters, ix->codes, ix->row_bytes, off, ix->lower, ix->upper,
-               ix->addc, ix->compsum);
-      return BBQ_OK;
-    }();
-    if (st != BBQ_OK) return bail(st);
-  }
-  st = finish_centroid(ix);
-  if (st != BBQ_OK) return bail(st);
-  *out_index = ix;
+  TRY(finish_centroid(ix));
+  TRY(append_impl(ix, rows, is_host, n));
+  *out_index = g.release();
   return BBQ_OK;
 }
 
@@ -548,45 +548,6 @@ extern "C" int bbq_index_build_device(bbq_ctx* c, const float* d_rows, uint64_t 
   return build_impl(c, d_rows, false, n, dim, centroid, out_index);
 }
 
-// quantise rows [0, n) of `rows` into index rows [row0, row0+n) with the index's centroid
-static int append_impl(bbq_index* ix, const float* rows, bool is_host, uint64_t n) {
-  if (!ix) return fail(BBQ_ERR_NULL, "null index");
-  if (!rows) return fail(BBQ_ERR_NULL, "rows is null");
-  if (ix->n + n > ix->capacity) return fail(BBQ_ERR_INVALID_ARG, "append exceeds the reserved capacity");
-  bbq_ctx* c = ix->ctx;
-  CU(cudaSetDevice(c->device));
-  const uint32_t dim = ix->dim;
-  const int sim = (int)c->cfg.similarity;
-  const int64_t R = (int64_t)std::min<uint64_t>(std::max<uint64_t>(n, 1), BUILD_CHUNK);
-  TRY(c->T.reserve((size_t)R * dim * sizeof(float)));
-  if (is_host) TRY(c->stage.reserve((size_t)R * dim * sizeof(float)));
-  float* T = c->T.as<float>();
-  for (int64_t off = 0; off < (int64_t)n; off += R) {
-    const int64_t rows_here = std::min<int64_t>(R, (int64_t)n - off);
-    const float* src = rows + off * (int64_t)dim;
-    if (is_host) {
-      CU(cudaMemcpyAsync(c->stage.p, src, (size_t)rows_here * dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-      src = c->stage.as<float>();
-    }
-    dim3 grid((unsigned)((rows_here + 31) / 32), (dim + 31) / 32), block(32, 8);
-    LAUNCH(c, k_transpose, grid, block, 0, c->stream, src, rows_here, (int)dim, T, R);
-    if (sim == BBQ_SIM_COSINE)
-      LAUNCH(c, k_normalize_T, (unsigned)((rows_here + 127) / 128), 128, 0, c->stream, T, R, rows_here, (int)dim, 1);
-    if (ix->ib == 1)
-      LAUNCH(c, k_osq_index<1>, (unsigned)((rows_here + 127) / 128), 128, 0, c->stream, T, R, rows_here, (int)dim,
-             ix->centroid, sim, c->cfg.lambda, (int)c->cfg.iters, ix->codes, ix->row_bytes, (int64_t)ix->n + off,
-             ix->lower, ix->upper, ix->addc, ix->compsum);
-    else
-      LAUNCH(c, k_osq_index<2>, (unsigned)((rows_here + 127) / 128), 128, 0, c->stream, T, R, rows_here, (int)dim,
-             ix->centroid, sim, c->cfg.lambda, (int)c->cfg.iters, ix->codes, ix->row_bytes, (int64_t)ix->n + off,
-             ix->lower, ix->upper, ix->addc, ix->compsum);
-    if (is_host) CU(cudaStreamSynchronize(c->stream));  // the staging buffer is reused by the next chunk
-  }
-  CU(cudaStreamSynchronize(c->stream));
-  ix->n += n;
-  return BBQ_OK;
-}
-
 extern "C" int bbq_index_reserve(bbq_ctx* c, uint64_t capacity, uint32_t dim, const float* centroid,
                                  bbq_index** out_index) {
   if (!c || !out_index) return fail(BBQ_ERR_NULL, "null ctx/out_index");
@@ -597,20 +558,12 @@ extern "C" int bbq_index_reserve(bbq_ctx* c, uint64_t capacity, uint32_t dim, co
   if (capacity > 0x7FFFFFF0ull) return fail(BBQ_ERR_UNSUPPORTED, "more than 2^31 rows per shard");
   if (c->cfg.index_bits > INDEX_BITS_MAX) return fail(BBQ_ERR_UNSUPPORTED, "indexBits > 2 is not built on device");
   CU(cudaSetDevice(c->device));
-  bbq_index* ix = nullptr;
-  int st = index_alloc(c, capacity, dim, &ix);
-  if (st == BBQ_OK) {
-    ix->n = 0;
-    st = [&]() -> int {
-      CU(cudaMemcpy(ix->centroid, centroid, dim * sizeof(float), cudaMemcpyHostToDevice));
-      return finish_centroid(ix);
-    }();
-  }
-  if (st != BBQ_OK) {
-    bbq_index_destroy(ix);
-    return st;
-  }
-  *out_index = ix;
+  IndexGuard g;
+  TRY(index_alloc(c, capacity, dim, &g.ix));
+  g.ix->n = 0;
+  CU(cudaMemcpy(g.ix->centroid, centroid, dim * sizeof(float), cudaMemcpyHostToDevice));
+  TRY(finish_centroid(g.ix));
+  *out_index = g.release();
   return BBQ_OK;
 }
 extern "C" int bbq_index_append(bbq_index* ix, const float* rows, uint64_t n) {
@@ -666,12 +619,9 @@ extern "C" int bbq_index_from_quantized(bbq_ctx* c, const uint8_t* packed, const
   if (dim == 0) return fail(BBQ_ERR_INVALID_ARG, "dim must be > 0");
   if (c->cfg.index_bits > INDEX_BITS_MAX) return fail(BBQ_ERR_UNSUPPORTED, "only 1- and 2-bit indexes can be adopted");
   CU(cudaSetDevice(c->device));
-  bbq_index* ix = nullptr;
-  int st = index_alloc(c, n, dim, &ix);
-  if (st != BBQ_OK) {
-    bbq_index_destroy(ix);
-    return st;
-  }
+  IndexGuard g;
+  TRY(index_alloc(c, n, dim, &g.ix));
+  bbq_index* ix = g.ix;
   const size_t P = caller_row_bytes(dim, ix->ib);
   const int RB = ix->row_bytes;
   std::vector<uint8_t> codes((size_t)n * RB, 0);
@@ -684,20 +634,14 @@ extern "C" int bbq_index_from_quantized(bbq_ctx* c, const uint8_t* packed, const
     ad[i] = corr4[4 * i + 2];
     cs[i] = (uint32_t)corr4[4 * i + 3];
   }
-  st = [&]() -> int {
-    CU(cudaMemcpy(ix->codes, codes.data(), codes.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(ix->lower, lo.data(), n * sizeof(double), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(ix->upper, up.data(), n * sizeof(double), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(ix->addc, ad.data(), n * sizeof(double), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(ix->compsum, cs.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(ix->centroid, centroid, dim * sizeof(float), cudaMemcpyHostToDevice));
-    return finish_centroid(ix);
-  }();
-  if (st != BBQ_OK) {
-    bbq_index_destroy(ix);
-    return st;
-  }
-  *out_index = ix;
+  CU(cudaMemcpy(ix->codes, codes.data(), codes.size(), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(ix->lower, lo.data(), n * sizeof(double), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(ix->upper, up.data(), n * sizeof(double), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(ix->addc, ad.data(), n * sizeof(double), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(ix->compsum, cs.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(ix->centroid, centroid, dim * sizeof(float), cudaMemcpyHostToDevice));
+  TRY(finish_centroid(ix));
+  *out_index = g.release();
   return BBQ_OK;
 }
 
@@ -1090,33 +1034,44 @@ static ScanParams base_scan_params(bbq_index* ix, int nq) {
   return p;
 }
 
-// Hierarchical deterministic merge of `lists` lists [lists][nq][k] held in (idx_a, score_a) into out.
-static int merge_lists(bbq_ctx* c, int32_t* idx_a, float* score_a, int32_t* idx_b, float* score_b, uint32_t lists,
-                       int nq, uint32_t k, int32_t* out_idx, float* out_score, cudaStream_t st) {
+// Deterministic merge of `lists` per-query lists [lists][nq][k] into out_idx / out_score [nq][k], in groups of
+// max(2, SELECT_MAX / k) lists per selection.  The input is read in place: idx/score pairs, or 64-bit keys when in_keys
+// is set.  The levels in between are keys, alternating between lists_a and lists_b (the first in the one that does not
+// hold the input).  A key carries exactly what its pair carries, so the result does not depend on the form.
+static int merge_topk(bbq_ctx* c, const int32_t* in_idx, const float* in_score, const uint64_t* in_keys, uint32_t lists,
+                      int nq, uint32_t k, int32_t* out_idx, float* out_score, cudaStream_t st) {
   const uint32_t group = std::max<uint32_t>(2u, (uint32_t)SELECT_MAX / k);
+  const size_t cnt = (size_t)nq * k;
+  const void* in = in_keys ? (const void*)in_keys : (const void*)in_idx;
+  DevBuf* dst = in == c->lists_a.p ? &c->lists_b : &c->lists_a;
   while (true) {
     const uint32_t ngroups = (lists + group - 1) / group;
+    if (ngroups > 1) TRY(dst->reserve((size_t)ngroups * cnt * sizeof(uint64_t)));
     for (uint32_t g = 0; g < ngroups; g++) {
-      const uint32_t l0 = g * group, ln = std::min(group, lists - l0);
       SelectParams s{};
       s.nq = nq;
       s.k = k;
-      s.in_idx = idx_a + (size_t)l0 * nq * k;
-      s.in_score = score_a + (size_t)l0 * nq * k;
-      s.lists = ln;
+      s.lists = std::min(group, lists - g * group);
       s.k_in = k;
+      const size_t off = (size_t)g * group * cnt;
       if (ngroups == 1) {
         s.out_idx = out_idx;
         s.out_score = out_score;
       } else {
-        s.out_idx = idx_b + (size_t)g * nq * k;
-        s.out_score = score_b + (size_t)g * nq * k;
+        s.out_keys = dst->as<uint64_t>() + (size_t)g * cnt;
       }
-      TRY(launch_select<SEL_PAIRS>(c, s, ln * k, st));
+      if (in_keys) {
+        s.keys = in_keys + off;
+        TRY(launch_select<SEL_KLISTS>(c, s, s.lists * k, st));
+      } else {
+        s.in_idx = in_idx + off;
+        s.in_score = in_score + off;
+        TRY(launch_select<SEL_PAIRS>(c, s, s.lists * k, st));
+      }
     }
     if (ngroups == 1) return BBQ_OK;
-    std::swap(idx_a, idx_b);
-    std::swap(score_a, score_b);
+    in_keys = dst->as<uint64_t>();
+    dst = dst == &c->lists_a ? &c->lists_b : &c->lists_a;
     lists = ngroups;
   }
 }
@@ -1131,14 +1086,9 @@ static int search_exact_chunked(bbq_index* ix, int nq, uint32_t k, int32_t* d_ou
   const int64_t ntiles = (n + TILE_ROWS - 1) / TILE_ROWS;
   const uint32_t nchunks = (uint32_t)((n + chunk_rows - 1) / chunk_rows);
   TRY(c->dump.reserve((size_t)nq * chunk_rows * sizeof(float)));
-  if (nchunks > 1) {
-    TRY(c->lists_a.reserve((size_t)nchunks * nq * k * (sizeof(int32_t) + sizeof(float))));
-    TRY(c->lists_b.reserve((size_t)nchunks * nq * k * (sizeof(int32_t) + sizeof(float))));
-  }
+  if (nchunks > 1) TRY(c->lists_a.reserve((size_t)nchunks * nq * k * (sizeof(int32_t) + sizeof(float))));
   int32_t* la_idx = c->lists_a.as<int32_t>();
   float* la_score = reinterpret_cast<float*>(la_idx + (size_t)nchunks * nq * k);
-  int32_t* lb_idx = c->lists_b.as<int32_t>();
-  float* lb_score = reinterpret_cast<float*>(lb_idx + (size_t)nchunks * nq * k);
   for (uint32_t ch = 0; ch < nchunks; ch++) {
     const int64_t t0 = (int64_t)ch * chunk_tiles, tn = std::min(chunk_tiles, ntiles - t0);
     const int64_t rows_here = std::min(chunk_rows, n - t0 * TILE_ROWS);
@@ -1165,7 +1115,7 @@ static int search_exact_chunked(bbq_index* ix, int nq, uint32_t k, int32_t* d_ou
     }
     TRY(launch_select<SEL_DENSE>(c, s, (uint32_t)rows_here, st));
   }
-  if (nchunks > 1) TRY(merge_lists(c, la_idx, la_score, lb_idx, lb_score, nchunks, nq, k, d_out_idx, d_out_score, st));
+  if (nchunks > 1) TRY(merge_topk(c, la_idx, la_score, nullptr, nchunks, nq, k, d_out_idx, d_out_score, st));
   return BBQ_OK;
 }
 
@@ -1325,33 +1275,60 @@ extern "C" int bbq_search_device(bbq_index* ix, const float* d_queries, uint32_t
   return BBQ_OK;
 }
 
-// Query screening on the device: arm (the K4 launches that follow screen the batch while they stage it, see
-// osq_query_team) -> [search] -> finish (disarm; D2H of the verdict into the pinned flag block) -> the caller's stream
-// synchronisation -> report.
-static int enqueue_query_validation(bbq_ctx* c, const float* d_queries, cudaStream_t st) {
-  TRY(c->bad.reserve(sizeof(unsigned long long)));
-  CU(cudaMemsetAsync(c->bad.p, 0xFF, sizeof(unsigned long long), st));
-  c->validate_base = d_queries;
-  return BBQ_OK;
-}
-struct ValidationScope {  // an entry point that fails half-way must not leave the screening armed for the next call
+// Query screening on the device (NaN / Infinity): while a QueryScreen is alive, the K4 launches that follow screen the
+// batch that starts at d_queries while they stage it (see osq_query_team) and zero an offending query in place.
+// read_back enqueues the copy of the verdict into the pinned flag block; verdict() reads it after the caller's
+// synchronisation.  Leaving the scope disarms: an entry point that fails half-way leaves nothing armed for the next.
+struct QueryScreen {
   bbq_ctx* c;
-  explicit ValidationScope(bbq_ctx* c_) : c(c_) {}
-  ~ValidationScope() { c->validate_base = nullptr; }
+  int armed;  // status of arming: returned by the caller before any device work
+  QueryScreen(bbq_ctx* c_, const float* d_queries, cudaStream_t st) : c(c_), armed(arm(d_queries, st)) {}
+  ~QueryScreen() { c->validate_base = nullptr; }
+  int read_back(cudaStream_t st) {
+    c->validate_base = nullptr;
+    CU(cudaMemcpyAsync(c->h_flag + QUERY_BATCH + 2, c->bad.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    return BBQ_OK;
+  }
+  static int verdict(bbq_ctx* c) {
+    unsigned long long v;
+    memcpy(&v, c->h_flag + QUERY_BATCH + 2, sizeof v);
+    if (v == ~0ull) return BBQ_OK;
+    const int64_t q = (int64_t)(v >> 34), pos = (int64_t)(v & 0xFFFFFFFFull);
+    if (((v >> 32) & 3ull) == 2ull) return fail(BBQ_ERR_INF, "vector contains Infinity", q, pos);
+    return fail(BBQ_ERR_NAN, "vector contains NaN", q, pos);
+  }
+
+ private:
+  int arm(const float* d_queries, cudaStream_t st) {
+    TRY(c->bad.reserve(sizeof(unsigned long long)));
+    CU(cudaMemsetAsync(c->bad.p, 0xFF, sizeof(unsigned long long), st));
+    c->validate_base = d_queries;
+    return BBQ_OK;
+  }
 };
-static int finish_query_validation(bbq_ctx* c, cudaStream_t st, bool sync) {
-  c->validate_base = nullptr;
-  CU(cudaMemcpyAsync(c->h_flag + QUERY_BATCH + 2, c->bad.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-  if (sync) CU(cudaStreamSynchronize(st));
+
+// the nq host queries of a host-pointer call into qrows, on the context's stream
+static int stage_queries(bbq_ctx* c, const float* queries, uint64_t nq, uint32_t dim) {
+  TRY(c->qrows.reserve((size_t)nq * dim * sizeof(float)));
+  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   return BBQ_OK;
 }
-static int report_query_validation(bbq_ctx* c) {
-  unsigned long long v;
-  memcpy(&v, c->h_flag + QUERY_BATCH + 2, sizeof v);
-  if (v == ~0ull) return BBQ_OK;
-  const int64_t q = (int64_t)(v >> 34), pos = (int64_t)(v & 0xFFFFFFFFull);
-  if (((v >> 32) & 3ull) == 2ull) return fail(BBQ_ERR_INF, "vector contains Infinity", q, pos);
-  return fail(BBQ_ERR_NAN, "vector contains NaN", q, pos);
+
+// nq device rows of kk elements (stride kk) into the caller's host rows of stride k
+static int copy_rows_out(void* dst, size_t k, const DevBuf& src, uint32_t kk, uint32_t nq, size_t elem, cudaStream_t st) {
+  if (kk == k)
+    CU(cudaMemcpyAsync(dst, src.p, (size_t)nq * kk * elem, cudaMemcpyDeviceToHost, st));
+  else
+    CU(cudaMemcpy2DAsync(dst, k * elem, src.p, (size_t)kk * elem, (size_t)kk * elem, nq, cudaMemcpyDeviceToHost, st));
+  return BBQ_OK;
+}
+
+// the lists of a host-pointer search (out_idx / out_score) into the caller's rows, then the call's synchronisation
+static int copy_results(bbq_ctx* c, uint32_t nq, size_t k, uint32_t kk, int32_t* out_idx, float* out_score) {
+  TRY(copy_rows_out(out_idx, k, c->out_idx, kk, nq, sizeof(int32_t), c->stream));
+  TRY(copy_rows_out(out_score, k, c->out_score, kk, nq, sizeof(float), c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return BBQ_OK;
 }
 
 extern "C" int bbq_search(bbq_index* ix, const float* queries, uint32_t nq, int64_t k, int32_t* out_idx,
@@ -1367,23 +1344,22 @@ extern "C" int bbq_search(bbq_index* ix, const float* queries, uint32_t nq, int6
   const uint32_t kk = (uint32_t)std::min<int64_t>(k, (int64_t)ix->n);  // :385 k2 = min(k, vectorCount)
   if (kk > K_MAX) return fail(BBQ_ERR_UNSUPPORTED, "k > 4096 is not supported by the device top-k");
   CU(cudaSetDevice(c->device));
-  TRY(c->qrows.reserve((size_t)nq * ix->dim * sizeof(float)));
   TRY(c->out_idx.reserve((size_t)nq * kk * sizeof(int32_t)));
   TRY(c->out_score.reserve((size_t)nq * kk * sizeof(float)));
-  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * ix->dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  TRY(stage_queries(c, queries, nq, ix->dim));
   // scalarQuantize validates the (normalised) query, optimizedScalarQuantizer.ts:138-148: done on the device, ahead
-  // of the search in the same stream (an offending query is zeroed), and read back at the one synchronisation below
-  ValidationScope vscope(c);
+  // of the search in the same stream (an offending query is zeroed), and read back at the one synchronisation below.
   // One host synchronisation per call (a single-batch call; larger ones keep the per-batch check): the overflow flag of
   // the filtered search travels with the results and is looked at after the synchronisation below.
   c->pending_overflow_nq = -1;
   auto enqueue_device_sequence = [&]() -> int {  // everything between the H2D of the queries and the D2H of the results
-    TRY(enqueue_query_validation(c, c->qrows.as<float>(), c->stream));
+    QueryScreen screen(c, c->qrows.as<float>(), c->stream);
+    TRY(screen.armed);
     c->defer_overflow = nq <= QUERY_BATCH;
     const int st_search = bbq_search_device(ix, c->qrows.as<float>(), nq, kk, c->out_idx.as<int32_t>(), c->out_score.as<float>(), c->stream);
     c->defer_overflow = false;
     TRY(st_search);
-    return finish_query_validation(c, c->stream, /*sync=*/false);
+    return screen.read_back(c->stream);
   };
   const bool graph_ok = c->graph_max_nq > 0 && nq <= (uint32_t)c->graph_max_nq && !c->profiling && c->mma_debug == 0;
   bbq_ctx::SearchGraphKey key;
@@ -1414,7 +1390,6 @@ extern "C" int bbq_search(bbq_index* ix, const float* queries, uint32_t nq, int6
     if (st_seq != BBQ_OK || ec != cudaSuccess || graph == nullptr || g_scratch_gen != key.scratch_gen) {
       if (graph) cudaGraphDestroy(graph);
       cudaGetLastError();
-      c->validate_base = nullptr;
       sg.seen = bbq_ctx::SearchGraphKey{};  // do not try again until the key has been seen twice more
       if (st_seq != BBQ_OK) return st_seq;
       c->pending_overflow_nq = -1;
@@ -1438,21 +1413,7 @@ extern "C" int bbq_search(bbq_index* ix, const float* queries, uint32_t nq, int6
     if (graph_ok) sg.seen = key;  // (if scratch grows during this call the next call's key differs and re-arms)
     TRY(enqueue_device_sequence());
   }
-  // results are written with stride kk; the caller's rows have stride k
-  auto copy_results = [&]() -> int {
-    if ((int64_t)kk == k) {
-      CU(cudaMemcpyAsync(out_idx, c->out_idx.p, (size_t)nq * kk * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-      CU(cudaMemcpyAsync(out_score, c->out_score.p, (size_t)nq * kk * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    } else {
-      CU(cudaMemcpy2DAsync(out_idx, (size_t)k * sizeof(int32_t), c->out_idx.p, (size_t)kk * sizeof(int32_t),
-                           (size_t)kk * sizeof(int32_t), nq, cudaMemcpyDeviceToHost, c->stream));
-      CU(cudaMemcpy2DAsync(out_score, (size_t)k * sizeof(float), c->out_score.p, (size_t)kk * sizeof(float),
-                           (size_t)kk * sizeof(float), nq, cudaMemcpyDeviceToHost, c->stream));
-    }
-    CU(cudaStreamSynchronize(c->stream));
-    return BBQ_OK;
-  };
-  TRY(copy_results());
+  TRY(copy_results(c, nq, (size_t)k, kk, out_idx, out_score));
   if (c->pending_overflow_nq >= 0) {
     const bool over = resolve_filtered(c, c->pending_overflow_nq);
     c->pending_overflow_nq = -1;
@@ -1460,10 +1421,10 @@ extern "C" int bbq_search(bbq_index* ix, const float* queries, uint32_t nq, int6
       c->stats.last_overflow = 1;
       c->stats.last_path = 2;
       TRY(search_exact_chunked(ix, (int)nq, kk, c->out_idx.as<int32_t>(), c->out_score.as<float>(), c->stream));
-      TRY(copy_results());
+      TRY(copy_results(c, nq, (size_t)k, kk, out_idx, out_score));
     }
   }
-  TRY(report_query_validation(c));
+  TRY(QueryScreen::verdict(c));
   if (out_count) *out_count = kk;
   return BBQ_OK;
 }
@@ -1532,19 +1493,11 @@ static int rerank_select_and_copy(bbq_ctx* c, cudaStream_t st, uint32_t nq, uint
     LAUNCH(c, k_rerank_select, nq, 256, 0, st, c->rr_true.as<double>(), c->out_idx.as<int32_t>(), c->out_score.as<float>(),
            (int)m, kk, c->rr_idx.as<int32_t>(), c->rr_q.as<float>(), c->rr_t.as<double>());
   }
-  auto copy_out = [&](void* dst, const void* src, size_t elem) -> int {
-    if (kk == k) {
-      CU(cudaMemcpyAsync(dst, src, (size_t)nq * kk * elem, cudaMemcpyDeviceToHost, st));
-    } else {
-      CU(cudaMemcpy2DAsync(dst, (size_t)k * elem, src, (size_t)kk * elem, (size_t)kk * elem, nq, cudaMemcpyDeviceToHost, st));
-    }
-    return BBQ_OK;
-  };
-  TRY(copy_out(out_idx, c->rr_idx.p, sizeof(int32_t)));
-  TRY(copy_out(out_qscore, c->rr_q.p, sizeof(float)));
-  TRY(copy_out(out_true, c->rr_t.p, sizeof(double)));
+  TRY(copy_rows_out(out_idx, k, c->rr_idx, kk, nq, sizeof(int32_t), st));
+  TRY(copy_rows_out(out_qscore, k, c->rr_q, kk, nq, sizeof(float), st));
+  TRY(copy_rows_out(out_true, k, c->rr_t, kk, nq, sizeof(double), st));
   CU(cudaStreamSynchronize(st));
-  return report_query_validation(c);
+  return QueryScreen::verdict(c);
 }
 
 extern "C" int bbq_search_rerank(bbq_index* ix, const float* queries, uint32_t nq, uint32_t k, uint32_t factor,
@@ -1562,11 +1515,13 @@ extern "C" int bbq_search_rerank(bbq_index* ix, const float* queries, uint32_t n
   CU(cudaSetDevice(c->device));
   cudaStream_t st = c->stream;
   TRY(reserve_rerank(c, ix->dim, nq, m, kk));
-  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * ix->dim * sizeof(float), cudaMemcpyHostToDevice, st));
-  ValidationScope vscope(c);
-  TRY(enqueue_query_validation(c, c->qrows.as<float>(), st));
-  TRY(bbq_search_device(ix, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(), c->out_score.as<float>(), st));
-  TRY(finish_query_validation(c, st, /*sync=*/false));
+  TRY(stage_queries(c, queries, nq, ix->dim));
+  {
+    QueryScreen screen(c, c->qrows.as<float>(), st);
+    TRY(screen.armed);
+    TRY(bbq_search_device(ix, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(), c->out_score.as<float>(), st));
+    TRY(screen.read_back(st));
+  }
   {
     ProfScope prof(c, st, PROF_SELECT);
     TRY(launch_rerank_scores(ix, /*owned_only=*/false, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(),
@@ -1584,30 +1539,7 @@ extern "C" int bbq_merge_topk_device(bbq_ctx* c, const int32_t* d_idx, const flo
   if (k > K_MAX) return fail(BBQ_ERR_UNSUPPORTED, "k > 4096");
   CU(cudaSetDevice(c->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
-  const uint32_t group = std::max<uint32_t>(2u, (uint32_t)SELECT_MAX / k);
-  if (lists <= group) {
-    SelectParams s{};
-    s.nq = (int)nq;
-    s.k = k;
-    s.in_idx = d_idx;
-    s.in_score = d_score;
-    s.lists = lists;
-    s.k_in = k;
-    s.out_idx = d_out_idx;
-    s.out_score = d_out_score;
-    return launch_select<SEL_PAIRS>(c, s, lists * k, st);
-  }
-  // many shards: copy into scratch and merge hierarchically
-  const size_t cnt = (size_t)lists * nq * k;
-  TRY(c->lists_a.reserve(cnt * (sizeof(int32_t) + sizeof(float))));
-  TRY(c->lists_b.reserve(cnt * (sizeof(int32_t) + sizeof(float))));
-  int32_t* la_idx = c->lists_a.as<int32_t>();
-  float* la_score = reinterpret_cast<float*>(la_idx + cnt);
-  int32_t* lb_idx = c->lists_b.as<int32_t>();
-  float* lb_score = reinterpret_cast<float*>(lb_idx + cnt);
-  CU(cudaMemcpyAsync(la_idx, d_idx, cnt * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
-  CU(cudaMemcpyAsync(la_score, d_score, cnt * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  return merge_lists(c, la_idx, la_score, lb_idx, lb_score, lists, (int)nq, k, d_out_idx, d_out_score, st);
+  return merge_topk(c, d_idx, d_score, nullptr, lists, (int)nq, k, d_out_idx, d_out_score, st);
 }
 
 
@@ -1776,36 +1708,8 @@ extern "C" int bbq_search_sharded_device(bbq_index* ix, const float* d_queries, 
   }
   NC(nccl_api()->AllGather(c->keys_local.p, c->keys_all.p, cnt, ncclUint64, c->comm, st));
   // merge: every rank selects the k best of world * k keys per query (identical result on every rank)
-  uint32_t lists = (uint32_t)c->world;
-  uint64_t* src = c->keys_all.as<uint64_t>();
-  const uint32_t group = std::max<uint32_t>(2u, (uint32_t)SELECT_MAX / k);
-  while (lists > group) {  // only for k * world > 16384: reduce groups of lists into keys_local-sized partials
-    const uint32_t ngroups = (lists + group - 1) / group;
-    TRY(c->lists_a.reserve((size_t)ngroups * cnt * sizeof(uint64_t)));
-    TRY(c->lists_b.reserve((size_t)ngroups * cnt * sizeof(uint64_t)));
-    uint64_t* dst = (src == c->lists_a.as<uint64_t>()) ? c->lists_b.as<uint64_t>() : c->lists_a.as<uint64_t>();
-    for (uint32_t g = 0; g < ngroups; g++) {
-      SelectParams s{};
-      s.nq = (int)nq;
-      s.k = k;
-      s.keys = src + (size_t)g * group * cnt;
-      s.lists = std::min(group, lists - g * group);
-      s.k_in = k;
-      s.out_keys = dst + (size_t)g * cnt;
-      TRY(launch_select<SEL_KLISTS>(c, s, s.lists * k, st));
-    }
-    src = dst;
-    lists = ngroups;
-  }
-  SelectParams s{};
-  s.nq = (int)nq;
-  s.k = k;
-  s.keys = src;
-  s.lists = lists;
-  s.k_in = k;
-  s.out_idx = d_out_idx;
-  s.out_score = d_out_score;
-  return launch_select<SEL_KLISTS>(c, s, lists * k, st);
+  return merge_topk(c, nullptr, nullptr, c->keys_all.as<uint64_t>(), (uint32_t)c->world, (int)nq, k, d_out_idx,
+                    d_out_score, st);
 }
 
 extern "C" int bbq_search_sharded(bbq_index* ix, const float* queries, uint32_t nq, int64_t k, int32_t* out_idx,
@@ -1823,26 +1727,18 @@ extern "C" int bbq_search_sharded(bbq_index* ix, const float* queries, uint32_t 
   TRY(global_rows(ix, c->stream, &n_all));
   const uint32_t kk = (uint32_t)std::min<int64_t>(k, (int64_t)std::min<uint64_t>(n_all, 0x7FFFFFFFull));
   if (kk > K_MAX) return fail(BBQ_ERR_UNSUPPORTED, "k > 4096 is not supported by the device top-k");
-  TRY(c->qrows.reserve((size_t)nq * ix->dim * sizeof(float)));
   TRY(c->out_idx.reserve((size_t)nq * kk * sizeof(int32_t)));
   TRY(c->out_score.reserve((size_t)nq * kk * sizeof(float)));
-  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * ix->dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-  ValidationScope vscope(c);
-  TRY(enqueue_query_validation(c, c->qrows.as<float>(), c->stream));
-  TRY(bbq_search_sharded_device(ix, c->qrows.as<float>(), nq, kk, c->out_idx.as<int32_t>(), c->out_score.as<float>(),
-                                c->stream));
-  TRY(finish_query_validation(c, c->stream, /*sync=*/false));
-  if ((int64_t)kk == k) {
-    CU(cudaMemcpyAsync(out_idx, c->out_idx.p, (size_t)nq * kk * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(out_score, c->out_score.p, (size_t)nq * kk * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-  } else {
-    CU(cudaMemcpy2DAsync(out_idx, (size_t)k * sizeof(int32_t), c->out_idx.p, (size_t)kk * sizeof(int32_t),
-                         (size_t)kk * sizeof(int32_t), nq, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpy2DAsync(out_score, (size_t)k * sizeof(float), c->out_score.p, (size_t)kk * sizeof(float),
-                         (size_t)kk * sizeof(float), nq, cudaMemcpyDeviceToHost, c->stream));
+  TRY(stage_queries(c, queries, nq, ix->dim));
+  {
+    QueryScreen screen(c, c->qrows.as<float>(), c->stream);
+    TRY(screen.armed);
+    TRY(bbq_search_sharded_device(ix, c->qrows.as<float>(), nq, kk, c->out_idx.as<int32_t>(), c->out_score.as<float>(),
+                                  c->stream));
+    TRY(screen.read_back(c->stream));
   }
-  CU(cudaStreamSynchronize(c->stream));
-  TRY(report_query_validation(c));
+  TRY(copy_results(c, nq, (size_t)k, kk, out_idx, out_score));
+  TRY(QueryScreen::verdict(c));
   if (out_count) *out_count = kk;
   return BBQ_OK;
 }
@@ -1933,11 +1829,13 @@ extern "C" int bbq_search_rerank_sharded(bbq_index* ix, const float* queries, ui
   const uint32_t m = (uint32_t)std::min<uint64_t>(mk, n_global);
   const uint32_t kk = std::min(k, m);
   if (m == 0) return BBQ_OK;
-  CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)nq * ix->dim * sizeof(float), cudaMemcpyHostToDevice, st));
-  ValidationScope vscope(c);
-  TRY(enqueue_query_validation(c, c->qrows.as<float>(), st));
-  TRY(bbq_search_sharded_device(ix, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(), c->out_score.as<float>(), st));
-  TRY(finish_query_validation(c, st, /*sync=*/false));
+  TRY(stage_queries(c, queries, nq, ix->dim));
+  {
+    QueryScreen screen(c, c->qrows.as<float>(), st);
+    TRY(screen.armed);
+    TRY(bbq_search_sharded_device(ix, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(), c->out_score.as<float>(), st));
+    TRY(screen.read_back(st));
+  }
   {
     ProfScope prof(c, st, PROF_SELECT);
     TRY(launch_rerank_scores(ix, /*owned_only=*/true, c->qrows.as<float>(), nq, m, c->out_idx.as<int32_t>(),
@@ -1976,19 +1874,18 @@ extern "C" int bbq_quantize_query(bbq_ctx* c, const float* query, const float* c
   CU(cudaSetDevice(c->device));
   cudaStream_t st = c->stream;
   const int row_bytes = row_bytes_for(dim, std::min<uint32_t>(c->cfg.index_bits, INDEX_BITS_MAX));
-  TRY(c->qrows.reserve((size_t)dim * sizeof(float)));
   TRY(c->cenv.reserve((size_t)dim * sizeof(float)));
-  TRY(c->bad.reserve(sizeof(unsigned long long)));
-  CU(cudaMemcpyAsync(c->qrows.p, query, (size_t)dim * sizeof(float), cudaMemcpyHostToDevice, st));
+  TRY(stage_queries(c, query, 1, dim));
   CU(cudaMemcpyAsync(c->cenv.p, centroid, (size_t)dim * sizeof(float), cudaMemcpyHostToDevice, st));
   const bool cosine = c->cfg.similarity == BBQ_SIM_COSINE;
-  ValidationScope vscope(c);
-  TRY(enqueue_query_validation(c, c->qrows.as<float>(), st));
+  QueryScreen screen(c, c->qrows.as<float>(), st);
+  TRY(screen.armed);
   TRY(quantize_rows(c, c->qrows.as<float>(), 1, (int)dim, row_bytes, c->cenv.as<float>(), cosine ? 1 : 0, st));
   if (codes) CU(cudaMemcpyAsync(codes, c->qcodes.p, dim, cudaMemcpyDeviceToHost, st));
   if (corr4) CU(cudaMemcpyAsync(corr4, c->qcorr.p, 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
-  TRY(finish_query_validation(c, st, /*sync=*/true));
-  return report_query_validation(c);
+  TRY(screen.read_back(st));
+  CU(cudaStreamSynchronize(st));
+  return QueryScreen::verdict(c);
 }
 
 extern "C" int bbq_quantization_accuracy(bbq_ctx* c, const float* rows, const float* queries, uint64_t n, uint32_t dim,
@@ -2001,35 +1898,32 @@ extern "C" int bbq_quantization_accuracy(bbq_ctx* c, const float* rows, const fl
   if (qb != 1 && qb != 4) return fail(BBQ_ERR_UNSUPPORTED, "unsupported query bits: only 1 and 4 (computeQuantizedScore)");
   if (c->cfg.index_bits != 1) return fail(BBQ_ERR_UNSUPPORTED, "computeQuantizationAccuracy scores through the single-vector scorer, which knows 1-bit indexes only");
   if (n > 0x7FFFFFF0ull) return fail(BBQ_ERR_UNSUPPORTED, "too many vectors");
-  bbq_index* ix = nullptr;
-  TRY(bbq_index_build(c, rows, n, dim, nullptr, &ix));   // 1. quantizeVectors(originalVectors), reference-order centroid
+  IndexGuard g;
+  TRY(bbq_index_build(c, rows, n, dim, nullptr, &g.ix));  // 1. quantizeVectors(originalVectors), reference-order centroid
+  bbq_index* ix = g.ix;
   cudaStream_t st = c->stream;
   const bool cosine = c->cfg.similarity == BBQ_SIM_COSINE;
-  int rc = [&]() -> int {
-    TRY(c->qrows.reserve((size_t)n * dim * sizeof(float)));
-    TRY(c->rr_q.reserve((size_t)dim * sizeof(float)));
-    TRY(c->rr_true.reserve((size_t)n * sizeof(double)));
-    TRY(c->rr_t.reserve((size_t)n * sizeof(double)));
-    TRY(c->cacc.reserve(5 * sizeof(double)));
-    CU(cudaMemcpyAsync(c->qrows.p, queries, (size_t)n * dim * sizeof(float), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(c->rr_q.p, rows + target_ord * dim, (size_t)dim * sizeof(float), cudaMemcpyHostToDevice, st));
-    ValidationScope vscope(c);
-    TRY(enqueue_query_validation(c, c->qrows.as<float>(), st));
-    // 2. quantizeQueryVector(query, centroid): ONE normalisation for COSINE (:271-299)
-    TRY(quantize_rows(c, c->qrows.as<float>(), (int)n, (int)dim, ix->row_bytes, ix->centroid, cosine ? 1 : 0, st));
-    LAUNCH(c, k_accuracy_scores, (unsigned)((n + RERANK_WARPS - 1) / RERANK_WARPS), RERANK_WARPS * 32, 0, st,
-           c->qcodes.as<uint8_t>(), ix->row_bytes * 8, c->qcorr.as<double>(), (int)n, qb == 1 ? 1 : 0,
-           ix->codes + target_ord * ix->row_bytes, ix->lower + target_ord, ix->upper + target_ord, ix->addc + target_ord,
-           ix->compsum + target_ord, c->qrows.as<float>(), c->rr_q.as<float>(), (int)dim, (int)c->cfg.similarity,
-           qb == 1 ? ix->cdp : 0.0, c->rr_true.as<double>(), c->rr_t.as<double>());
-    // 3. statistics (sequential sums, one thread: the reference's order)
-    LAUNCH(c, k_accuracy_stats, 1, 32, 0, st, c->rr_true.as<double>(), c->rr_t.as<double>(), (int64_t)n, c->cacc.as<double>());
-    CU(cudaMemcpyAsync(out5, c->cacc.p, 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    TRY(finish_query_validation(c, st, /*sync=*/true));
-    return report_query_validation(c);
-  }();
-  bbq_index_destroy(ix);
-  return rc;
+  TRY(c->rr_q.reserve((size_t)dim * sizeof(float)));
+  TRY(c->rr_true.reserve((size_t)n * sizeof(double)));
+  TRY(c->rr_t.reserve((size_t)n * sizeof(double)));
+  TRY(c->cacc.reserve(5 * sizeof(double)));
+  TRY(stage_queries(c, queries, n, dim));
+  CU(cudaMemcpyAsync(c->rr_q.p, rows + target_ord * dim, (size_t)dim * sizeof(float), cudaMemcpyHostToDevice, st));
+  QueryScreen screen(c, c->qrows.as<float>(), st);
+  TRY(screen.armed);
+  // 2. quantizeQueryVector(query, centroid): ONE normalisation for COSINE (:271-299)
+  TRY(quantize_rows(c, c->qrows.as<float>(), (int)n, (int)dim, ix->row_bytes, ix->centroid, cosine ? 1 : 0, st));
+  LAUNCH(c, k_accuracy_scores, (unsigned)((n + RERANK_WARPS - 1) / RERANK_WARPS), RERANK_WARPS * 32, 0, st,
+         c->qcodes.as<uint8_t>(), ix->row_bytes * 8, c->qcorr.as<double>(), (int)n, qb == 1 ? 1 : 0,
+         ix->codes + target_ord * ix->row_bytes, ix->lower + target_ord, ix->upper + target_ord, ix->addc + target_ord,
+         ix->compsum + target_ord, c->qrows.as<float>(), c->rr_q.as<float>(), (int)dim, (int)c->cfg.similarity,
+         qb == 1 ? ix->cdp : 0.0, c->rr_true.as<double>(), c->rr_t.as<double>());
+  // 3. statistics (sequential sums, one thread: the reference's order)
+  LAUNCH(c, k_accuracy_stats, 1, 32, 0, st, c->rr_true.as<double>(), c->rr_t.as<double>(), (int64_t)n, c->cacc.as<double>());
+  CU(cudaMemcpyAsync(out5, c->cacc.p, 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
+  TRY(screen.read_back(st));
+  CU(cudaStreamSynchronize(st));
+  return QueryScreen::verdict(c);
 }
 
 // ------------------------------------------------------------------------------------------------

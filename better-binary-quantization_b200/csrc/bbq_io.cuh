@@ -250,54 +250,48 @@ extern "C" int bbq_index_load(bbq_ctx* c, const char* veb_path, const char* vemb
   struct stat sb;
   if (fstat(veb.fd, &sb) != 0) return io_fail("cannot stat", veb_path);
 
-  bbq_index* ix = nullptr;
-  int st = index_alloc(c, h.vectorCount, h.dimensions, &ix);
-  if (st == BBQ_OK) st = [&]() -> int {
-    bbqio::Section s[5];
-    io_sections(ix, s);
-    const uint64_t want[5] = {h.vectorDataOffset, h.lowerOffset, h.upperOffset, h.additionalOffset, h.componentSumOffset};
-    for (int i = 0; i < 5; i++)
-      if (want[i] != s[i].offset) return fail(BBQ_ERR_FORMAT, std::string("unexpected offset of section ") + s[i].name);
-    if ((uint64_t)sb.st_size < s[4].offset + s[4].bytes || h.vectorDataLength != s[4].offset + s[4].bytes)
-      return fail(BBQ_ERR_FORMAT, std::string("truncated vector data file '") + veb_path + "'");
-    bbqio::Pinned pin;
-    TRY(io_pinned(pin));
-    bool busy[2] = {false, false};
-    int b = 0;
-    for (int i = 0; i < 5; i++) {
-      uint64_t done = 0;
-      while (done < s[i].bytes) {
-        if (busy[b]) CU(cudaEventSynchronize(pin.ev[b]));  // the copy that last used this buffer has drained
-        const uint64_t len = std::min<uint64_t>(bbqio::STAGE_BYTES, s[i].bytes - done);
-        uint64_t r = 0;
-        while (r < len) {
-          const ssize_t g = pread(veb.fd, (char*)pin.p[b] + r, len - r, (off_t)(s[i].offset + done + r));
-          if (g < 0) return io_fail("read failed on", veb_path);
-          if (g == 0) return fail(BBQ_ERR_FORMAT, std::string("truncated vector data file '") + veb_path + "'");
-          r += (uint64_t)g;
-        }
-        CU(cudaMemcpyAsync((char*)s[i].dev + done, pin.p[b], len, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaEventRecord(pin.ev[b], c->stream));
-        busy[b] = true;
-        done += len;
-        b ^= 1;
+  IndexGuard g;
+  TRY(index_alloc(c, h.vectorCount, h.dimensions, &g.ix));
+  bbq_index* ix = g.ix;
+  bbqio::Section s[5];
+  io_sections(ix, s);
+  const uint64_t want[5] = {h.vectorDataOffset, h.lowerOffset, h.upperOffset, h.additionalOffset, h.componentSumOffset};
+  for (int i = 0; i < 5; i++)
+    if (want[i] != s[i].offset) return fail(BBQ_ERR_FORMAT, std::string("unexpected offset of section ") + s[i].name);
+  if ((uint64_t)sb.st_size < s[4].offset + s[4].bytes || h.vectorDataLength != s[4].offset + s[4].bytes)
+    return fail(BBQ_ERR_FORMAT, std::string("truncated vector data file '") + veb_path + "'");
+  bbqio::Pinned pin;
+  TRY(io_pinned(pin));
+  bool busy[2] = {false, false};
+  int b = 0;
+  for (int i = 0; i < 5; i++) {
+    uint64_t done = 0;
+    while (done < s[i].bytes) {
+      if (busy[b]) CU(cudaEventSynchronize(pin.ev[b]));  // the copy that last used this buffer has drained
+      const uint64_t len = std::min<uint64_t>(bbqio::STAGE_BYTES, s[i].bytes - done);
+      uint64_t r = 0;
+      while (r < len) {
+        const ssize_t got = pread(veb.fd, (char*)pin.p[b] + r, len - r, (off_t)(s[i].offset + done + r));
+        if (got < 0) return io_fail("read failed on", veb_path);
+        if (got == 0) return fail(BBQ_ERR_FORMAT, std::string("truncated vector data file '") + veb_path + "'");
+        r += (uint64_t)got;
       }
+      CU(cudaMemcpyAsync((char*)s[i].dev + done, pin.p[b], len, cudaMemcpyHostToDevice, c->stream));
+      CU(cudaEventRecord(pin.ev[b], c->stream));
+      busy[b] = true;
+      done += len;
+      b ^= 1;
     }
-    CU(cudaMemcpyAsync(ix->centroid, centroid.data(), centroid.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    uint64_t sums[5];
-    TRY(io_checksums(ix, s, sums));
-    for (int i = 0; i < 5; i++)
-      if (sums[i] != h.checksum[i]) return fail(BBQ_ERR_FORMAT, std::string("checksum mismatch in section ") + s[i].name);
-    TRY(finish_centroid(ix));
-    if (memcmp(&ix->cdp, &h.centroidSquareMagnitude, sizeof(double)) != 0)
-      return fail(BBQ_ERR_FORMAT, "centroidSquareMagnitude does not match the stored centroid");
-    return BBQ_OK;
-  }();
-  if (st != BBQ_OK) {
-    bbq_index_destroy(ix);
-    return st;
   }
-  *out_index = ix;
+  CU(cudaMemcpyAsync(ix->centroid, centroid.data(), centroid.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  uint64_t sums[5];
+  TRY(io_checksums(ix, s, sums));
+  for (int i = 0; i < 5; i++)
+    if (sums[i] != h.checksum[i]) return fail(BBQ_ERR_FORMAT, std::string("checksum mismatch in section ") + s[i].name);
+  TRY(finish_centroid(ix));
+  if (memcmp(&ix->cdp, &h.centroidSquareMagnitude, sizeof(double)) != 0)
+    return fail(BBQ_ERR_FORMAT, "centroidSquareMagnitude does not match the stored centroid");
+  *out_index = g.release();
   return BBQ_OK;
 }
