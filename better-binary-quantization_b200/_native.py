@@ -67,6 +67,11 @@ SYMBOLS = {
     "bbq_index_set_base": (C.c_int, [_vp, C.c_uint64]),
     "bbq_index_save": (C.c_int, [_vp, C.c_char_p, C.c_char_p]),
     "bbq_index_load": (C.c_int, [_vp, C.c_char_p, C.c_char_p, C.POINTER(_vp)]),
+    "bbq_index_load_rows": (C.c_int, [_vp, C.c_char_p, C.c_char_p, C.c_uint64, C.c_uint64, C.POINTER(_vp), _vp]),
+    "bbq_index_write_rows": (C.c_int, [_vp, C.c_char_p, C.c_uint64, _vp]),
+    "bbq_index_write_meta": (C.c_int, [_vp, C.c_char_p, C.c_uint64, _vp]),
+    "bbq_index_save_sharded": (C.c_int, [_vp, C.c_char_p, C.c_char_p]),
+    "bbq_index_load_sharded": (C.c_int, [_vp, C.c_char_p, C.c_char_p, C.POINTER(_vp)]),
     "bbq_index_destroy": (None, [_vp]),
     "bbq_search": (C.c_int, [_vp, _vp, C.c_uint32, C.c_int64, _vp, _vp, C.POINTER(C.c_uint32)]),
     "bbq_search_device": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, _vp, _vp, _vp]),

@@ -262,31 +262,37 @@ static int get_path(napi_env env, napi_value v, char* buf, size_t cap) {
 
 /* saveIndex(index, vebPath, vembPath) / loadIndex(ctx, vebPath, vembPath) -> external index
  * the on-disk form of serializeVectorData / deserializeVectorData, src/binaryQuantizationFormat.ts:483-560 */
-static napi_value n_save_index(napi_env env, napi_callback_info info) {
+static napi_value save_common(napi_env env, napi_callback_info info, int sharded) {
   ARGS(3);
   void* ix;
   char veb[4096], vemb[4096];
   napi_get_value_external(env, argv[0], &ix);
   if (!get_path(env, argv[1], veb, sizeof veb) || !get_path(env, argv[2], vemb, sizeof vemb)) return throw_status(env, BBQ_ERR_NULL);
-  const int st = bbq_index_save((bbq_index*)ix, veb, vemb);
+  const int st = sharded ? bbq_index_save_sharded((bbq_index*)ix, veb, vemb) : bbq_index_save((bbq_index*)ix, veb, vemb);
   if (st != BBQ_OK) return throw_status(env, st);
   napi_value u;
   napi_get_undefined(env, &u);
   return u;
 }
-static napi_value n_load_index(napi_env env, napi_callback_info info) {
+static napi_value load_common(napi_env env, napi_callback_info info, int sharded) {
   ARGS(3);
   void* ctx;
   char veb[4096], vemb[4096];
   napi_get_value_external(env, argv[0], &ctx);
   if (!get_path(env, argv[1], veb, sizeof veb) || !get_path(env, argv[2], vemb, sizeof vemb)) return throw_status(env, BBQ_ERR_NULL);
   bbq_index* ix = NULL;
-  const int st = bbq_index_load((bbq_ctx*)ctx, veb, vemb, &ix);
+  const int st = sharded ? bbq_index_load_sharded((bbq_ctx*)ctx, veb, vemb, &ix) : bbq_index_load((bbq_ctx*)ctx, veb, vemb, &ix);
   if (st != BBQ_OK) return throw_status(env, st);
   napi_value out;
   napi_create_external(env, ix, fin_index, NULL, &out);
   return out;
 }
+static napi_value n_save_index(napi_env env, napi_callback_info info) { return save_common(env, info, 0); }
+static napi_value n_load_index(napi_env env, napi_callback_info info) { return load_common(env, info, 0); }
+/* saveIndexSharded(index, vebPath, vembPath) / loadIndexSharded(ctx, vebPath, vembPath) -> external index (this rank's
+ * row range, base set): one image of all row shards of the box (collective; bbq_index_save_sharded / _load_sharded) */
+static napi_value n_save_index_sharded(napi_env env, napi_callback_info info) { return save_common(env, info, 1); }
+static napi_value n_load_index_sharded(napi_env env, napi_callback_info info) { return load_common(env, info, 1); }
 
 /* quantizeQuery(ctx, query Float32Array[dim], centroid Float32Array[dim]) -> {codes: Uint8Array[dim], corrections: Float64Array[4]}
  * replaces format.quantizeQueryVector(queryVector, centroid), src/binaryQuantizationFormat.ts:271-299 */
@@ -417,6 +423,8 @@ NAPI_MODULE_INIT() {
       {"searchRerankSharded", NULL, n_search_rerank_sharded, NULL, NULL, NULL, 0, NULL},
       {"saveIndex", NULL, n_save_index, NULL, NULL, NULL, 0, NULL},
       {"loadIndex", NULL, n_load_index, NULL, NULL, NULL, 0, NULL},
+      {"saveIndexSharded", NULL, n_save_index_sharded, NULL, NULL, NULL, 0, NULL},
+      {"loadIndexSharded", NULL, n_load_index_sharded, NULL, NULL, NULL, 0, NULL},
       {"quantizeQuery", NULL, n_quantize_query, NULL, NULL, NULL, 0, NULL},
       {"accuracy", NULL, n_accuracy, NULL, NULL, NULL, 0, NULL},
       {"fromQuantized", NULL, n_from_quantized, NULL, NULL, NULL, 0, NULL},

@@ -43,6 +43,8 @@ const addon = require('./bbq_b200.node') as {
     { indices: Int32Array; quantizedScores: Float32Array; trueScores: Float64Array; count: number };
   saveIndex(index: Handle, veb: string, vemb: string): void;
   loadIndex(ctx: Handle, veb: string, vemb: string): Handle;
+  saveIndexSharded(index: Handle, veb: string, vemb: string): void;
+  loadIndexSharded(ctx: Handle, veb: string, vemb: string): Handle;
   quantizeQuery(ctx: Handle, query: Float32Array, centroid: Float32Array): { codes: Uint8Array; corrections: Float64Array };
   accuracy(ctx: Handle, rows: Float32Array, queries: Float32Array, n: number, dim: number, targetOrd: number): Float64Array;
   fromQuantized(ctx: Handle, packed: Uint8Array, corrections: Float64Array, centroid: Float32Array, n: number, dim: number): Handle;
@@ -226,12 +228,14 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
 
   /** Sharded search over the GPUs of one box (one Node process per GPU; SURVEY §8e).  Rank 0 creates the id and
    *  ships it to its peers (IPC message / env var / file); every rank then joins and declares its shard's base row.
-   *  After that searchBatch(..., sharded = true) returns, on every rank, the lists of the whole corpus. */
+   *  After that searchBatch(..., sharded = true) returns, on every rank, the lists of the whole corpus.  A rank that is
+   *  about to load its shard with loadIndex(prefix, true) has no shard yet: it joins without one (the load sets the
+   *  base). */
   public static createShardGroupId(): Uint8Array { return addon.commUniqueId(); }
-  public joinShardGroup(id: Uint8Array, rank: number, world: number, shard: BinarizedByteVectorValues, baseRow: number): void {
+  public joinShardGroup(id: Uint8Array, rank: number, world: number, shard?: BinarizedByteVectorValues, baseRow?: number): void {
     try {
       addon.commInit(this.ctx, id, rank, world);
-      addon.setBase(deviceHandle(shard), baseRow);
+      if (shard !== undefined) addon.setBase(deviceHandle(shard), baseRow ?? 0);
     } catch (e) { throw toReferenceError(e, 'build'); }
   }
 
@@ -256,13 +260,21 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
   }
 
   /** On-disk form of serializeVectorData / deserializeVectorData (:483-560): `${prefix}.veb` + `${prefix}.vemb`
-   *  (FILE_EXTENSIONS, src/constants.ts:52-57), streamed between the files and device memory natively. */
-  public saveIndex(targetVectors: BinarizedByteVectorValues, prefix: string): void {
-    try { addon.saveIndex(deviceHandle(targetVectors), `${prefix}.veb`, `${prefix}.vemb`); }
-    catch (e) { throw toReferenceError(e, 'build'); }
+   *  (FILE_EXTENSIONS, src/constants.ts:52-57), streamed between the files and device memory natively.
+   *  With sharded = true (after joinShardGroup) both are collective: every rank saves its own rows into ONE image of
+   *  the whole corpus, or loads its own row range of one image (its base set), on any number of ranks. */
+  public saveIndex(targetVectors: BinarizedByteVectorValues, prefix: string, sharded = false): void {
+    try {
+      const h = deviceHandle(targetVectors);
+      if (sharded) addon.saveIndexSharded(h, `${prefix}.veb`, `${prefix}.vemb`);
+      else addon.saveIndex(h, `${prefix}.veb`, `${prefix}.vemb`);
+    } catch (e) { throw toReferenceError(e, 'build'); }
   }
-  public loadIndex(prefix: string): BinarizedByteVectorValues {
-    try { return new DeviceBinarizedByteVectorValues(addon.loadIndex(this.ctx, `${prefix}.veb`, `${prefix}.vemb`)); }
-    catch (e) { throw toReferenceError(e, 'build'); }
+  public loadIndex(prefix: string, sharded = false): BinarizedByteVectorValues {
+    try {
+      const h = sharded ? addon.loadIndexSharded(this.ctx, `${prefix}.veb`, `${prefix}.vemb`)
+                        : addon.loadIndex(this.ctx, `${prefix}.veb`, `${prefix}.vemb`);
+      return new DeviceBinarizedByteVectorValues(h);
+    } catch (e) { throw toReferenceError(e, 'build'); }
   }
 }

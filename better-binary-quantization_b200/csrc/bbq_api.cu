@@ -690,8 +690,6 @@ extern "C" int bbq_index_export(const bbq_index* ix, uint64_t first, uint64_t co
   return BBQ_OK;
 }
 
-#include "bbq_io.cuh"
-
 // ------------------------------------------------------------------------------------------------
 // search
 // ------------------------------------------------------------------------------------------------
@@ -1848,6 +1846,8 @@ extern "C" int bbq_search_rerank_sharded(bbq_index* ix, const float* queries, ui
   if (out_count) *out_count = kk;
   return BBQ_OK;
 }
+
+#include "bbq_io.cuh"  // index image on disk, whole and across row shards (uses the NCCL plumbing above)
 
 // Page-locked host buffers for hosts that want the H2D / D2H copies of bbq_search* to run at full PCIe speed
 // (a Node host wraps them in external ArrayBuffers; any host pointer works, pageable memory is merely slower).

@@ -231,17 +231,52 @@ class BinaryQuantizationFormat:
         # FILE_EXTENSIONS, src/constants.ts:52-57
         return (os.fsencode(prefix + ".veb"), os.fsencode(prefix + ".vemb"))
 
-    def saveIndex(self, targetVectors: BinarizedByteVectorValues, prefix: str) -> None:
-        """Writes <prefix>.veb (vector data) and <prefix>.vemb (metadata + centroid): bbq_index_save."""
+    def saveIndex(self, targetVectors: BinarizedByteVectorValues, prefix: str, sharded: bool = False) -> None:
+        """Writes <prefix>.veb (vector data) and <prefix>.vemb (metadata + centroid): bbq_index_save.  sharded=True: one
+        image of all row shards of the communicator, each rank writing its own rows (bbq_index_save_sharded,
+        collective); the files equal those of one index holding the whole corpus."""
         veb, vemb = self._image_paths(prefix)
-        _check(_native.load().bbq_index_save(targetVectors._h, veb, vemb), "build")
+        L = _native.load()
+        fn = L.bbq_index_save_sharded if sharded else L.bbq_index_save
+        _check(fn(targetVectors._h, veb, vemb), "build")
 
-    def loadIndex(self, prefix: str) -> BinarizedByteVectorValues:
-        """Reads an image written by saveIndex straight into device memory: bbq_index_load."""
+    def loadIndex(self, prefix: str, sharded: bool = False) -> BinarizedByteVectorValues:
+        """Reads an image written by saveIndex straight into device memory: bbq_index_load.  sharded=True: this rank's
+        row range of the image (shard_bounds), with its base set (bbq_index_load_sharded, collective)."""
         veb, vemb = self._image_paths(prefix)
         h = C.c_void_p()
-        _check(_native.load().bbq_index_load(self._ctx, veb, vemb, C.byref(h)), "build")
+        L = _native.load()
+        fn = L.bbq_index_load_sharded if sharded else L.bbq_index_load
+        _check(fn(self._ctx, veb, vemb, C.byref(h)), "build")
         return BinarizedByteVectorValues(self, h)
+
+    def loadIndexRows(self, prefix: str, first: int, count: int):
+        """Rows [first, first + count) of an image as an index whose base is `first` (bbq_index_load_rows, not
+        collective) -> (index, the five partial section checksums of the rows loaded)."""
+        veb, vemb = self._image_paths(prefix)
+        h = C.c_void_p()
+        part = (C.c_uint64 * 5)()
+        _check(_native.load().bbq_index_load_rows(self._ctx, veb, vemb, first, count, C.byref(h), part), "build")
+        return BinarizedByteVectorValues(self, h), [int(x) for x in part]
+
+    def writeIndexRows(self, shard: BinarizedByteVectorValues, prefix: str, totalRows: int):
+        """This shard's rows at rows [base, base + size) of an image of totalRows rows (bbq_index_write_rows)
+        -> the five partial section checksums of the rows written."""
+        veb, _ = self._image_paths(prefix)
+        part = (C.c_uint64 * 5)()
+        _check(_native.load().bbq_index_write_rows(shard._h, veb, totalRows, part), "build")
+        return [int(x) for x in part]
+
+    def writeIndexMeta(self, shard: BinarizedByteVectorValues, prefix: str, totalRows: int, checksums) -> None:
+        """<prefix>.vemb for an image of totalRows rows whose sections have the given checksums (the sums mod 2^64 of
+        every shard's partials) and this shard's centroid (bbq_index_write_meta)."""
+        _, vemb = self._image_paths(prefix)
+        sums = (C.c_uint64 * 5)(*[int(x) & 0xFFFFFFFFFFFFFFFF for x in checksums])
+        _check(_native.load().bbq_index_write_meta(shard._h, vemb, totalRows, sums), "build")
+
+    def setBase(self, targetVectors: BinarizedByteVectorValues, base: int) -> None:
+        """Global row id of this shard's row 0 (bbq_index_set_base)."""
+        _check(_native.load().bbq_index_set_base(targetVectors._h, base))
 
     # -- query side -------------------------------------------------------------------------------------
     def quantizeQueryVector(self, queryVector, centroid) -> dict:
@@ -322,9 +357,10 @@ class BinaryQuantizationFormat:
         idx, sc = self.searchBatch(q[None, :], targetVectors, k)
         return [{"index": int(i), "score": float(s)} for i, s in zip(idx[0], sc[0])]
 
-    def searchBatch(self, queries, targetVectors: BinarizedByteVectorValues, k: int):
+    def searchBatch(self, queries, targetVectors: BinarizedByteVectorValues, k: int, sharded: bool = False):
         """Additive batched entry (SURVEY §8b): row i == searchNearestNeighbors(queries[i]).
-        -> (idx i32[nq, min(k,n)], score f32[nq, min(k,n)])"""
+        -> (idx i32[nq, min(k,n)], score f32[nq, min(k,n)]).  sharded=True: over all row shards of the communicator
+        (bbq_search_sharded, collective; n = the rows of all shards), the same lists on every rank."""
         if k < 0:
             raise BbqError(7, "k值不能为负数")
         qs = np.ascontiguousarray(queries, np.float32)
@@ -335,9 +371,10 @@ class BinaryQuantizationFormat:
         idx = np.empty((nq, max(k, 1)), np.int32)
         sc = np.empty((nq, max(k, 1)), np.float32)
         cnt = C.c_uint32(0)
-        _check(_native.load().bbq_search(targetVectors._h, qs.ctypes.data, nq, k, idx.ctypes.data, sc.ctypes.data,
-                                         C.byref(cnt)), "search")
-        assert cnt.value == (kk if nq else 0) or k == 0
+        L = _native.load()
+        fn = L.bbq_search_sharded if sharded else L.bbq_search
+        _check(fn(targetVectors._h, qs.ctypes.data, nq, k, idx.ctypes.data, sc.ctypes.data, C.byref(cnt)), "search")
+        assert sharded or cnt.value == (kk if nq else 0) or k == 0
         return idx[:, :cnt.value].copy(), sc[:, :cnt.value].copy()
 
     # -- oversampled search + exact re-rank (src/topKSelector.ts) -------------------------------------------

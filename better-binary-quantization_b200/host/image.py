@@ -41,15 +41,17 @@ def section_layout(vector_count: int, dimensions: int):
     return out
 
 
-def section_checksum(raw) -> int:
-    """sum over 32-bit words of splitmix64(index << 32 | word), mod 2^64 — what k_section_checksum computes."""
+def section_checksum(raw, first_word: int = 0) -> int:
+    """sum over 32-bit words of splitmix64(index << 32 | word), mod 2^64 — what k_section_checksum computes.
+    first_word: the position of raw's first word in its section (rows [r, ...) of a section of stride S bytes start at
+    word r * S / 4), so the checksums of the slices of a section add up, mod 2^64, to the checksum of the section."""
     words = np.frombuffer(memoryview(raw), dtype="<u4").astype(np.uint64)
     total = 0
     step = 1 << 22
     with np.errstate(over="ignore"):
         for s in range(0, words.size, step):
             w = words[s:s + step]
-            z = (np.arange(s, s + w.size, dtype=np.uint64) << np.uint64(32)) | w
+            z = (np.arange(first_word + s, first_word + s + w.size, dtype=np.uint64) << np.uint64(32)) | w
             z = z + np.uint64(0x9E3779B97F4A7C15)
             z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
             z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)

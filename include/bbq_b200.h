@@ -127,6 +127,41 @@ int bbq_index_centroid(const bbq_index* index, float* out_centroid /* dim */, do
 int bbq_index_save(const bbq_index* index, const char* veb_path, const char* vemb_path);
 int bbq_index_load(bbq_ctx* ctx, const char* veb_path, const char* vemb_path, bbq_index** out_index);
 
+/* One image across row shards.  A section's checksum is Σ splitmix64(i << 32 | word_i) over its 32-bit words with i
+ * counted from the image's row 0, so the checksums of disjoint row ranges add up (mod 2^64) to the section's.  The
+ * shard-local primitives below are not collective; out_partial / checksums: {codes, lower, upper, additional,
+ * componentSum}.
+ * bbq_index_load_rows: rows [first, first + count) of an image into a new index whose base (bbq_index_set_base) is
+ *   `first`, reading only that range of each section; the checks of bbq_index_load, plus first + count <= vectorCount
+ *   (else BBQ_ERR_INVALID_ARG).  out_partial (may be NULL) receives the checksums of the rows uploaded; only when the
+ *   range is the whole image are they compared with the header here.  count = 0 gives an index of 0 rows.
+ * bbq_index_write_rows: this shard's rows at rows [base, base + n) of an image of total_rows rows (base + n <=
+ *   total_rows, else BBQ_ERR_INVALID_ARG).  Opens the .veb with O_CREAT and without O_TRUNC and sets its length to the
+ *   image's, so calls may come in any order from any process; start from a new (or truncated) file.
+ * bbq_index_write_meta: the .vemb of an image of total_rows rows with the given checksums (the sums of every shard's
+ *   partials) and this shard's dimension, similarity, centroid and centroidSquareMagnitude.
+ * The files equal, byte for byte, what bbq_index_save writes for one index holding all the rows. */
+int bbq_index_load_rows(bbq_ctx* ctx, const char* veb_path, const char* vemb_path, uint64_t first, uint64_t count,
+                        bbq_index** out_index, uint64_t out_partial[5]);
+int bbq_index_write_rows(const bbq_index* shard, const char* veb_path, uint64_t total_rows, uint64_t out_partial[5]);
+int bbq_index_write_meta(const bbq_index* shard, const char* vemb_path, uint64_t total_rows, const uint64_t checksums[5]);
+
+/* Collective (every rank of the communicator calls them; see bbq_comm_init below).  Without a communicator, or with
+ * world == 1, they are bbq_index_save and bbq_index_load.
+ * bbq_index_save_sharded: one all-gather of every rank's {base, rows, dim, similarity, indexBits, centroid}: shards
+ *   that do not tile [0, N) exactly, a dimension, similarity or centroid other than rank 0's, or indexBits != 1 make
+ *   every rank fail alike (empty shards may sit anywhere).  Rank 0 then removes the old .vemb and creates the .veb,
+ *   every rank writes its rows, the partials are summed in one integer ncclAllReduce and rank 0 writes the .vemb.
+ *   The files equal what bbq_index_save writes for one index holding the whole corpus.
+ * bbq_index_load_sharded: rank r loads rows [r*per, min(N, (r+1)*per)), per = ceil(N / world) (host/sharded.py
+ *   shard_bounds), with its base set; the partials are summed and checked against the header on every rank, and the
+ *   ranks compare the headers they read, so a corrupted section, or paths naming different images, fail every rank
+ *   with BBQ_ERR_FORMAT.
+ * Every phase of both ends in an exchange of each rank's status: a rank that fails (open, read, out of memory, bad
+ * header) makes every rank return the same status and message ("sharded save: rank r: ..."), none is left waiting. */
+int bbq_index_save_sharded(const bbq_index* shard, const char* veb_path, const char* vemb_path);
+int bbq_index_load_sharded(bbq_ctx* ctx, const char* veb_path, const char* vemb_path, bbq_index** out_index);
+
 /* vectorValue(ord) / getCorrectiveTerms(ord) for ord in [first, first+count): lazy device->host copy.
  * packed: count*ceil(dim/8) bytes; corr4: count*4 doubles.  Either may be NULL. */
 int bbq_index_export(const bbq_index* index, uint64_t first, uint64_t count, uint8_t* packed,
