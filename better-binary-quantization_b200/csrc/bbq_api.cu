@@ -1117,12 +1117,19 @@ static int search_exact_chunked(bbq_index* ix, int nq, uint32_t k, int32_t* d_ou
   return BBQ_OK;
 }
 
-// after the stream has been synchronised: did a candidate list of the last filtered search overflow?
-static bool resolve_filtered(bbq_ctx* c, int nq) {
+// after the stream has been synchronised: must the last filtered search be redone on the exact chunked path?  Yes when a
+// candidate list overflowed, and when a query has fewer than want = min(k, n) candidates.  tau is a lower bound of the
+// k-th best finite score and the scans never admit a NaN score, so a short list means that fewer than k rows score
+// finitely and rows that score NaN belong at the tail of the answer.
+static bool resolve_filtered(bbq_ctx* c, int nq, uint32_t want) {
   uint64_t tot = 0;
-  for (int q = 0; q < nq; q++) tot += c->h_flag[q];
+  bool short_list = false;
+  for (int q = 0; q < nq; q++) {
+    tot += c->h_flag[q];
+    short_list |= c->h_flag[q] < want;
+  }
   c->stats.last_candidates = tot;
-  return c->h_flag[nq] != 0;
+  return c->h_flag[nq] != 0 || short_list;
 }
 
 // Sampled-threshold path: tau[q] = k-th best score over a strided sample of full tiles (a valid lower
@@ -1144,7 +1151,6 @@ static int search_filtered(bbq_index* ix, int nq, uint32_t k, int32_t* d_out_idx
   if (!running) {
     const int64_t need_rows = (int64_t)std::min<double>(4.0 * (double)k * (double)n / (double)CAND_CAP, 1e12);
     want_tiles = std::max(want_tiles, std::min<int64_t>(SAMPLE_TILES_MAX, (need_rows + TILE_ROWS - 1) / TILE_ROWS));
-    if (k > (uint32_t)TAU_THREADS) want_tiles = std::min<int64_t>(want_tiles, SELECT_MAX / TILE_ROWS);  // k_select sorts the sample
     // the sample's scores are dumped densely: keep that scratch below ~1 GiB whatever the batch size
     want_tiles = std::max<int64_t>(SAMPLE_TILES, std::min<int64_t>(want_tiles, (int64_t)(1ll << 28) / ((int64_t)nq * TILE_ROWS)));
   }
@@ -1170,22 +1176,15 @@ static int search_filtered(bbq_index* ix, int nq, uint32_t k, int32_t* d_out_idx
                           nullptr, st));
     else
       TRY(launch_scan(ix, SCAN_DUMP, p, stiles, st));
-    SelectParams s{};
-    s.nq = nq;
-    s.k = k;
-    s.scores = c->dump.as<float>();
-    s.ld = sample_ld;
-    s.m = (uint32_t)(stiles * TILE_ROWS);
-    s.tile_first = 0;
-    s.tile_stride = stride;
-    s.base = (uint32_t)ix->base;
-    s.tau_out = c->tau.as<float>();
+    ProfScope prof(c, st, PROF_SELECT);
     if (k <= (uint32_t)TAU_THREADS) {
-      ProfScope prof(c, st, PROF_SELECT);
-      LAUNCH(c, k_tau_from_sample, nq, TAU_THREADS, 0, st, c->dump.as<float>(), sample_ld, s.m, k,
-             c->tau.as<float>());
+      LAUNCH(c, k_tau_from_sample<TAU_THREADS>, nq, TAU_THREADS, 0, st, c->dump.as<float>(),
+             sample_ld, (uint32_t)sample_ld, k, c->tau.as<float>());
     } else {
-      TRY(launch_select<SEL_DENSE>(c, s, s.m, st));
+      const size_t smem = TAU_BINS_MAX * sizeof(uint32_t);
+      CU(cudaFuncSetAttribute(k_tau_from_sample<TAU_BINS_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      LAUNCH(c, k_tau_from_sample<TAU_BINS_MAX>, nq, TAU_THREADS, smem, st, c->dump.as<float>(), sample_ld,
+             (uint32_t)sample_ld, k, c->tau.as<float>());
     }
   }
   uint32_t* cnt = c->cand_cnt.as<uint32_t>();
@@ -1230,7 +1229,7 @@ static int search_filtered(bbq_index* ix, int nq, uint32_t k, int32_t* d_out_idx
     return BBQ_OK;
   }
   CU(cudaStreamSynchronize(st));
-  *overflowed = resolve_filtered(c, nq);
+  *overflowed = resolve_filtered(c, nq, (uint32_t)std::min<int64_t>(k, n));
   return BBQ_OK;
 }
 
@@ -1413,9 +1412,9 @@ extern "C" int bbq_search(bbq_index* ix, const float* queries, uint32_t nq, int6
   }
   TRY(copy_results(c, nq, (size_t)k, kk, out_idx, out_score));
   if (c->pending_overflow_nq >= 0) {
-    const bool over = resolve_filtered(c, c->pending_overflow_nq);
+    const bool over = resolve_filtered(c, c->pending_overflow_nq, kk);
     c->pending_overflow_nq = -1;
-    if (over) {  // a candidate list overflowed (adversarial input): the exact chunked path redoes the batch
+    if (over) {  // a candidate list overflowed (adversarial input) or came up short: the exact chunked path redoes the batch
       c->stats.last_overflow = 1;
       c->stats.last_path = 2;
       TRY(search_exact_chunked(ix, (int)nq, kk, c->out_idx.as<int32_t>(), c->out_score.as<float>(), c->stream));

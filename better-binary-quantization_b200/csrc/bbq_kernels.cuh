@@ -571,29 +571,35 @@ __global__ void __launch_bounds__(OSQC_THREADS) k_osq_query_cta(
                  qcodes + (int64_t)q * code_ld, code_ld, qcorr + 4 * (int64_t)q, bad, (long long)q_base + q);
 }
 
-// Threshold from the sample: tau[q] = k-th largest of the per-thread maxima over the sampled scores.  The k
-// largest maxima belong to k distinct rows, so tau is a valid lower bound of the final k-th best score — and
-// almost as tight as the exact k-th of the sample (the top few rarely share a thread), at a fraction of the cost
-// of sorting the whole sample.  Requires k <= TAU_THREADS.
-constexpr int TAU_THREADS = 512;
+// Threshold from the sample: tau[q] = k-th largest of the maxima of BINS disjoint bins of the sampled scores (bin b
+// holds the scores i with i % BINS == b).  The k largest maxima belong to k distinct rows, so tau is a valid lower
+// bound of the final k-th best score — and almost as tight as the exact k-th of the sample while k is small against
+// BINS (the top few rarely share a bin), at a fraction of the cost of sorting the whole sample.  Requires k <= BINS;
+// BINS > TAU_THREADS takes its BINS keys as dynamic shared memory.  tau = -inf when fewer than k bins hold a finite score.
+constexpr int TAU_THREADS = 512;     // k <= 512: one bin per thread
+constexpr int TAU_BINS_MAX = 16384;  // k > 512: even at k = 4096 the k-th maximum is about the 1.15 k-th score of the sample
+template <int BINS>
 __global__ void __launch_bounds__(TAU_THREADS) k_tau_from_sample(const float* __restrict__ scores, int64_t ld, uint32_t m,
                                                                   uint32_t k, float* __restrict__ tau) {
-  __shared__ uint32_t keys[TAU_THREADS];
+  __shared__ uint32_t tau_keys_s[BINS <= TAU_THREADS ? BINS : 1];
+  extern __shared__ uint32_t tau_keys_d[];
+  uint32_t* const tau_keys = BINS <= TAU_THREADS ? tau_keys_s : tau_keys_d;
   const int q = blockIdx.x, tid = threadIdx.x;
-  uint32_t best = 0u;  // ordered-score key; 0 = nothing / NaN
-  for (uint32_t i = tid; i < m; i += TAU_THREADS)
-    best = max(best, (uint32_t)(bbqn::topk_key(scores[(int64_t)q * ld + i], 0u) >> 32));
-  keys[tid] = best;
-  for (uint32_t size = 2; size <= TAU_THREADS; size <<= 1) {
+  for (uint32_t b = tid; b < (uint32_t)BINS; b += TAU_THREADS) {
+    uint32_t best = 0u;  // ordered-score key; 0 = nothing / NaN
+    for (uint32_t i = b; i < m; i += BINS) best = max(best, (uint32_t)(bbqn::topk_key(scores[(int64_t)q * ld + i], 0u) >> 32));
+    tau_keys[b] = best;
+  }
+  for (uint32_t size = 2; size <= (uint32_t)BINS; size <<= 1) {
     for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
       __syncthreads();
-      if (tid < TAU_THREADS / 2) {
-        const uint32_t i = 2 * tid - (tid & (stride - 1)), j = i + stride;
-        const uint32_t x = keys[i], y = keys[j];
+      for (uint32_t t = tid; t < (uint32_t)BINS / 2; t += TAU_THREADS) {
+        const uint32_t i = 2 * t - (t & (stride - 1)), j = i + stride;
+        const uint32_t x = tau_keys[i], y = tau_keys[j];
         const bool desc = (i & size) == 0;
         if (desc ? (x < y) : (x > y)) {
-          keys[i] = y;
-          keys[j] = x;
+          tau_keys[i] = y;
+          tau_keys[j] = x;
         }
       }
     }
@@ -601,7 +607,7 @@ __global__ void __launch_bounds__(TAU_THREADS) k_tau_from_sample(const float* __
   __syncthreads();
   if (tid == 0) {
     float t = -INFINITY;
-    if (k >= 1 && k <= TAU_THREADS && keys[k - 1] != 0u) t = bbqn::topk_key_score((uint64_t)keys[k - 1] << 32);
+    if (k >= 1 && k <= (uint32_t)BINS && tau_keys[k - 1] != 0u) t = bbqn::topk_key_score((uint64_t)tau_keys[k - 1] << 32);
     tau[q] = t;
   }
 }
@@ -971,7 +977,6 @@ struct SelectParams {
   uint32_t k_in;
   // outputs (any may be null)
   uint64_t* out_keys; // [nq][k] the selected keys themselves (0 = empty slot)
-  float* tau_out;     // [nq]: score of the k-th best, -inf if fewer than k keys
   int32_t* out_idx;   // [nq][k]
   float* out_score;   // [nq][k]
 };
@@ -1025,17 +1030,6 @@ __global__ void __launch_bounds__(SELECT_THREADS) k_select(const SelectParams p,
     }
   }
   __syncthreads();
-  if (p.tau_out != nullptr && tid == 0) {
-    float t = -INFINITY;
-    if (p.k >= 1 && p.k <= m2) {
-      const uint64_t key = keys_s[p.k - 1];
-      if (key != 0ull) {
-        const float s = bbqn::topk_key_score(key);
-        if (s == s) t = s;
-      }
-    }
-    p.tau_out[q] = t;
-  }
   if (p.out_keys != nullptr)
     for (uint32_t j = tid; j < p.k; j += SELECT_THREADS) p.out_keys[(size_t)q * p.k + j] = j < m2 ? keys_s[j] : 0ull;
   if (p.out_idx != nullptr) {

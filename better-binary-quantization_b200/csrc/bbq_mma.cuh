@@ -1127,7 +1127,7 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
       }
       asm volatile("bar.sync 1, %0;" ::"n"(MMA_EPI_WARPS * 32) : "memory");
       auto row_of = [&](int64_t ti) { return (p.tile_first + ti * p.tile_stride) * TILE_ROWS + r; };
-      // per-row screen constants: prefetched one tile ahead.  Rows past the end of the shard fail every screen.
+      // per-row screen constants: prefetched one tile ahead (placeholders for rows past the end of the shard).
       const float4 rs_none = make_float4(0.f, 0.f, -INFINITY, 1.f);
       auto load_rs = [&](int64_t ti) -> float4 {
         if (MODE != SCAN_FILTER || ti >= p.ntiles) return rs_none;
@@ -1266,6 +1266,9 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
             }
             const uint32_t vmask = (nvq - qc >= 32) ? 0xFFFFFFFFu : ((1u << (nvq - qc)) - 1u);  // never a padding slot: its query id would alias
             if (always) mask = 0xFFFFFFFFu;
+            // a row past the end of the shard never parks: with tau = -inf its placeholder constants make the EUCLIDEAN
+            // lower test NaN, and fminf returns the (+inf) window test instead
+            if (!valid) mask = 0u;
             mask &= vmask;
             if (dbg & 2u) mask = 0u;
             auto v_at = [&](int j) { return j < NVC ? val[j < NVC ? j : 0] : 0; };
