@@ -59,6 +59,11 @@ SYMBOLS = {
     "bbq_index_reserve": (C.c_int, [_vp, C.c_uint64, C.c_uint32, _vp, C.POINTER(_vp)]),
     "bbq_index_append": (C.c_int, [_vp, _vp, C.c_uint64]),
     "bbq_index_append_device": (C.c_int, [_vp, _vp, C.c_uint64]),
+    "bbq_centroid_accumulate": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32, C.c_uint64, _vp]),
+    "bbq_centroid_accumulate_device": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32, C.c_uint64, _vp]),
+    "bbq_centroid_finish": (C.c_int, [_vp, C.c_uint32, C.c_uint64, _vp]),
+    "bbq_index_build_sharded": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32, _vp, C.POINTER(_vp)]),
+    "bbq_index_build_sharded_device": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32, _vp, C.POINTER(_vp)]),
     "bbq_index_from_quantized": (C.c_int, [_vp, _vp, _vp, _vp, C.c_uint64, C.c_uint32, C.POINTER(_vp)]),
     "bbq_index_size": (C.c_uint64, [_vp]),
     "bbq_index_dim": (C.c_uint32, [_vp]),

@@ -104,6 +104,31 @@ static napi_value n_build(napi_env env, napi_callback_info info) {
   return out;
 }
 
+/* buildSharded(ctx, rows: Float32Array, n, dim, centroid: Float32Array | null) -> index handle: this rank's rows of a
+ * corpus split over the ranks of the communicator (bbq_index_build_sharded, collective).  n may be 0 (dim then too). */
+static napi_value n_build_sharded(napi_env env, napi_callback_info info) {
+  ARGS(5);
+  void* ctx;
+  const float *rows, *cen = NULL;
+  size_t len, clen;
+  int64_t n;
+  uint32_t dim;
+  napi_valuetype ct;
+  napi_get_value_external(env, argv[0], &ctx);
+  if (!get_f32(env, argv[1], &rows, &len)) return throw_status(env, BBQ_ERR_INVALID_ARG);
+  napi_get_value_int64(env, argv[2], &n);
+  napi_get_value_uint32(env, argv[3], &dim);
+  napi_typeof(env, argv[4], &ct);
+  if (ct == napi_object && !get_f32(env, argv[4], &cen, &clen)) return throw_status(env, BBQ_ERR_INVALID_ARG);
+  if (n < 0 || (uint64_t)len != (uint64_t)n * dim || (cen && clen != dim)) return throw_invalid(env, "rows / centroid length does not match n * dim");
+  bbq_index* ix = NULL;
+  const int st = bbq_index_build_sharded((bbq_ctx*)ctx, rows, (uint64_t)n, dim, cen, &ix);
+  if (st != BBQ_OK) return throw_status(env, st);
+  napi_value out;
+  napi_create_external(env, ix, fin_index, NULL, &out);
+  return out;
+}
+
 /* info(index) -> {size, dimension, centroid: Float32Array, centroidDP}
  * BinarizedByteVectorValues.size()/dimension()/getCentroid()/getCentroidDP(), src/types.ts:32-49 */
 static napi_value n_info(napi_env env, napi_callback_info info) {
@@ -416,6 +441,7 @@ static napi_value n_set_base(napi_env env, napi_callback_info info) {
 NAPI_MODULE_INIT() {
   const napi_property_descriptor props[] = {
       {"create", NULL, n_create, NULL, NULL, NULL, 0, NULL}, {"build", NULL, n_build, NULL, NULL, NULL, 0, NULL},
+      {"buildSharded", NULL, n_build_sharded, NULL, NULL, NULL, 0, NULL},
       {"info", NULL, n_info, NULL, NULL, NULL, 0, NULL},     {"search", NULL, n_search, NULL, NULL, NULL, 0, NULL},
       {"rows", NULL, n_rows, NULL, NULL, NULL, 0, NULL},
       {"attachRows", NULL, n_attach_rows, NULL, NULL, NULL, 0, NULL},

@@ -30,6 +30,7 @@ type Handle = unknown;
 const addon = require('./bbq_b200.node') as {
   create(queryBits: number, indexBits: number, sim: number, lambda: number, iters: number, device: number): Handle;
   build(ctx: Handle, rows: Float32Array, n: number, dim: number, centroid: Float32Array | null): Handle;
+  buildSharded(ctx: Handle, rows: Float32Array, n: number, dim: number, centroid: Float32Array | null): Handle;
   info(index: Handle): { size: number; dimension: number; centroid: Float32Array; centroidDP: number };
   search(index: Handle, queries: Float32Array, nq: number, k: number):
     { indices: Int32Array; scores: Float32Array; count: number; stride: number };
@@ -119,14 +120,18 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
     } catch (e) { throw toReferenceError(e, 'build'); }
   }
 
-  public override quantizeVectors(vectors: Float32Array[]): {              // :165-263
+  /** With sharded = true (after joinShardGroup) the build is collective: every rank passes its own rows, ranks hold
+   *  consecutive row ranges in rank order, and a rank may pass none.  Every rank gets the centroid of the whole corpus
+   *  and its rows of the whole-corpus index, its base row set. */
+  public override quantizeVectors(vectors: Float32Array[], sharded = false): {              // :165-263
     quantizedVectors: BinarizedByteVectorValues; queryQuantizer: OptimizedScalarQuantizer;
   } {
-    if (vectors.length === 0) throw new Error('向量集合不能为空');
-    const dim = vectors[0]!.length;
+    if (vectors.length === 0 && !sharded) throw new Error('向量集合不能为空');
+    const dim = vectors.length === 0 ? 0 : vectors[0]!.length;
     const flat = flatten(vectors, dim);
     try {
-      const handle = addon.build(this.ctx, flat, vectors.length, dim, null);
+      const handle = sharded ? addon.buildSharded(this.ctx, flat, vectors.length, dim, null)
+                             : addon.build(this.ctx, flat, vectors.length, dim, null);
       // :261 hands out `this.quantizer` (an OptimizedScalarQuantizer): the inherited helper object, as getQuantizer() does
       return { quantizedVectors: new DeviceBinarizedByteVectorValues(handle), queryQuantizer: this.getQuantizer() };
     } catch (e) { throw toReferenceError(e, 'build'); }

@@ -82,7 +82,7 @@ struct bbq_ctx {
   bbq_stats stats{};
   int force_path = -1;  // BBQ_FORCE_PATH: 1 sampled+filtered, 2 exact chunked (tests)
   // build scratch
-  DevBuf T, stage, cacc;
+  DevBuf T, stage, cacc, chain, norms;  // chain: the centroid's running sum, dim words + one status word
   // query scratch
   DevBuf qrows, qT, qcodes, qcorr, planes, qterms, tau, dump, cand, cand_cnt, lists_a, lists_b,
       out_idx, out_score, dots, images, qscreen, tau_bits, trace, rr_true, rr_idx, rr_q, rr_t, cenv, qoff, qenv;
@@ -468,6 +468,52 @@ static int append_impl(bbq_index* ix, const float* rows, bool is_host, uint64_t 
   return BBQ_OK;
 }
 
+// COSINE: the f64 norms of device rows [0, n) into c->norms, ahead of a chain over them (they do not depend on the sum)
+static int row_norms(bbq_ctx* c, const float* d_rows, int64_t n, uint32_t dim) {
+  if (c->cfg.similarity != BBQ_SIM_COSINE || n == 0) return BBQ_OK;
+  TRY(c->norms.reserve((size_t)n * sizeof(double)));
+  LAUNCH(c, k_row_norms, (unsigned)((n + 127) / 128), 128, 0, c->stream, d_rows, n, (int)dim, c->norms.as<double>());
+  return BBQ_OK;
+}
+
+// The reference's running sum (device, d_acc[0, dim)) continued over rows [0, n) (host when is_host, else device), in
+// stream order.  starts_corpus: rows[0] is the corpus's row 0.  norms_ready: c->norms already holds the COSINE norms
+// of all n device rows (row_norms); otherwise they are computed chunk by chunk here.  COSINE chunks are normalised into
+// the scratch T (row-major here) by a parallel pass, so that the chain itself only adds.
+static int chain_rows(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, uint32_t dim, bool starts_corpus,
+                      float* d_acc, bool norms_ready = false) {
+  const bool cosine = c->cfg.similarity == BBQ_SIM_COSINE;
+  const unsigned grid = (dim + 31) / 32;
+  if (!is_host && !cosine) {  // one pass over the caller's rows
+    LAUNCH(c, k_centroid_chain, grid, 32, 0, c->stream, rows, (int64_t)n, (int)dim, d_acc, starts_corpus ? 1 : 0);
+    return BBQ_OK;
+  }
+  const int64_t R = (int64_t)std::min<uint64_t>(std::max<uint64_t>(n, 1), BUILD_CHUNK);
+  for (int64_t off = 0; off < (int64_t)n; off += R) {
+    const int64_t rows_here = std::min<int64_t>(R, (int64_t)n - off);
+    const float* src = rows + off * (int64_t)dim;
+    if (is_host) {  // the stream orders this copy behind the previous chunk's kernels
+      TRY(c->stage.reserve((size_t)R * dim * sizeof(float)));
+      CU(cudaMemcpyAsync(c->stage.p, src, (size_t)rows_here * dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+      src = c->stage.as<float>();
+    }
+    if (cosine) {
+      const double* norms = c->norms.as<double>() + off;
+      if (is_host || !norms_ready) {
+        TRY(row_norms(c, src, rows_here, dim));
+        norms = c->norms.as<double>();
+      }
+      TRY(c->T.reserve((size_t)R * dim * sizeof(float)));
+      const int64_t elems = rows_here * (int64_t)dim;
+      LAUNCH(c, k_normalize_rows, (unsigned)std::min<int64_t>((elems + 255) / 256, 8 * (int64_t)c->sm_count * 8), 256, 0,
+             c->stream, src, rows_here, (int)dim, norms, c->T.as<float>());
+      src = c->T.as<float>();
+    }
+    LAUNCH(c, k_centroid_chain, grid, 32, 0, c->stream, src, rows_here, (int)dim, d_acc, starts_corpus && off == 0 ? 1 : 0);
+  }
+  return BBQ_OK;
+}
+
 // rows: host (is_host) or device pointer.  The centroid (unless given) from one pass over the rows, then the rows are
 // appended to an index reserved for all of them.
 static int build_impl(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, uint32_t dim, const float* centroid,
@@ -490,13 +536,7 @@ static int build_impl(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, u
   if (centroid) {
     CU(cudaMemcpyAsync(ix->centroid, centroid, dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   } else {
-    const int64_t R = (int64_t)std::min<uint64_t>(n, BUILD_CHUNK);
-    for (int64_t off = 0; off < (int64_t)n; off += R) {
-      const int64_t rows_here = std::min<int64_t>(R, (int64_t)n - off);
-      TRY(stage_chunk(c, rows, is_host, dim, R, off, rows_here));
-      LAUNCH(c, k_centroid_accum, (dim + 63) / 64, 64, 0, c->stream, c->T.as<float>(), R, rows_here, (int)dim,
-             ix->centroid, off == 0 ? 1 : 0);
-    }
+    TRY(chain_rows(c, rows, is_host, n, dim, /*starts_corpus=*/true, ix->centroid));
     LAUNCH(c, k_centroid_finish, (dim + 127) / 128, 128, 0, c->stream, ix->centroid, (int)dim, (double)n);
   }
   TRY(finish_centroid(ix));
@@ -576,6 +616,42 @@ extern "C" int bbq_index_append(bbq_index* ix, const float* rows, uint64_t n) {
 extern "C" int bbq_index_append_device(bbq_index* ix, const float* d_rows, uint64_t n) {
   if (n == 0) return BBQ_OK;
   return append_impl(ix, d_rows, false, n);
+}
+
+// The reference centroid's running sum over a slice of the corpus: host running[0, dim) in and out
+static int accumulate_impl(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, uint32_t dim, uint64_t rows_before,
+                           float* running) {
+  if (!c || !running) return fail(BBQ_ERR_NULL, "null ctx/running");
+  if (dim == 0) return fail(BBQ_ERR_INVALID_ARG, "dim must be > 0");
+  if (n == 0) return BBQ_OK;
+  if (!rows) return fail(BBQ_ERR_NULL, "rows is null");
+  if (is_host) {
+    const int st = validate_rows(rows, n, dim, c->cfg.similarity == BBQ_SIM_COSINE);
+    if (st != BBQ_OK) return fail(st, g_err, (int64_t)rows_before + g_err_vec, g_err_pos);  // the corpus's vector index
+  }
+  CU(cudaSetDevice(c->device));
+  TRY(c->chain.reserve((size_t)dim * sizeof(float)));
+  float* acc = c->chain.as<float>();
+  if (rows_before > 0) CU(cudaMemcpyAsync(acc, running, dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  TRY(chain_rows(c, rows, is_host, n, dim, rows_before == 0, acc));
+  CU(cudaMemcpyAsync(running, acc, dim * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return BBQ_OK;
+}
+extern "C" int bbq_centroid_accumulate(bbq_ctx* c, const float* rows, uint64_t n, uint32_t dim, uint64_t rows_before,
+                                       float* running) {
+  return accumulate_impl(c, rows, true, n, dim, rows_before, running);
+}
+extern "C" int bbq_centroid_accumulate_device(bbq_ctx* c, const float* d_rows, uint64_t n, uint32_t dim,
+                                              uint64_t rows_before, float* running) {
+  return accumulate_impl(c, d_rows, false, n, dim, rows_before, running);
+}
+// k_centroid_finish on the host: f32(f64 sum / f64 N).  Dividing by float(N) instead rounds N once N > 2^24.
+extern "C" int bbq_centroid_finish(const float* running, uint32_t dim, uint64_t n_total, float* centroid) {
+  if (!running || !centroid) return fail(BBQ_ERR_NULL, "null running/centroid");
+  if (n_total == 0) return fail(BBQ_ERR_EMPTY, "vector set must not be empty");
+  for (uint32_t i = 0; i < dim; i++) centroid[i] = (float)((double)running[i] / (double)n_total);
+  return BBQ_OK;
 }
 
 // Host-side conversion between the caller's row form and the device row (cold paths: adopt / export).
@@ -1847,6 +1923,156 @@ extern "C" int bbq_search_rerank_sharded(bbq_index* ix, const float* queries, ui
 }
 
 #include "bbq_io.cuh"  // index image on disk, whole and across row shards (uses the NCCL plumbing above)
+
+// ------------------------------------------------------------------------------------------------
+// the index build across row shards (collective).  Ranks hold consecutive row ranges in rank order.  The reference
+// centroid is one f32 sum in row order, which shards cannot split, so it is CHAINED: rank r continues the running sum
+// of ranks 0 .. r-1 over its rows (k_centroid_chain), and one integer-sum ncclAllReduce, to which every other rank
+// contributes 0, hands the owner's bits to every rank.  Everything else (validation, norms, quantisation) runs on all
+// ranks at once.  Every phase ends in an exchange of each rank's status, as in the sharded save and load.
+// ------------------------------------------------------------------------------------------------
+// the verdict on an exchange whose words 0 and 1 carry the failing rank's (vector, position) in the whole corpus
+static int first_failure_at(const std::vector<RankWord>& all, const char* what) {
+  for (size_t r = 0; r < all.size(); r++)
+    if (all[r].status != BBQ_OK)
+      return fail((int)all[r].status, std::string(what) + ": rank " + std::to_string(r) + ": " + all[r].msg,
+                  (int64_t)all[r].w[0], (int64_t)all[r].w[1]);
+  return BBQ_OK;
+}
+
+// this rank's shard once the centroid is known: the chained sum over N rows (d_sum) or the caller's centroid, its
+// centroidDP, then its rows quantised, and its base
+static int finish_shard(bbq_index* ix, const float* d_sum, const float* centroid, uint64_t total, const float* rows,
+                        bool is_host, uint64_t n, uint64_t base) {
+  bbq_ctx* c = ix->ctx;
+  if (centroid) {
+    CU(cudaMemcpyAsync(ix->centroid, centroid, ix->dim * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  } else {
+    CU(cudaMemcpyAsync(ix->centroid, d_sum, ix->dim * sizeof(float), cudaMemcpyDeviceToDevice, c->stream));
+    LAUNCH(c, k_centroid_finish, (ix->dim + 127) / 128, 128, 0, c->stream, ix->centroid, (int)ix->dim, (double)total);
+  }
+  TRY(finish_centroid(ix));
+  if (n > 0) TRY(append_impl(ix, rows, is_host, n));
+  return bbq_index_set_base(ix, base);
+}
+
+static int build_sharded(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, uint32_t dim, const float* centroid,
+                         bbq_index** out_index) {
+  if (!c) return fail(BBQ_ERR_NULL, "null ctx/out_index");
+  if (!c->comm || c->world == 1)  // one shard: the plain entry
+    return is_host ? bbq_index_build(c, rows, n, dim, centroid, out_index)
+                   : bbq_index_build_device(c, rows, n, dim, centroid, out_index);
+  if (out_index) *out_index = nullptr;
+  CU(cudaSetDevice(c->device));
+  const char* what = "sharded build";
+  const int world = c->world;
+  std::vector<RankWord> all;
+  // 1. every rank's {rows, dim, similarity, indexBits, centroid given, centroid fingerprint} and argument status
+  int st = BBQ_OK;
+  if (!out_index) st = fail(BBQ_ERR_NULL, "null ctx/out_index");
+  else if (n > 0 && !rows) st = fail(BBQ_ERR_NULL, "rows is null");
+  else if (n > 0 && dim == 0) st = fail(BBQ_ERR_INVALID_ARG, "dim must be > 0");
+  RankWord mine = rank_word(st);
+  const uint64_t shape[6] = {n, dim, (uint64_t)c->cfg.similarity, (uint64_t)c->cfg.index_bits, centroid ? 1u : 0u,
+                             centroid ? bbqio::fingerprint(centroid, (size_t)dim * sizeof(float)) : 0};
+  memcpy(mine.w, shape, sizeof shape);
+  TRY(gather_ranks(c, mine, all));
+  TRY(first_failure(all, what));
+  std::vector<uint64_t> rows_of((size_t)world);
+  uint64_t total = 0, base = 0;
+  uint32_t D = 0;
+  int first_full = -1;
+  for (int r = 0; r < world; r++) {
+    rows_of[r] = all[r].w[0];
+    if (rows_of[r] > 0x7FFFFFF0ull)
+      return fail(BBQ_ERR_UNSUPPORTED, std::string(what) + ": rank " + std::to_string(r) +
+                                           " holds more than 2^31 rows (result ids are int32)");
+    if (r < c->rank) base += rows_of[r];
+    total += rows_of[r];
+    if (rows_of[r] > 0 && first_full < 0) {
+      first_full = r;
+      D = (uint32_t)all[r].w[1];
+    }
+  }
+  if (total == 0) return fail(BBQ_ERR_EMPTY, "vector set must not be empty");
+  if (total > 0x7FFFFFFFull)
+    return fail(BBQ_ERR_UNSUPPORTED, std::string(what) + ": " + std::to_string(total) +
+                                         " rows over all ranks (global row ids are int32)");
+  for (int r = 0; r < world; r++) {
+    const uint64_t d = all[r].w[1];
+    if (d != D && (rows_of[r] > 0 || d != 0))
+      return fail(BBQ_ERR_INVALID_ARG, std::string(what) + ": rank " + std::to_string(r) + " has dimension " +
+                                           std::to_string(d) + ", the rows of rank " + std::to_string(first_full) +
+                                           " have " + std::to_string(D));
+    if (all[r].w[2] != all[0].w[2] || all[r].w[3] != all[0].w[3])
+      return fail(BBQ_ERR_INVALID_ARG, std::string(what) + ": rank " + std::to_string(r) + " has similarity " +
+                                           std::to_string(all[r].w[2]) + " and indexBits " + std::to_string(all[r].w[3]) +
+                                           ", rank 0 has " + std::to_string(all[0].w[2]) + " and " +
+                                           std::to_string(all[0].w[3]));
+    if (all[r].w[4] != all[0].w[4] || all[r].w[5] != all[0].w[5])
+      return fail(BBQ_ERR_INVALID_ARG, std::string(what) + ": the centroid of rank " + std::to_string(r) +
+                                           " differs from rank 0's (every rank passes NULL, or the same centroid)");
+  }
+  if (c->cfg.index_bits > INDEX_BITS_MAX)
+    return fail(BBQ_ERR_UNSUPPORTED, "indexBits > 2 is not built on device");
+  // 2. host rows validated (positions in the whole corpus), this rank's index reserved and, for device rows, the
+  //    COSINE norms computed ahead of its turn in the chain
+  const bool cosine = c->cfg.similarity == BBQ_SIM_COSINE;
+  int64_t bad_vec = -1, bad_pos = -1;
+  st = is_host && n > 0 ? validate_rows(rows, n, D, cosine) : BBQ_OK;
+  if (st != BBQ_OK) {
+    bad_vec = (int64_t)base + g_err_vec;
+    bad_pos = g_err_pos;
+  }
+  IndexGuard g;
+  if (st == BBQ_OK && (st = index_alloc(c, std::max<uint64_t>(n, 1), D, &g.ix)) == BBQ_OK) g.ix->n = 0;
+  if (st == BBQ_OK && !centroid) st = c->chain.reserve(((size_t)D + 1) * sizeof(uint32_t));
+  if (st == BBQ_OK && !centroid && !is_host) st = row_norms(c, rows, (int64_t)n, D);
+  mine = rank_word(st);
+  mine.w[0] = (uint64_t)bad_vec;
+  mine.w[1] = (uint64_t)bad_pos;
+  TRY(gather_ranks(c, mine, all));
+  TRY(first_failure_at(all, what));
+  // 3. the chain, rank by rank (ranks without rows are skipped: every rank knows the row counts)
+  float* sum = c->chain.as<float>();
+  if (!centroid) {
+    uint32_t* status_word = c->chain.as<uint32_t>() + D;
+    for (int r = 0; r < world; r++) {
+      if (rows_of[r] == 0) continue;
+      int mine_st = BBQ_OK;
+      if (r == c->rank) {
+        mine_st = chain_rows(c, rows, is_host, n, D, base == 0, sum, /*norms_ready=*/!is_host);
+        const uint32_t s = (uint32_t)mine_st;
+        CU(cudaMemcpyAsync(status_word, &s, sizeof s, cudaMemcpyHostToDevice, c->stream));
+      } else {
+        CU(cudaMemsetAsync(sum, 0, ((size_t)D + 1) * sizeof(uint32_t), c->stream));
+      }
+      // integer sum: the owner's bits arrive unchanged (-0.0, subnormals and NaN payloads included)
+      NC(nccl_api()->AllReduce(sum, sum, (size_t)D + 1, ncclUint32, ncclSum, c->comm, c->stream));
+      uint32_t verdict = 0;
+      CU(cudaMemcpyAsync(&verdict, status_word, sizeof verdict, cudaMemcpyDeviceToHost, c->stream));
+      CU(cudaStreamSynchronize(c->stream));
+      if (verdict != BBQ_OK) {  // the owner's message reaches every rank
+        TRY(gather_ranks(c, rank_word(mine_st), all));
+        return first_failure(all, what);
+      }
+    }
+  }
+  // 4. every rank quantises its rows; a failure on any rank fails all, and none keeps a half-built shard
+  TRY(gather_ranks(c, rank_word(finish_shard(g.ix, sum, centroid, total, rows, is_host, n, base)), all));
+  TRY(first_failure(all, what));
+  *out_index = g.release();
+  return BBQ_OK;
+}
+
+extern "C" int bbq_index_build_sharded(bbq_ctx* c, const float* rows, uint64_t n, uint32_t dim, const float* centroid,
+                                       bbq_index** out_index) {
+  return build_sharded(c, rows, true, n, dim, centroid, out_index);
+}
+extern "C" int bbq_index_build_sharded_device(bbq_ctx* c, const float* d_rows, uint64_t n, uint32_t dim,
+                                              const float* centroid, bbq_index** out_index) {
+  return build_sharded(c, d_rows, false, n, dim, centroid, out_index);
+}
 
 // Page-locked host buffers for hosts that want the H2D / D2H copies of bbq_search* to run at full PCIe speed
 // (a Node host wraps them in external ArrayBuffers; any host pointer works, pageable memory is merely slower).

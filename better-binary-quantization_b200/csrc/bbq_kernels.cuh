@@ -67,23 +67,79 @@ __global__ void k_normalize_T(float* __restrict__ T, int64_t ld, int64_t nrows, 
   }
 }
 
-// computeCentroid, src/vectorOperations.ts:126-163: centroid = copy(V[0]); for j>=1: c_i = f32(c_i + V[j]_i)
-// strictly in row order.  One thread per component walks the chunk's rows sequentially.
-__global__ void k_centroid_accum(const float* __restrict__ T, int64_t ld, int64_t nrows, int dim,
-                                 float* __restrict__ acc, int first_chunk) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= dim) return;
-  const float* row = T + (int64_t)i * ld;
-  int64_t t = 0;
-  float c;
-  if (first_chunk) {
-    c = row[0];
-    t = 1;
-  } else {
-    c = acc[i];
+// The f64 norm of each row-major row, in bbqn::l2norm_seq order: the divisor k_normalize_T uses for COSINE.
+struct RAcc {
+  const float* p;
+  __device__ __forceinline__ float operator()(int i) const { return p[i]; }
+};
+__global__ void k_row_norms(const float* __restrict__ rows, int64_t nrows, int dim, double* __restrict__ norms) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < nrows) norms[t] = bbqn::l2norm_seq(RAcc{rows + t * dim}, dim);
+}
+
+__device__ __forceinline__ void cp_async4(float* smem, const float* gmem) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
+
+// COSINE rows for the centroid chain, normalised into row-major scratch: out = f32((double)v / norm), or 0 when
+// norm == 0, exactly as k_normalize_T computes it, with the norms of k_row_norms.  One thread per element, so that the
+// f64 divisions run on the whole GPU instead of inside the chain.
+__global__ void k_normalize_rows(const float* __restrict__ rows, int64_t nrows, int dim, const double* __restrict__ norms,
+                                 float* __restrict__ out) {
+  const int64_t total = nrows * dim;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const double nn = norms[e / dim];
+    out[e] = nn == 0 ? 0.0f : (float)((double)rows[e] / nn);
   }
-  for (; t < nrows; t++) c = (float)((double)c + (double)row[t]);
-  acc[i] = c;
+}
+
+// computeCentroid, src/vectorOperations.ts:126-163: centroid = copy(V[0]); for j>=1: c_i = f32(c_i + V[j]_i) strictly in
+// row order.  The running sum acc[0, dim) is continued over rows [0, nrows) (row-major, COSINE rows already normalised
+// by k_normalize_rows); starts_corpus: rows[0] is the corpus's row 0 and is copied, otherwise every row is added.  Each
+// step is __fadd_rn: for two f32 operands the correctly rounded f32 sum equals f32(f64 sum) (53 >= 2*24 + 2), the same
+// bits for +-0, subnormals, +-Inf and NaN.  One warp per 32 components (grid: ceil(dim / 32) blocks of 32 threads): the
+// lanes read one row's 128 contiguous bytes, and cp.async keeps CHAIN_GROUPS groups of CHAIN_ROWS rows in flight in
+// shared memory, so the only dependent work per row is one shared load and one FADD.
+constexpr int CHAIN_ROWS = 16;
+constexpr int CHAIN_GROUPS = 16;
+__global__ void __launch_bounds__(32) k_centroid_chain(const float* __restrict__ rows, int64_t nrows, int dim,
+                                                       float* __restrict__ acc, int starts_corpus) {
+  __shared__ float ring[CHAIN_GROUPS * CHAIN_ROWS][32];
+  const int lane = threadIdx.x;
+  const int i = blockIdx.x * 32 + lane;
+  const bool on = i < dim;
+  const float* col = rows + (on ? i : 0);
+  const int64_t ngroups = (nrows + CHAIN_ROWS - 1) / CHAIN_ROWS;
+  auto issue = [&](int64_t g) {  // one commit per call, empty past the end, so that wait_group counts uniformly
+    if (g < ngroups) {
+      const int slot = (int)(g % CHAIN_GROUPS) * CHAIN_ROWS;
+      const int m = (int)min((int64_t)CHAIN_ROWS, nrows - g * CHAIN_ROWS);
+      const float* src = col + g * CHAIN_ROWS * dim;
+#pragma unroll
+      for (int u = 0; u < CHAIN_ROWS; u++)
+        if (on && u < m) cp_async4(&ring[slot + u][lane], src + (int64_t)u * dim);
+    }
+    cp_async_commit();
+  };
+#pragma unroll
+  for (int g = 0; g < CHAIN_GROUPS - 1; g++) issue(g);
+  float c = (on && !starts_corpus) ? acc[i] : 0.0f;
+  for (int64_t g = 0; g < ngroups; g++) {
+    issue(g + CHAIN_GROUPS - 1);  // into the slot group g - 1 used (each lane reads back only what it copied)
+    cp_async_wait<CHAIN_GROUPS - 1>();
+    const int slot = (int)(g % CHAIN_GROUPS) * CHAIN_ROWS;
+    const int u0 = (g == 0 && starts_corpus) ? 1 : 0;
+    const int m = (int)min((int64_t)CHAIN_ROWS, nrows - g * CHAIN_ROWS);
+    if (u0) c = ring[slot][lane];
+#pragma unroll
+    for (int u = 0; u < CHAIN_ROWS; u++)
+      if (u >= u0 && u < m) c = __fadd_rn(c, ring[slot + u][lane]);
+  }
+  cp_async_wait<0>();
+  if (on) acc[i] = c;
 }
 __global__ void k_centroid_finish(float* __restrict__ acc, int dim, double n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;

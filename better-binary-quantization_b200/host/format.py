@@ -178,25 +178,64 @@ class BinaryQuantizationFormat:
         return dict(self.config)
 
     # -- index build ----------------------------------------------------------------------------------
-    def quantizeVectors(self, vectors, centroid: Optional[np.ndarray] = None) -> dict:
-        if vectors is None or len(vectors) == 0:
+    def quantizeVectors(self, vectors, centroid: Optional[np.ndarray] = None, sharded: bool = False) -> dict:
+        """sharded=True: this rank's rows of a corpus split over the communicator in rank order (bbq_index_build_sharded,
+        collective); the rank may hold no rows.  Without a centroid every rank gets the reference-order centroid of the
+        whole corpus, and its shard (base set) equals its rows of the whole-corpus build."""
+        if not sharded and (vectors is None or len(vectors) == 0):
             raise BbqError(3, "向量集合不能为空")
-        m = _as_matrix(vectors)
+        m = _as_matrix(vectors if vectors is not None else [])
         h = C.c_void_p()
         cen = np.ascontiguousarray(centroid, np.float32) if centroid is not None else None
-        _check(_native.load().bbq_index_build(self._ctx, m.ctypes.data, m.shape[0], m.shape[1],
-                                              cen.ctypes.data if cen is not None else None, C.byref(h)), "build")
+        L = _native.load()
+        if sharded:
+            dim = m.shape[1] if m.shape[0] else (cen.size if cen is not None else 0)
+            _check(L.bbq_index_build_sharded(self._ctx, m.ctypes.data, m.shape[0], dim,
+                                             cen.ctypes.data if cen is not None else None, C.byref(h)), "build")
+        else:
+            _check(L.bbq_index_build(self._ctx, m.ctypes.data, m.shape[0], m.shape[1],
+                                     cen.ctypes.data if cen is not None else None, C.byref(h)), "build")
         # (the reference hands out its OptimizedScalarQuantizer helper as queryQuantizer, :261, and so does the TypeScript
         # drop-in; this Python stand-in has no such host-side object: the format itself quantises queries)
         return {"quantizedVectors": BinarizedByteVectorValues(self, h), "queryQuantizer": self}
 
-    def quantizeVectorsDevice(self, d_rows_ptr: int, n: int, dim: int, centroid: Optional[np.ndarray] = None):
-        """Rows already in device memory (e.g. a torch tensor's data_ptr())."""
+    def quantizeVectorsDevice(self, d_rows_ptr: int, n: int, dim: int, centroid: Optional[np.ndarray] = None,
+                              sharded: bool = False):
+        """Rows already in device memory (e.g. a torch tensor's data_ptr()).  sharded=True: as quantizeVectors
+        (bbq_index_build_sharded_device, collective)."""
         h = C.c_void_p()
         cen = np.ascontiguousarray(centroid, np.float32) if centroid is not None else None
-        _check(_native.load().bbq_index_build_device(self._ctx, d_rows_ptr, n, dim,
-                                                     cen.ctypes.data if cen is not None else None, C.byref(h)), "build")
+        L = _native.load()
+        fn = L.bbq_index_build_sharded_device if sharded else L.bbq_index_build_device
+        _check(fn(self._ctx, d_rows_ptr or None, n, dim, cen.ctypes.data if cen is not None else None, C.byref(h)),
+               "build")
         return {"quantizedVectors": BinarizedByteVectorValues(self, h), "queryQuantizer": self}
+
+    def accumulateCentroid(self, running: np.ndarray, rowsBefore: int, rows=None, d_rows_ptr: int = 0, n: int = 0):
+        """The reference centroid's running sum (f32[dim], updated in place and returned) continued over the rows that
+        follow the corpus's first rowsBefore rows: host `rows`, or n device rows at d_rows_ptr
+        (bbq_centroid_accumulate / _device).  rowsBefore == 0 starts the corpus."""
+        if running.dtype != np.float32 or not running.flags.c_contiguous:
+            raise BbqError(10, "running must be a contiguous float32 array")
+        L = _native.load()
+        if rows is not None:
+            m = _as_matrix(rows)
+            if m.shape[0] and m.shape[1] != running.size:
+                raise BbqError(4, "向量维度不匹配")
+            _check(L.bbq_centroid_accumulate(self._ctx, m.ctypes.data, m.shape[0], running.size, rowsBefore,
+                                             running.ctypes.data), "build")
+        else:
+            _check(L.bbq_centroid_accumulate_device(self._ctx, d_rows_ptr or None, n, running.size, rowsBefore,
+                                                    running.ctypes.data), "build")
+        return running
+
+    @staticmethod
+    def finishCentroid(running, nTotal: int) -> np.ndarray:
+        """f32(running / N) in f64 (bbq_centroid_finish): the centroid bbq_index_build computes for N rows."""
+        r = np.ascontiguousarray(running, np.float32)
+        out = np.empty(r.size, np.float32)
+        _check(_native.load().bbq_centroid_finish(r.ctypes.data, r.size, nTotal, out.ctypes.data), "build")
+        return out
 
     def reserveIndex(self, capacity: int, dim: int, centroid) -> BinarizedByteVectorValues:
         """Streaming build (bbq_index_reserve): explicit centroid, rows appended chunk by chunk."""

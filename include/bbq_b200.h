@@ -96,12 +96,46 @@ int bbq_index_build_device(bbq_ctx* ctx, const float* d_rows, uint64_t n, uint32
                            const float* centroid_host_or_null, bbq_index** out_index);
 
 /* Streaming build for corpora that never exist whole (SURVEY §7 hard-part 5): reserve `capacity` rows with an
- * EXPLICIT centroid (host pointer, required — the reference-order centroid needs every row first), then append
+ * EXPLICIT centroid (host pointer, required — the reference-order centroid needs every row first: one pass of
+ * bbq_centroid_accumulate + bbq_centroid_finish below gives it), then append
  * row chunks (host or device memory) in order; each chunk is quantised exactly as quantizeVectors would with
  * that centroid (src/binaryQuantizationFormat.ts:221-249).  bbq_index_size() grows with each append. */
 int bbq_index_reserve(bbq_ctx* ctx, uint64_t capacity, uint32_t dim, const float* centroid, bbq_index** out_index);
 int bbq_index_append(bbq_index* index, const float* rows, uint64_t n);
 int bbq_index_append_device(bbq_index* index, const float* d_rows, uint64_t n);
+
+/* The reference-order centroid of a corpus that is streamed or split (src/vectorOperations.ts:126-163:
+ * c = copy(V[0]); c = f32(c + V[j]) for j = 1 .. N-1 in row order; then f32(c / N)).  Not collective.
+ * bbq_centroid_accumulate(_device): continues the running sum `running` (HOST, dim floats, read and written) over the
+ *   n rows that follow the corpus's first rows_before rows; rows_before == 0: this slice starts the corpus (row 0 is
+ *   copied, `running` is only written).  COSINE rows are normalised first, as bbq_index_build does.  Host rows are
+ *   validated like bbq_index_build's (the vector index reported counts from the corpus's row 0); device rows are not.
+ *   n == 0 leaves `running` unchanged.
+ * bbq_centroid_finish: centroid[i] = f32((double)running[i] / (double)n_total), what bbq_index_build computes (dividing
+ *   by float(N) instead is wrong once N > 2^24).  Host only, needs no device.
+ * One pass of accumulate over all slices, finish, then bbq_index_reserve + bbq_index_append* of the slices gives the
+ * index bbq_index_build gives for the whole corpus. */
+int bbq_centroid_accumulate(bbq_ctx* ctx, const float* rows, uint64_t n, uint32_t dim, uint64_t rows_before,
+                            float* running);
+int bbq_centroid_accumulate_device(bbq_ctx* ctx, const float* d_rows, uint64_t n, uint32_t dim, uint64_t rows_before,
+                                   float* running);
+int bbq_centroid_finish(const float* running, uint32_t dim, uint64_t n_total, float* centroid);
+
+/* quantizeVectors over row shards (collective: every rank of the communicator calls it with its own rows; see
+ * bbq_comm_init).  Ranks hold consecutive row ranges in rank order; a rank may hold 0 rows (and pass dim 0, unless it
+ * passes a centroid).  centroid: NULL on every rank = the reference-order centroid of the whole corpus, chained across
+ * the ranks (rank r continues the running sum of ranks 0 .. r-1, one ncclAllReduce per non-empty rank); or the same
+ * explicit centroid on every rank.  Each rank gets the index of rows [base, base + n) of bbq_index_build over the whole
+ * corpus, byte for byte, with its base set (base = the rows of the ranks before it).
+ * Every rank returns the same status and message: Σ n == 0 -> BBQ_ERR_EMPTY; a shard over 2^31 - 16 rows or Σ n over
+ * 2^31 - 1 -> BBQ_ERR_UNSUPPORTED; dimensions, similarity, indexBits or centroids that differ -> BBQ_ERR_INVALID_ARG;
+ * a NaN / Infinity in host rows -> the lowest such rank's status, with bbq_last_error_pos naming the vector in the
+ * whole corpus; out of memory on any rank fails every rank.  Without a communicator (or world == 1) they are
+ * bbq_index_build and bbq_index_build_device. */
+int bbq_index_build_sharded(bbq_ctx* ctx, const float* rows, uint64_t n, uint32_t dim, const float* centroid,
+                            bbq_index** out_index);
+int bbq_index_build_sharded_device(bbq_ctx* ctx, const float* d_rows, uint64_t n, uint32_t dim,
+                                   const float* centroid_host_or_null, bbq_index** out_index);
 
 /* Adopt an index quantised elsewhere (e.g. by the reference itself): packed = n*ceil(dim/8) bytes,
  * MSB-first rows exactly as BinarizedByteVectorValuesImpl.vectors holds them
