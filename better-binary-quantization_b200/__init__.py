@@ -8,7 +8,7 @@ from . import _native
 from ._native import build_library
 from .host.sharded import ShardedSearcher, broadcast_comm_id, merge_host, shard_bounds
 from .host.format import (BbqError, BinarizedByteVectorValues, BinaryQuantizationFormat,
-                          VectorSimilarityFunction)
+                          GroupBinarizedByteVectorValues, VectorSimilarityFunction)
 
 VERSION = "1.0.0"  # src/index.ts:139
 
@@ -17,9 +17,9 @@ DEFAULT_CONFIG = {"queryBits": 4, "indexBits": 1,
                   "quantizer": {"similarityFunction": VectorSimilarityFunction.COSINE, "lambda": 0.1, "iters": 5}}
 
 
-def createBinaryQuantizationFormat(config=None, device: int = -1) -> BinaryQuantizationFormat:
-    """src/index.ts:62-64"""
-    return BinaryQuantizationFormat(config if config is not None else DEFAULT_CONFIG, device=device)
+def createBinaryQuantizationFormat(config=None, device: int = -1, devices=None) -> BinaryQuantizationFormat:
+    """src/index.ts:62-64.  devices: a device group over those GPUs (BinaryQuantizationFormat)."""
+    return BinaryQuantizationFormat(config if config is not None else DEFAULT_CONFIG, device=device, devices=devices)
 
 
 _QUICK_FORMATS = {}
@@ -63,7 +63,7 @@ def getOversampledTopKWithSort(query, quantizedVectors, vectors, k, oversampleFa
 getOversampledTopKWithHeap = getOversampledTopKWithSort  # :29-78 — same set unless true scores tie at the k-th place
 
 
-__all__ = ["BinaryQuantizationFormat", "BinarizedByteVectorValues", "VectorSimilarityFunction", "BbqError",
+__all__ = ["BinaryQuantizationFormat", "BinarizedByteVectorValues", "GroupBinarizedByteVectorValues", "VectorSimilarityFunction", "BbqError",
            "createBinaryQuantizationFormat", "quickQuantize", "quickSearch", "DEFAULT_CONFIG", "VERSION",
            "build_library", "ShardedSearcher", "shard_bounds", "merge_host", "broadcast_comm_id", "getOversampledTopKWithSort",
            "getOversampledTopKWithHeap"]

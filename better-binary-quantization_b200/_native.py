@@ -98,6 +98,23 @@ SYMBOLS = {
     "bbq_search_sharded_device": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, _vp, _vp, _vp]),
     "bbq_quantize_query": (C.c_int, [_vp, _vp, _vp, C.c_uint32, _vp, _vp]),
     "bbq_quantization_accuracy": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint32, C.c_uint64, _vp]),
+    "bbq_group_create": (C.c_int, [C.POINTER(BbqConfig), _vp, C.c_uint32, C.POINTER(_vp)]),
+    "bbq_group_destroy": (C.c_int, [_vp]),
+    "bbq_group_info": (C.c_int, [_vp, C.POINTER(C.c_uint32), _vp]),
+    "bbq_group_context": (C.c_void_p, [_vp, C.c_uint32]),
+    "bbq_group_index_build": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint32, _vp, C.POINTER(_vp)]),
+    "bbq_group_index_from_quantized": (C.c_int, [_vp, _vp, _vp, _vp, C.c_uint64, C.c_uint32, C.POINTER(_vp)]),
+    "bbq_group_index_load": (C.c_int, [_vp, C.c_char_p, C.c_char_p, C.POINTER(_vp)]),
+    "bbq_group_index_save": (C.c_int, [_vp, C.c_char_p, C.c_char_p]),
+    "bbq_group_index_size": (C.c_uint64, [_vp]),
+    "bbq_group_index_dim": (C.c_uint32, [_vp]),
+    "bbq_group_index_centroid": (C.c_int, [_vp, _vp, C.POINTER(C.c_double)]),
+    "bbq_group_index_export": (C.c_int, [_vp, C.c_uint64, C.c_uint64, _vp, _vp]),
+    "bbq_group_index_attach_rows": (C.c_int, [_vp, _vp]),
+    "bbq_group_search": (C.c_int, [_vp, _vp, C.c_uint32, C.c_int64, _vp, _vp, C.POINTER(C.c_uint32)]),
+    "bbq_group_search_rerank": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp, _vp,
+                                          C.POINTER(C.c_uint32)]),
+    "bbq_group_index_destroy": (None, [_vp]),
     "bbq_host_alloc": (C.c_void_p, [C.c_size_t]),
     "bbq_host_free": (None, [_vp]),
     "bbq_debug_scores": (C.c_int, [_vp, _vp, _vp]),

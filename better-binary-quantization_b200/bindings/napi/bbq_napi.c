@@ -13,6 +13,7 @@
 #include "node_api_min.h"
 #endif
 #include <stdio.h>
+#include <stdlib.h>
 #include <string.h>
 #include "bbq_b200.h"
 
@@ -438,6 +439,275 @@ static napi_value n_set_base(napi_env env, napi_callback_info info) {
   return u;
 }
 
+/* ---- device groups: one process, every GPU of the box (bbq_group_*) ------------------------------------------------
+ * A group index keeps a strong reference to its group, so that the group's finalizer (bbq_group_destroy, which refuses
+ * while group indexes are alive) runs only after the finalizers of all its indexes. */
+typedef struct {
+  bbq_group_index* gi;
+  napi_ref group;
+} group_index_handle;
+static void fin_group(napi_env env, void* data, void* hint) { (void)env; (void)hint; bbq_group_destroy((bbq_group*)data); }
+static void fin_group_index(napi_env env, void* data, void* hint) {
+  (void)hint;
+  group_index_handle* h = (group_index_handle*)data;
+  bbq_group_index_destroy(h->gi);
+  napi_delete_reference(env, h->group);
+  free(h);
+}
+static napi_value wrap_group_index(napi_env env, napi_value group, bbq_group_index* gi) {
+  group_index_handle* h = (group_index_handle*)malloc(sizeof *h);
+  if (!h) {
+    bbq_group_index_destroy(gi);
+    napi_throw_error(env, "BBQ:102:-1:-1", "out of memory");
+    return NULL;
+  }
+  h->gi = gi;
+  napi_create_reference(env, group, 1, &h->group);
+  napi_value out;
+  napi_create_external(env, h, fin_group_index, NULL, &out);
+  return out;
+}
+static bbq_group_index* group_index_of(napi_env env, napi_value v) {
+  void* h = NULL;
+  if (napi_get_value_external(env, v, &h) != napi_ok || !h) return NULL;
+  return ((group_index_handle*)h)->gi;
+}
+
+/* groupCreate(queryBits, indexBits, similarity, lambda, iters, devices Int32Array) -> external group */
+static napi_value n_group_create(napi_env env, napi_callback_info info) {
+  ARGS(6);
+  bbq_config cfg;
+  memset(&cfg, 0, sizeof cfg);
+  napi_typedarray_type t;
+  size_t n;
+  void* devs;
+  napi_get_value_uint32(env, argv[0], &cfg.query_bits);
+  napi_get_value_uint32(env, argv[1], &cfg.index_bits);
+  napi_get_value_uint32(env, argv[2], &cfg.similarity);
+  napi_get_value_double(env, argv[3], &cfg.lambda);
+  napi_get_value_uint32(env, argv[4], &cfg.iters);
+  if (napi_get_typedarray_info(env, argv[5], &t, &n, &devs, NULL, NULL) != napi_ok || t != napi_int32_array)
+    return throw_invalid(env, "devices must be an Int32Array");
+  bbq_group* g = NULL;
+  const int st = bbq_group_create(&cfg, (const int32_t*)devs, (uint32_t)n, &g);
+  if (st != BBQ_OK) return throw_status(env, st);
+  napi_value out;
+  napi_create_external(env, g, fin_group, NULL, &out);
+  return out;
+}
+
+/* groupContext(group) -> the first GPU's context (no finalizer: the group owns it), for quantizeQuery / accuracy */
+static napi_value n_group_context(napi_env env, napi_callback_info info) {
+  ARGS(1);
+  void* g;
+  napi_get_value_external(env, argv[0], &g);
+  bbq_ctx* c = bbq_group_context((bbq_group*)g, 0);
+  if (!c) return throw_status(env, BBQ_ERR_INVALID_ARG);
+  napi_value out;
+  napi_create_external(env, c, NULL, NULL, &out);
+  return out;
+}
+
+/* groupBuild(group, rows Float32Array[n*dim], n, dim, centroid | null) -> group index (rows split over the GPUs) */
+static napi_value n_group_build(napi_env env, napi_callback_info info) {
+  ARGS(5);
+  void* g;
+  const float *rows, *cen = NULL;
+  size_t len, clen;
+  int64_t n;
+  uint32_t dim;
+  napi_valuetype ct;
+  napi_get_value_external(env, argv[0], &g);
+  if (!get_f32(env, argv[1], &rows, &len)) return throw_status(env, BBQ_ERR_INVALID_ARG);
+  napi_get_value_int64(env, argv[2], &n);
+  napi_get_value_uint32(env, argv[3], &dim);
+  napi_typeof(env, argv[4], &ct);
+  if (ct == napi_object && !get_f32(env, argv[4], &cen, &clen)) return throw_status(env, BBQ_ERR_INVALID_ARG);
+  if (n < 0 || dim == 0 || (uint64_t)len != (uint64_t)n * dim || (cen && clen != dim)) return throw_invalid(env, "rows / centroid length does not match n * dim");
+  bbq_group_index* gi = NULL;
+  const int st = bbq_group_index_build((bbq_group*)g, rows, (uint64_t)n, dim, cen, &gi);
+  if (st != BBQ_OK) return throw_status(env, st);
+  return wrap_group_index(env, argv[0], gi);
+}
+
+/* groupFromQuantized(group, packed, corrections, centroid, n, dim) -> group index (deserializeVectorData) */
+static napi_value n_group_from_quantized(napi_env env, napi_callback_info info) {
+  ARGS(6);
+  void *g, *pk, *cr;
+  const float* cen;
+  size_t plen, clen, cenlen;
+  napi_typedarray_type t1, t2;
+  int64_t n;
+  uint32_t dim;
+  napi_get_value_external(env, argv[0], &g);
+  if (napi_get_typedarray_info(env, argv[1], &t1, &plen, &pk, NULL, NULL) != napi_ok || t1 != napi_uint8_array ||
+      napi_get_typedarray_info(env, argv[2], &t2, &clen, &cr, NULL, NULL) != napi_ok || t2 != napi_float64_array ||
+      !get_f32(env, argv[3], &cen, &cenlen))
+    return throw_status(env, BBQ_ERR_NULL);
+  napi_get_value_int64(env, argv[4], &n);
+  napi_get_value_uint32(env, argv[5], &dim);
+  if (n <= 0 || cenlen != dim || (uint64_t)plen != (uint64_t)n * ((dim + 7) / 8) || (uint64_t)clen != (uint64_t)n * 4)
+    return throw_invalid(env, "packed / corrections / centroid lengths do not match n and dim");
+  bbq_group_index* gi = NULL;
+  const int st = bbq_group_index_from_quantized((bbq_group*)g, (const uint8_t*)pk, (const double*)cr, cen, (uint64_t)n, dim, &gi);
+  if (st != BBQ_OK) return throw_status(env, st);
+  return wrap_group_index(env, argv[0], gi);
+}
+
+/* groupLoadIndex(group, vebPath, vembPath) -> group index; groupSaveIndex(groupIndex, vebPath, vembPath) */
+static napi_value n_group_load_index(napi_env env, napi_callback_info info) {
+  ARGS(3);
+  void* g;
+  char veb[4096], vemb[4096];
+  napi_get_value_external(env, argv[0], &g);
+  if (!get_path(env, argv[1], veb, sizeof veb) || !get_path(env, argv[2], vemb, sizeof vemb)) return throw_status(env, BBQ_ERR_NULL);
+  bbq_group_index* gi = NULL;
+  const int st = bbq_group_index_load((bbq_group*)g, veb, vemb, &gi);
+  if (st != BBQ_OK) return throw_status(env, st);
+  return wrap_group_index(env, argv[0], gi);
+}
+static napi_value n_group_save_index(napi_env env, napi_callback_info info) {
+  ARGS(3);
+  char veb[4096], vemb[4096];
+  bbq_group_index* gi = group_index_of(env, argv[0]);
+  if (!get_path(env, argv[1], veb, sizeof veb) || !get_path(env, argv[2], vemb, sizeof vemb)) return throw_status(env, BBQ_ERR_NULL);
+  const int st = bbq_group_index_save(gi, veb, vemb);
+  if (st != BBQ_OK) return throw_status(env, st);
+  napi_value u;
+  napi_get_undefined(env, &u);
+  return u;
+}
+
+/* groupInfo(groupIndex) -> {size, dimension, centroid, centroidDP}, as info() */
+static napi_value n_group_info(napi_env env, napi_callback_info info) {
+  ARGS(1);
+  bbq_group_index* gi = group_index_of(env, argv[0]);
+  const uint32_t dim = bbq_group_index_dim(gi);
+  napi_value out, ab, cen, v;
+  void* data;
+  double cdp = 0;
+  napi_create_object(env, &out);
+  napi_create_arraybuffer(env, dim * sizeof(float), &data, &ab);
+  bbq_group_index_centroid(gi, (float*)data, &cdp);
+  napi_create_typedarray(env, napi_float32_array, dim, ab, 0, &cen);
+  napi_create_double(env, (double)bbq_group_index_size(gi), &v);
+  napi_set_named_property(env, out, "size", v);
+  napi_create_uint32(env, dim, &v);
+  napi_set_named_property(env, out, "dimension", v);
+  napi_set_named_property(env, out, "centroid", cen);
+  napi_create_double(env, cdp, &v);
+  napi_set_named_property(env, out, "centroidDP", v);
+  return out;
+}
+
+/* groupRows(groupIndex, first, count) -> {packed, corrections}, as rows(): each part from the GPU that holds it */
+static napi_value n_group_rows(napi_env env, napi_callback_info info) {
+  ARGS(3);
+  int64_t first, count;
+  bbq_group_index* gi = group_index_of(env, argv[0]);
+  napi_get_value_int64(env, argv[1], &first);
+  napi_get_value_int64(env, argv[2], &count);
+  if (first < 0 || count < 0 || (uint64_t)first + (uint64_t)count > bbq_group_index_size(gi))
+    return throw_invalid(env, "row range out of bounds");
+  const size_t p = (bbq_group_index_dim(gi) + 7) / 8;
+  napi_value out, ab1, ab2, t1, t2;
+  void* d1 = new_buffer(env, (size_t)count * p, &ab1);
+  void* d2 = d1 ? new_buffer(env, (size_t)count * 4 * sizeof(double), &ab2) : NULL;
+  if (!d1 || !d2) return NULL;
+  const int st = bbq_group_index_export(gi, (uint64_t)first, (uint64_t)count, (uint8_t*)d1, (double*)d2);
+  if (st != BBQ_OK) return throw_status(env, st);
+  napi_create_typedarray(env, napi_uint8_array, (size_t)count * p, ab1, 0, &t1);
+  napi_create_typedarray(env, napi_float64_array, (size_t)count * 4, ab2, 0, &t2);
+  napi_create_object(env, &out);
+  napi_set_named_property(env, out, "packed", t1);
+  napi_set_named_property(env, out, "corrections", t2);
+  return out;
+}
+
+/* groupAttachRows(groupIndex, rowsFlat Float32Array[n*dim]): every GPU keeps its slice for the exact re-rank */
+static napi_value n_group_attach_rows(napi_env env, napi_callback_info info) {
+  ARGS(2);
+  const float* rows;
+  size_t len;
+  bbq_group_index* gi = group_index_of(env, argv[0]);
+  if (!get_f32(env, argv[1], &rows, &len)) return throw_status(env, BBQ_ERR_NULL);
+  if (len != (size_t)bbq_group_index_size(gi) * bbq_group_index_dim(gi)) return throw_status(env, BBQ_ERR_DIM_MISMATCH);
+  const int st = bbq_group_index_attach_rows(gi, rows);
+  if (st != BBQ_OK) return throw_status(env, st);
+  napi_value u;
+  napi_get_undefined(env, &u);
+  return u;
+}
+
+/* groupSearch(groupIndex, queriesFlat, nq, k) -> {indices, scores, count, stride}, as search() */
+static napi_value n_group_search(napi_env env, napi_callback_info info) {
+  ARGS(4);
+  const float* q;
+  size_t len;
+  uint32_t nq, count = 0;
+  int64_t k;
+  bbq_group_index* gi = group_index_of(env, argv[0]);
+  if (!gi) return throw_status(env, BBQ_ERR_NULL);
+  if (!get_f32(env, argv[1], &q, &len)) return throw_status(env, BBQ_ERR_NULL);
+  if (napi_get_value_uint32(env, argv[2], &nq) != napi_ok || napi_get_value_int64(env, argv[3], &k) != napi_ok)
+    return throw_invalid(env, "nq / k must be numbers");
+  if (len != (size_t)nq * bbq_group_index_dim(gi)) return throw_status(env, BBQ_ERR_DIM_MISMATCH);
+  const int64_t n = (int64_t)bbq_group_index_size(gi);
+  int64_t kcap = k > n ? n : k;
+  if (kcap > 4096) return throw_status(env, BBQ_ERR_UNSUPPORTED);
+  const int64_t kcall = k < 0 ? k : kcap;
+  const size_t slots = (size_t)nq * (size_t)(kcap > 0 ? kcap : 0);
+  napi_value out, abi, abs_, ti, ts, v;
+  void* pi = new_buffer(env, slots * sizeof(int32_t), &abi);
+  void* ps = pi ? new_buffer(env, slots * sizeof(float), &abs_) : NULL;
+  if (!pi || !ps) return NULL;
+  const int st = bbq_group_search(gi, q, nq, kcall, (int32_t*)pi, (float*)ps, &count);
+  if (st != BBQ_OK) return throw_status(env, st);
+  napi_create_typedarray(env, napi_int32_array, slots, abi, 0, &ti);
+  napi_create_typedarray(env, napi_float32_array, slots, abs_, 0, &ts);
+  napi_create_object(env, &out);
+  napi_set_named_property(env, out, "indices", ti);
+  napi_set_named_property(env, out, "scores", ts);
+  napi_create_uint32(env, count, &v);
+  napi_set_named_property(env, out, "count", v);
+  napi_create_uint32(env, (uint32_t)(kcap > 0 ? kcap : 0), &v);
+  napi_set_named_property(env, out, "stride", v);
+  return out;
+}
+
+/* groupSearchRerank(groupIndex, queriesFlat, nq, k, oversampleFactor) -> as searchRerank() */
+static napi_value n_group_search_rerank(napi_env env, napi_callback_info info) {
+  ARGS(5);
+  const float* q;
+  size_t len;
+  uint32_t nq, k, factor, count = 0;
+  bbq_group_index* gi = group_index_of(env, argv[0]);
+  if (!get_f32(env, argv[1], &q, &len)) return throw_status(env, BBQ_ERR_NULL);
+  napi_get_value_uint32(env, argv[2], &nq);
+  napi_get_value_uint32(env, argv[3], &k);
+  napi_get_value_uint32(env, argv[4], &factor);
+  if (len != (size_t)nq * bbq_group_index_dim(gi)) return throw_status(env, BBQ_ERR_DIM_MISMATCH);
+  if (k > 4096) return throw_status(env, BBQ_ERR_UNSUPPORTED);
+  const size_t slots = (size_t)nq * k;
+  napi_value out, a1, a2, a3, t1, t2, t3, v;
+  void* p1 = new_buffer(env, slots * sizeof(int32_t), &a1);
+  void* p2 = p1 ? new_buffer(env, slots * sizeof(float), &a2) : NULL;
+  void* p3 = p2 ? new_buffer(env, slots * sizeof(double), &a3) : NULL;
+  if (!p1 || !p2 || !p3) return NULL;
+  const int st = bbq_group_search_rerank(gi, q, nq, k, factor, (int32_t*)p1, (float*)p2, (double*)p3, &count);
+  if (st != BBQ_OK) return throw_status(env, st);
+  napi_create_typedarray(env, napi_int32_array, slots, a1, 0, &t1);
+  napi_create_typedarray(env, napi_float32_array, slots, a2, 0, &t2);
+  napi_create_typedarray(env, napi_float64_array, slots, a3, 0, &t3);
+  napi_create_object(env, &out);
+  napi_set_named_property(env, out, "indices", t1);
+  napi_set_named_property(env, out, "quantizedScores", t2);
+  napi_set_named_property(env, out, "trueScores", t3);
+  napi_create_uint32(env, count, &v);
+  napi_set_named_property(env, out, "count", v);
+  return out;
+}
+
 NAPI_MODULE_INIT() {
   const napi_property_descriptor props[] = {
       {"create", NULL, n_create, NULL, NULL, NULL, 0, NULL}, {"build", NULL, n_build, NULL, NULL, NULL, 0, NULL},
@@ -457,7 +727,18 @@ NAPI_MODULE_INIT() {
       {"searchSharded", NULL, n_search_sharded, NULL, NULL, NULL, 0, NULL},
       {"commUniqueId", NULL, n_comm_unique_id, NULL, NULL, NULL, 0, NULL},
       {"commInit", NULL, n_comm_init, NULL, NULL, NULL, 0, NULL},
-      {"setBase", NULL, n_set_base, NULL, NULL, NULL, 0, NULL}};
+      {"setBase", NULL, n_set_base, NULL, NULL, NULL, 0, NULL},
+      {"groupCreate", NULL, n_group_create, NULL, NULL, NULL, 0, NULL},
+      {"groupContext", NULL, n_group_context, NULL, NULL, NULL, 0, NULL},
+      {"groupBuild", NULL, n_group_build, NULL, NULL, NULL, 0, NULL},
+      {"groupFromQuantized", NULL, n_group_from_quantized, NULL, NULL, NULL, 0, NULL},
+      {"groupLoadIndex", NULL, n_group_load_index, NULL, NULL, NULL, 0, NULL},
+      {"groupSaveIndex", NULL, n_group_save_index, NULL, NULL, NULL, 0, NULL},
+      {"groupInfo", NULL, n_group_info, NULL, NULL, NULL, 0, NULL},
+      {"groupRows", NULL, n_group_rows, NULL, NULL, NULL, 0, NULL},
+      {"groupAttachRows", NULL, n_group_attach_rows, NULL, NULL, NULL, 0, NULL},
+      {"groupSearch", NULL, n_group_search, NULL, NULL, NULL, 0, NULL},
+      {"groupSearchRerank", NULL, n_group_search_rerank, NULL, NULL, NULL, 0, NULL}};
   napi_define_properties(env, exports, sizeof props / sizeof props[0], props);
   return exports;
 }

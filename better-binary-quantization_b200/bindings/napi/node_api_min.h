@@ -41,5 +41,7 @@ napi_status napi_get_named_property(napi_env, napi_value object, const char* nam
 napi_status napi_define_properties(napi_env, napi_value object, size_t count, const napi_property_descriptor*);
 napi_status napi_throw_error(napi_env, const char* code, const char* msg);
 napi_status napi_get_undefined(napi_env, napi_value* result);
+napi_status napi_create_reference(napi_env, napi_value value, uint32_t initial_refcount, napi_ref* result);
+napi_status napi_delete_reference(napi_env, napi_ref ref);
 #define NAPI_MODULE_INIT() napi_value napi_register_module_v1(napi_env env, napi_value exports)
 #endif

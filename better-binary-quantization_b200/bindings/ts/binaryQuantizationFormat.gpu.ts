@@ -52,6 +52,19 @@ const addon = require('./bbq_b200.node') as {
   commUniqueId(): Uint8Array;
   commInit(ctx: Handle, id: Uint8Array, rank: number, world: number): void;
   setBase(index: Handle, base: number): void;
+  groupCreate(queryBits: number, indexBits: number, sim: number, lambda: number, iters: number, devices: Int32Array): Handle;
+  groupContext(group: Handle): Handle;
+  groupBuild(group: Handle, rows: Float32Array, n: number, dim: number, centroid: Float32Array | null): Handle;
+  groupFromQuantized(group: Handle, packed: Uint8Array, corrections: Float64Array, centroid: Float32Array, n: number, dim: number): Handle;
+  groupLoadIndex(group: Handle, veb: string, vemb: string): Handle;
+  groupSaveIndex(index: Handle, veb: string, vemb: string): void;
+  groupInfo(index: Handle): { size: number; dimension: number; centroid: Float32Array; centroidDP: number };
+  groupRows(index: Handle, first: number, count: number): { packed: Uint8Array; corrections: Float64Array };
+  groupAttachRows(index: Handle, rows: Float32Array): void;
+  groupSearch(index: Handle, queries: Float32Array, nq: number, k: number):
+    { indices: Int32Array; scores: Float32Array; count: number; stride: number };
+  groupSearchRerank(index: Handle, queries: Float32Array, nq: number, k: number, factor: number):
+    { indices: Int32Array; quantizedScores: Float32Array; trueScores: Float64Array; count: number };
 };
 
 const SIM_CODE: Record<string, number> = { EUCLIDEAN: 0, COSINE: 1, MAXIMUM_INNER_PRODUCT: 2 };
@@ -68,10 +81,16 @@ function flatten(vectors: Float32Array[], dim: number): Float32Array {
   return flat;
 }
 
-/** src/binaryQuantizationFormat.ts:24-126 — the index now lives in HBM; this object is a handle. */
+/** src/binaryQuantizationFormat.ts:24-126 — the index now lives in HBM; this object is a handle.  `grouped`: an index
+ *  of a device group, one row shard per GPU (its members read through the group entries). */
 class DeviceBinarizedByteVectorValues implements BinarizedByteVectorValues {
   private readonly meta: { size: number; dimension: number; centroid: Float32Array; centroidDP: number };
-  constructor(public readonly handle: Handle) { this.meta = addon.info(handle); }
+  constructor(public readonly handle: Handle, public readonly grouped = false) {
+    this.meta = grouped ? addon.groupInfo(handle) : addon.info(handle);
+  }
+  rows(first: number, count: number): { packed: Uint8Array; corrections: Float64Array } {
+    return this.grouped ? addon.groupRows(this.handle, first, count) : addon.rows(this.handle, first, count);
+  }
   dimension(): number { return this.meta.dimension; }                       // :45
   size(): number { return this.meta.size; }                                 // :49
   getCentroid(): Float32Array { return this.meta.centroid; }                // :123
@@ -83,7 +102,7 @@ class DeviceBinarizedByteVectorValues implements BinarizedByteVectorValues {
   }
   vectorValue(ord: number): Uint8Array {                                    // :53 (lazy device->host copy)
     if (ord < 0 || ord >= this.meta.size) throw new Error(`向量索引 ${ord} 不存在`);
-    return addon.rows(this.handle, ord, 1).packed;
+    return this.rows(ord, 1).packed;
   }
   getUnpackedVector(ord: number): Uint8Array {                              // :68
     if (ord < 0 || ord >= this.meta.size) throw new Error(`未打包向量索引 ${ord} 不存在`);
@@ -94,29 +113,50 @@ class DeviceBinarizedByteVectorValues implements BinarizedByteVectorValues {
   }
   getCorrectiveTerms(ord: number): QuantizationResult {                     // :105
     if (ord < 0 || ord >= this.meta.size) throw new Error(`修正项索引 ${ord} 不存在`);
-    const c = addon.rows(this.handle, ord, 1).corrections;
+    const c = this.rows(ord, 1).corrections;
     return { lowerInterval: c[0]!, upperInterval: c[1]!, additionalCorrection: c[2]!, quantizedComponentSum: c[3]! };
   }
   clearUnpackedVectorCache(): void { /* nothing is cached on the host */ }
 }
 
-function deviceHandle(targetVectors: BinarizedByteVectorValues): Handle {
+function deviceIndex(targetVectors: BinarizedByteVectorValues): DeviceBinarizedByteVectorValues {
   if (!(targetVectors instanceof DeviceBinarizedByteVectorValues))
     throw new Error('[bbq-b200] 目标向量集合 is not a device index (build it with quantizeVectors / deserializeVectorData of this class)');
-  return targetVectors.handle;
+  return targetVectors;
 }
+function deviceHandle(targetVectors: BinarizedByteVectorValues): Handle { return deviceIndex(targetVectors).handle; }
+
+/** The GPUs of a device group: config.devices, else BBQ_DEVICES=0,1,... in the environment; null without either. */
+function groupDevices(config: BinaryQuantizationConfig): number[] | null {
+  const given = (config as BinaryQuantizationConfig & { devices?: number[] }).devices;
+  if (given !== undefined && given !== null) return given;
+  const env = process.env.BBQ_DEVICES;
+  if (env === undefined || env.trim() === '') return null;
+  return env.split(',').map((d) => Number(d.trim()));
+}
+const GROUP_NOT_SHARDED = '[bbq-b200] this format drives a device group, which is already sharded over its GPUs: ' +
+  'sharded = true and joinShardGroup do not apply';
 
 export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat {
   private readonly ctx: Handle;
+  /** A device group over config.devices / BBQ_DEVICES (one process, every GPU listed), or null: one GPU. */
+  private readonly group: Handle | null = null;
 
   constructor(config: BinaryQuantizationConfig) {                            // :141-158 (super validates 1..8)
     super(config);
     const cfg = { queryBits: QUERY_BITS, indexBits: INDEX_BITS, ...config };
     const q = config.quantizer;
+    const sim = SIM_CODE[q.similarityFunction ?? VectorSimilarityFunction.EUCLIDEAN]!;
+    const devices = groupDevices(config);
     try {
-      this.ctx = addon.create(cfg.queryBits!, cfg.indexBits!,
-        SIM_CODE[q.similarityFunction ?? VectorSimilarityFunction.EUCLIDEAN]!, q.lambda ?? 0.1, q.iters ?? 5,
-        Number(process.env.BBQ_DEVICE ?? -1));
+      if (devices === null) {
+        this.ctx = addon.create(cfg.queryBits!, cfg.indexBits!, sim, q.lambda ?? 0.1, q.iters ?? 5,
+          Number(process.env.BBQ_DEVICE ?? -1));
+      } else {
+        this.group = addon.groupCreate(cfg.queryBits!, cfg.indexBits!, sim, q.lambda ?? 0.1, q.iters ?? 5,
+          Int32Array.from(devices));
+        this.ctx = addon.groupContext(this.group);   // the group's first GPU: quantizeQueryVector, accuracy
+      }
     } catch (e) { throw toReferenceError(e, 'build'); }
   }
 
@@ -126,10 +166,15 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
   public override quantizeVectors(vectors: Float32Array[], sharded = false): {              // :165-263
     quantizedVectors: BinarizedByteVectorValues; queryQuantizer: OptimizedScalarQuantizer;
   } {
+    if (this.group !== null && sharded) throw new Error(GROUP_NOT_SHARDED);
     if (vectors.length === 0 && !sharded) throw new Error('向量集合不能为空');
     const dim = vectors.length === 0 ? 0 : vectors[0]!.length;
     const flat = flatten(vectors, dim);
     try {
+      if (this.group !== null) {
+        const handle = addon.groupBuild(this.group, flat, vectors.length, dim, null);
+        return { quantizedVectors: new DeviceBinarizedByteVectorValues(handle, true), queryQuantizer: this.getQuantizer() };
+      }
       const handle = sharded ? addon.buildSharded(this.ctx, flat, vectors.length, dim, null)
                              : addon.build(this.ctx, flat, vectors.length, dim, null);
       // :261 hands out `this.quantizer` (an OptimizedScalarQuantizer): the inherited helper object, as getQuantizer() does
@@ -157,7 +202,9 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
     if (k === 0) return [];
     try {
       // a fractional k: the reference's heap loop (`size() < k2`, :386-389) ends up with ceil(k) results
-      const r = addon.search(deviceHandle(targetVectors), queryVector, 1, Math.ceil(k));
+      const ix = deviceIndex(targetVectors);
+      const r = ix.grouped ? addon.groupSearch(ix.handle, queryVector, 1, Math.ceil(k))
+                           : addon.search(ix.handle, queryVector, 1, Math.ceil(k));
       const out = new Array(r.count);
       for (let i = 0; i < r.count; i++) out[i] = { index: r.indices[i]!, score: r.scores[i]! };
       return out;
@@ -183,7 +230,7 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
   public override serializeVectorData(vectors: Float32Array[]): { vectorData: VectorDataFormat[]; metadata: MetadataFormat } {  // :483-525
     const { quantizedVectors } = this.quantizeVectors(vectors);
     const n = quantizedVectors.size(), centroid = quantizedVectors.getCentroid();
-    const all = addon.rows(deviceHandle(quantizedVectors), 0, n);
+    const all = deviceIndex(quantizedVectors).rows(0, n);
     const p = Math.ceil(centroid.length / 8);
     const vectorData: VectorDataFormat[] = [];
     for (let i = 0; i < n; i++) {
@@ -207,6 +254,8 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
       corr.set([d.lowerInterval, d.upperInterval, d.additionalCorrection, d.quantizedComponentSum], 4 * i);
     });
     try {
+      if (this.group !== null)
+        return new DeviceBinarizedByteVectorValues(addon.groupFromQuantized(this.group, packed, corr, metadata.centroid, n, dim), true);
       return new DeviceBinarizedByteVectorValues(addon.fromQuantized(this.ctx, packed, corr, metadata.centroid, n, dim));
     } catch (e) { throw toReferenceError(e, 'build'); }
   }
@@ -217,6 +266,7 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
 
   /** A batch of queries in one call; row i equals searchNearestNeighbors(queries[i], ...). */
   public searchBatch(queries: Float32Array[], targetVectors: BinarizedByteVectorValues, k: number, sharded = false) {
+    if (this.group !== null && sharded) throw new Error(GROUP_NOT_SHARDED);
     const dim = targetVectors.dimension();
     const flat = new Float32Array(queries.length * dim);
     queries.forEach((q, i) => {
@@ -224,8 +274,9 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
       flat.set(q, i * dim);
     });
     try {
-      const h = deviceHandle(targetVectors);
-      const r = sharded ? addon.searchSharded(h, flat, queries.length, k) : addon.search(h, flat, queries.length, k);
+      const ix = deviceIndex(targetVectors), h = ix.handle;
+      const r = ix.grouped ? addon.groupSearch(h, flat, queries.length, k)
+              : sharded ? addon.searchSharded(h, flat, queries.length, k) : addon.search(h, flat, queries.length, k);
       return queries.map((_, i) => Array.from({ length: r.count }, (_u, j) =>
         ({ index: r.indices[i * r.stride + j]!, score: r.scores[i * r.stride + j]! })));
     } catch (e) { throw toReferenceError(e, 'search'); }
@@ -238,6 +289,7 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
    *  base). */
   public static createShardGroupId(): Uint8Array { return addon.commUniqueId(); }
   public joinShardGroup(id: Uint8Array, rank: number, world: number, shard?: BinarizedByteVectorValues, baseRow?: number): void {
+    if (this.group !== null) throw new Error(GROUP_NOT_SHARDED);
     try {
       addon.commInit(this.ctx, id, rank, world);
       if (shard !== undefined) addon.setBase(deviceHandle(shard), baseRow ?? 0);
@@ -248,16 +300,22 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
    *  exact cosine against the attached original rows, best k by true score. */
   public attachOriginalVectors(targetVectors: BinarizedByteVectorValues, vectors: Float32Array[]): void {
     const flat = flatten(vectors, targetVectors.dimension());
-    try { addon.attachRows(deviceHandle(targetVectors), flat); }
+    try {
+      const ix = deviceIndex(targetVectors);
+      if (ix.grouped) addon.groupAttachRows(ix.handle, flat);
+      else addon.attachRows(ix.handle, flat);
+    }
     catch (e) { throw toReferenceError(e, 'build'); }
   }
   /** With sharded = true (after joinShardGroup, each rank's own rows attached) the re-rank runs over ALL row shards
    *  of the box and returns, on every rank, what the unsharded call returns on the whole corpus. */
   public searchOversampled(queryVector: Float32Array, targetVectors: BinarizedByteVectorValues, k: number,
       oversampleFactor: number, sharded = false): Array<{ index: number; quantizedScore: number; trueScore: number }> {
+    if (this.group !== null && sharded) throw new Error(GROUP_NOT_SHARDED);
     try {
-      const h = deviceHandle(targetVectors);
-      const r = sharded ? addon.searchRerankSharded(h, queryVector, 1, k, oversampleFactor)
+      const ix = deviceIndex(targetVectors), h = ix.handle;
+      const r = ix.grouped ? addon.groupSearchRerank(h, queryVector, 1, k, oversampleFactor)
+              : sharded ? addon.searchRerankSharded(h, queryVector, 1, k, oversampleFactor)
                         : addon.searchRerank(h, queryVector, 1, k, oversampleFactor);
       return Array.from({ length: r.count }, (_u, i) =>
         ({ index: r.indices[i]!, quantizedScore: r.quantizedScores[i]!, trueScore: r.trueScores[i]! }));
@@ -269,14 +327,19 @@ export class BinaryQuantizationFormat extends ReferenceBinaryQuantizationFormat 
    *  With sharded = true (after joinShardGroup) both are collective: every rank saves its own rows into ONE image of
    *  the whole corpus, or loads its own row range of one image (its base set), on any number of ranks. */
   public saveIndex(targetVectors: BinarizedByteVectorValues, prefix: string, sharded = false): void {
+    if (this.group !== null && sharded) throw new Error(GROUP_NOT_SHARDED);
     try {
-      const h = deviceHandle(targetVectors);
-      if (sharded) addon.saveIndexSharded(h, `${prefix}.veb`, `${prefix}.vemb`);
+      const ix = deviceIndex(targetVectors), h = ix.handle;
+      if (ix.grouped) addon.groupSaveIndex(h, `${prefix}.veb`, `${prefix}.vemb`);
+      else if (sharded) addon.saveIndexSharded(h, `${prefix}.veb`, `${prefix}.vemb`);
       else addon.saveIndex(h, `${prefix}.veb`, `${prefix}.vemb`);
     } catch (e) { throw toReferenceError(e, 'build'); }
   }
   public loadIndex(prefix: string, sharded = false): BinarizedByteVectorValues {
+    if (this.group !== null && sharded) throw new Error(GROUP_NOT_SHARDED);
     try {
+      if (this.group !== null)
+        return new DeviceBinarizedByteVectorValues(addon.groupLoadIndex(this.group, `${prefix}.veb`, `${prefix}.vemb`), true);
       const h = sharded ? addon.loadIndexSharded(this.ctx, `${prefix}.veb`, `${prefix}.vemb`)
                         : addon.loadIndex(this.ctx, `${prefix}.veb`, `${prefix}.vemb`);
       return new DeviceBinarizedByteVectorValues(h);

@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -129,15 +130,27 @@ struct bbq_ctx {
   uint32_t* h_flag = nullptr;  // pinned: [0..nq) candidate counts, [nq] overflow flag, then 2 words: first invalid query
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;  // ordering between the context's stream and a caller's stream (StreamBridge)
   // sharded search (bbq_comm_init): one NCCL communicator per context = per GPU = per process
-  ncclComm_t comm = nullptr;
+  // atomic: a device group's caller thread clears it (then aborts the communicator) while the workers may read it
+  std::atomic<ncclComm_t> comm{nullptr};
   int rank = 0, world = 1;
   DevBuf keys_local, keys_all, loc_idx, loc_score, bad, nglob;
+  const bbq_group* group = nullptr;  // the device group that owns this context: its collectives run on that group's worker
   // profiling (bbq_set_profiling): event pairs per kernel group, drained by bbq_get_stats
   bool profiling = false;
   struct EvPair { cudaEvent_t a, b; int kind; };
   std::vector<EvPair> ev_pending;
   std::vector<cudaEvent_t> ev_pool;
 };
+
+// The worker thread of a device group runs the collective entries of its own context; anyone else calling them on a
+// group's context would wait forever for peers that are not coming.
+static thread_local const bbq_ctx* t_group_worker = nullptr;
+static int group_guard(const bbq_ctx* c) {
+  if (c->group && t_group_worker != c)
+    return fail(BBQ_ERR_INVALID_ARG, "this context belongs to a device group: its collective entries run through the "
+                                     "bbq_group_* entries");
+  return BBQ_OK;
+}
 
 enum { PROF_SCAN = 0, PROF_QUANT = 1, PROF_SELECT = 2, PROF_SAMPLE = 3 };
 struct ProfScope {  // records an event pair around a group of launches when profiling is on
@@ -232,18 +245,29 @@ extern "C" void bbq_last_error_pos(int64_t* vector, int64_t* position) {
   if (position) *position = g_err_pos;
 }
 
-extern "C" int bbq_create(const bbq_config* config, bbq_ctx** out_ctx) {
-  if (!config || !out_ctx) return fail(BBQ_ERR_NULL, "config/out_ctx is null");
-  *out_ctx = nullptr;
-  // src/binaryQuantizationFormat.ts:143-148
+// src/binaryQuantizationFormat.ts:143-148
+static int check_config(const bbq_config* config) {
   if (config->query_bits < 1 || config->query_bits > 8) return fail(BBQ_ERR_QUERY_BITS, "queryBits must be in 1..8");
   if (config->index_bits < 1 || config->index_bits > 8) return fail(BBQ_ERR_INDEX_BITS, "indexBits must be in 1..8");
   if (config->similarity > 2) return fail(BBQ_ERR_INVALID_ARG, "unknown similarity function");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+  return BBQ_OK;
+}
+static int device_count(int* ndev) {
+  *ndev = 0;
+  if (cudaGetDeviceCount(ndev) != cudaSuccess || *ndev == 0) {
     cudaGetLastError();
+    *ndev = 0;
     return fail(BBQ_ERR_NO_DEVICE, "no CUDA device: libbbq_b200 has no CPU fallback");
   }
+  return BBQ_OK;
+}
+
+extern "C" int bbq_create(const bbq_config* config, bbq_ctx** out_ctx) {
+  if (!config || !out_ctx) return fail(BBQ_ERR_NULL, "config/out_ctx is null");
+  *out_ctx = nullptr;
+  TRY(check_config(config));
+  int ndev = 0;
+  TRY(device_count(&ndev));
   int dev = config->device;
   if (dev < 0) CU(cudaGetDevice(&dev));
   if (dev >= ndev) return fail(BBQ_ERR_NO_DEVICE, "device ordinal out of range");
@@ -1633,11 +1657,7 @@ struct NcclApi {
   std::string error;
   bool ok = false;
 };
-static NcclApi* nccl_api() {
-  static NcclApi api;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
+static void nccl_load(NcclApi& api) {
     void* h = nullptr;
     const char* names[] = {getenv("BBQ_NCCL_LIB"), "libnccl.so.2", "libnccl.so"};
     for (const char* nm : names) {
@@ -1645,13 +1665,13 @@ static NcclApi* nccl_api() {
     }
     if (!h) {
       api.error = std::string("cannot load NCCL (libnccl.so.2): ") + (dlerror() ? dlerror() : "not found");
-      return &api;
+      return;
     }
 #define BBQ_NCCL_SYM(field, name)                                            \
   api.field = reinterpret_cast<decltype(api.field)>(dlsym(h, name));        \
   if (!api.field) {                                                          \
     api.error = std::string("NCCL symbol missing: ") + name;                 \
-    return &api;                                                             \
+    return;                                                                  \
   }
     BBQ_NCCL_SYM(GetUniqueId, "ncclGetUniqueId")
     BBQ_NCCL_SYM(CommInitRank, "ncclCommInitRank")
@@ -1663,7 +1683,12 @@ static NcclApi* nccl_api() {
     BBQ_NCCL_SYM(GetVersion, "ncclGetVersion")
 #undef BBQ_NCCL_SYM
     api.ok = true;
-  }
+}
+// the workers of a device group reach this at the same time
+static NcclApi* nccl_api() {
+  static NcclApi api;
+  static std::once_flag once;
+  std::call_once(once, nccl_load, std::ref(api));
   return &api;
 }
 #define NC(expr)                                                                                        \
@@ -1697,6 +1722,7 @@ extern "C" int bbq_comm_unique_id(uint8_t* out_id) {
 
 extern "C" int bbq_comm_init(bbq_ctx* c, const uint8_t* id_bytes, int rank, int world) {
   if (!c || !id_bytes) return fail(BBQ_ERR_NULL, "null");
+  TRY(group_guard(c));
   if (world < 1 || rank < 0 || rank >= world) return fail(BBQ_ERR_INVALID_ARG, "rank/world out of range");
   if (c->comm) return fail(BBQ_ERR_INVALID_ARG, "this context already has a communicator");
   NcclApi* a = nccl_api();
@@ -1704,7 +1730,9 @@ extern "C" int bbq_comm_init(bbq_ctx* c, const uint8_t* id_bytes, int rank, int 
   CU(cudaSetDevice(c->device));
   ncclUniqueId id;
   memcpy(&id, id_bytes, sizeof id);
-  NC(a->CommInitRank(&c->comm, world, id, rank));
+  ncclComm_t comm = nullptr;
+  NC(a->CommInitRank(&comm, world, id, rank));
+  c->comm = comm;
   c->rank = rank;
   c->world = world;
   return BBQ_OK;
@@ -1712,6 +1740,7 @@ extern "C" int bbq_comm_init(bbq_ctx* c, const uint8_t* id_bytes, int rank, int 
 
 extern "C" int bbq_comm_destroy(bbq_ctx* c) {
   if (!c) return fail(BBQ_ERR_NULL, "null");
+  TRY(group_guard(c));
   CU(cudaSetDevice(c->device));
   CU(cudaStreamSynchronize(c->stream));
   if (c->comm) {
@@ -1764,6 +1793,7 @@ extern "C" int bbq_search_sharded_device(bbq_index* ix, const float* d_queries, 
   if (nq == 0 || k == 0) return BBQ_OK;
   if (k > K_MAX) return fail(BBQ_ERR_UNSUPPORTED, "k > 4096 is not supported by the device top-k");
   bbq_ctx* c = ix->ctx;
+  TRY(group_guard(c));
   if (!c->comm || c->world == 1) return bbq_search_device(ix, d_queries, nq, k, d_out_idx, d_out_score, stream);
   CU(cudaSetDevice(c->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
@@ -1794,6 +1824,7 @@ extern "C" int bbq_search_sharded(bbq_index* ix, const float* queries, uint32_t 
   if (k == 0 || nq == 0) return BBQ_OK;
   if (!out_idx || !out_score) return fail(BBQ_ERR_NULL, "output buffers must not be null");
   bbq_ctx* c = ix->ctx;
+  TRY(group_guard(c));
   if (!c->comm || c->world == 1) return bbq_search(ix, queries, nq, k, out_idx, out_score, out_count);  // one shard: the plain entry
   CU(cudaSetDevice(c->device));
   uint64_t n_all = 0;
@@ -1886,6 +1917,7 @@ extern "C" int bbq_search_rerank_sharded(bbq_index* ix, const float* queries, ui
   if (!ix) return fail(BBQ_ERR_NULL, "target vector set must not be null");
   if (!queries) return fail(BBQ_ERR_NULL, "query vector must not be null");
   bbq_ctx* c = ix->ctx;
+  TRY(group_guard(c));
   if (!c->comm || c->world == 1)  // one shard: the plain entry
     return bbq_search_rerank(ix, queries, nq, k, factor, out_idx, out_qscore, out_true, out_count);
   // the replicated arguments: every rank reaches the same verdict on them without communicating
@@ -1956,12 +1988,16 @@ static int finish_shard(bbq_index* ix, const float* d_sum, const float* centroid
   return bbq_index_set_base(ix, base);
 }
 
+// rows_validated: the caller has validated the host rows already (a device group does it before any collective)
 static int build_sharded(bbq_ctx* c, const float* rows, bool is_host, uint64_t n, uint32_t dim, const float* centroid,
-                         bbq_index** out_index) {
+                         bbq_index** out_index, bool rows_validated = false) {
   if (!c) return fail(BBQ_ERR_NULL, "null ctx/out_index");
-  if (!c->comm || c->world == 1)  // one shard: the plain entry
+  TRY(group_guard(c));
+  if (!c->comm || c->world == 1) {  // one shard: the plain entry
+    if (is_host && rows_validated) return build_impl(c, rows, true, n, dim, centroid, out_index);
     return is_host ? bbq_index_build(c, rows, n, dim, centroid, out_index)
                    : bbq_index_build_device(c, rows, n, dim, centroid, out_index);
+  }
   if (out_index) *out_index = nullptr;
   CU(cudaSetDevice(c->device));
   const char* what = "sharded build";
@@ -2019,7 +2055,7 @@ static int build_sharded(bbq_ctx* c, const float* rows, bool is_host, uint64_t n
   //    COSINE norms computed ahead of its turn in the chain
   const bool cosine = c->cfg.similarity == BBQ_SIM_COSINE;
   int64_t bad_vec = -1, bad_pos = -1;
-  st = is_host && n > 0 ? validate_rows(rows, n, D, cosine) : BBQ_OK;
+  st = is_host && n > 0 && !rows_validated ? validate_rows(rows, n, D, cosine) : BBQ_OK;
   if (st != BBQ_OK) {
     bad_vec = (int64_t)base + g_err_vec;
     bad_pos = g_err_pos;
@@ -2231,3 +2267,5 @@ extern "C" int bbq_debug_qcdist_batch(bbq_index* ix, const float* queries, uint3
   }
   return BBQ_OK;
 }
+
+#include "bbq_group.cuh"  // device groups: one process, one caller thread, the collectives above on every GPU

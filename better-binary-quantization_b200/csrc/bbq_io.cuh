@@ -491,6 +491,7 @@ extern "C" int bbq_index_save_sharded(const bbq_index* cix, const char* veb_path
   bbq_index* ix = const_cast<bbq_index*>(cix);
   if (!ix) return fail(BBQ_ERR_NULL, "null index/path");
   bbq_ctx* c = ix->ctx;
+  TRY(group_guard(c));
   if (!c->comm || c->world == 1) return bbq_index_save(ix, veb_path, vemb_path);  // one shard: the plain entry
   CU(cudaSetDevice(c->device));
   std::vector<RankWord> all;
@@ -533,6 +534,7 @@ extern "C" int bbq_index_save_sharded(const bbq_index* cix, const char* veb_path
 extern "C" int bbq_index_load_sharded(bbq_ctx* c, const char* veb_path, const char* vemb_path, bbq_index** out_index) {
   if (!c || !out_index) return fail(BBQ_ERR_NULL, "null ctx/out_index");
   *out_index = nullptr;
+  TRY(group_guard(c));
   if (!c->comm || c->world == 1) return bbq_index_load(c, veb_path, vemb_path, out_index);  // one shard: the plain entry
   CU(cudaSetDevice(c->device));
   // 1. the header this rank reads decides its range (the split of host/sharded.py:shard_bounds); 2. its rows

@@ -79,28 +79,18 @@ def _as_matrix(vectors) -> np.ndarray:
     return np.ascontiguousarray(np.stack(rows), dtype=np.float32)
 
 
-class BinarizedByteVectorValues:
-    """Device-resident index shard.  size()/dimension()/getCentroid() answer from cached host metadata;
-    vectorValue()/getCorrectiveTerms() do a lazy device->host copy (cold path, SURVEY §8b)."""
+class _VectorValues:
+    """The read-only members of src/types.ts:32-49 over a device index, whatever its handle type.
+    size()/dimension()/getCentroid() answer from cached host metadata; vectorValue()/getCorrectiveTerms() do a lazy
+    device->host copy (cold path, SURVEY §8b) through _export_rows, which each handle type provides."""
 
-    def __init__(self, fmt: "BinaryQuantizationFormat", handle):
-        self._fmt = fmt
-        self._h = handle
-        L = _native.load()
-        self._n = int(L.bbq_index_size(handle))
-        self._dim = int(L.bbq_index_dim(handle))
+    def _read_meta(self, size, dim, centroid):
+        self._n = int(size(self._h))
+        self._dim = int(dim(self._h))
         c = np.empty(self._dim, np.float32)
         cdp = C.c_double()
-        _check(L.bbq_index_centroid(handle, c.ctypes.data, C.byref(cdp)))
+        _check(centroid(self._h, c.ctypes.data, C.byref(cdp)))
         self._centroid, self._cdp = c, cdp.value
-
-    def __del__(self):
-        try:
-            if self._h is not None:
-                _native.load().bbq_index_destroy(self._h)
-                self._h = None
-        except Exception:
-            pass
 
     def dimension(self) -> int:
         return self._dim
@@ -128,7 +118,7 @@ class BinarizedByteVectorValues:
         p = (self._dim + 7) // 8 if self._fmt.config["indexBits"] == 1 else self._dim
         packed = np.empty((count, p), np.uint8)
         corr = np.empty((count, 4), np.float64)
-        _check(_native.load().bbq_index_export(self._h, ord_, count, packed.ctypes.data, corr.ctypes.data))
+        self._export_rows(ord_, count, packed.ctypes.data, corr.ctypes.data)
         return packed, corr
 
     def vectorValue(self, ord_: int) -> np.ndarray:
@@ -150,8 +140,65 @@ class BinarizedByteVectorValues:
         return self._export(0, self._n)
 
 
+class BinarizedByteVectorValues(_VectorValues):
+    """Device-resident index shard on one GPU (a bbq_index)."""
+
+    def __init__(self, fmt: "BinaryQuantizationFormat", handle):
+        self._fmt = fmt
+        self._h = handle
+        L = _native.load()
+        self._read_meta(L.bbq_index_size, L.bbq_index_dim, L.bbq_index_centroid)
+
+    def __del__(self):
+        try:
+            if self._h is not None:
+                _native.load().bbq_index_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def _export_rows(self, first, count, packed, corr):
+        _check(_native.load().bbq_index_export(self._h, first, count, packed, corr))
+
+
+class GroupBinarizedByteVectorValues(_VectorValues):
+    """An index of a device group: one row shard per GPU of the group (a bbq_group_index), the same read-only members
+    as BinarizedByteVectorValues.  vectorValue()/getCorrectiveTerms() read from the shard that holds the row.  It is
+    not a BinarizedByteVectorValues: its handle never reaches a bbq_index_* entry (_index refuses it)."""
+
+    def __init__(self, fmt: "BinaryQuantizationFormat", handle):
+        self._fmt = fmt
+        self._h = handle
+        L = _native.load()
+        self._read_meta(L.bbq_group_index_size, L.bbq_group_index_dim, L.bbq_group_index_centroid)
+
+    def __del__(self):
+        try:
+            if self._h is not None:
+                _native.load().bbq_group_index_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def _export_rows(self, first, count, packed, corr):
+        _check(_native.load().bbq_group_index_export(self._h, first, count, packed, corr))
+
+
+def _index(targetVectors):
+    """The bbq_index* of a one-GPU index, for the entries that take one.  A device group's index is another type in C
+    (bbq_group_index*): it is refused here, never handed over."""
+    if isinstance(targetVectors, GroupBinarizedByteVectorValues):
+        raise BbqError(10, "this member takes an index on one GPU; a device group's index is served by quantizeVectors, "
+                           "searchNearestNeighbors, searchBatch, attachOriginalVectors, searchOversampledBatch, saveIndex "
+                           "and its own members")
+    return targetVectors._h
+
+
 class BinaryQuantizationFormat:
-    def __init__(self, config: dict, device: int = -1):
+    def __init__(self, config: dict, device: int = -1, devices: Optional[Sequence[int]] = None):
+        """devices: the GPUs of a device group (bbq_group_create): one process drives all of them, every index is split
+        into one row shard per GPU, and builds, searches, re-ranks and images run on all of them at once.
+        quantizeQueryVector and computeQuantizationAccuracy run on the group's first GPU."""
         q = config.get("quantizer") or {}
         self.config = {"queryBits": QUERY_BITS, "indexBits": INDEX_BITS, **config}
         cfg = _native.BbqConfig()
@@ -164,15 +211,53 @@ class BinaryQuantizationFormat:
         cfg.iters = int(q.get("iters", 5))
         cfg.device = device
         self._ctx = C.c_void_p()
-        _check(_native.load().bbq_create(C.byref(cfg), C.byref(self._ctx)))
+        self._group = None
+        L = _native.load()
+        if devices is None:
+            _check(L.bbq_create(C.byref(cfg), C.byref(self._ctx)))
+            return
+        devs = (C.c_int32 * max(len(devices), 1))(*[int(d) for d in devices])
+        group = C.c_void_p()
+        _check(L.bbq_group_create(C.byref(cfg), devs, len(devices), C.byref(group)))
+        self._group = group
+        self._in_group = True
+        self._ctx = C.c_void_p(L.bbq_group_context(group, 0))   # owned by the group
 
     def __del__(self):
         try:
-            if getattr(self, "_ctx", None):
+            if getattr(self, "_group", None):
+                _native.load().bbq_group_destroy(self._group)
+                self._group = None
+            elif getattr(self, "_ctx", None) and not getattr(self, "_in_group", False):
                 _native.load().bbq_destroy(self._ctx)
-                self._ctx = None
+            self._ctx = None
         except Exception:
             pass
+
+    def devices(self) -> List[int]:
+        """The GPUs of this format's device group ([] without one)."""
+        if not self._group:
+            return []
+        L = _native.load()
+        n = C.c_uint32(0)
+        _check(L.bbq_group_info(self._group, C.byref(n), None))
+        out = (C.c_int32 * n.value)()
+        _check(L.bbq_group_info(self._group, C.byref(n), out))
+        return list(out)
+
+    def groupContext(self, rank: int) -> int:
+        """The context of rank `rank` of the device group (bbq_group_context), for statistics."""
+        return _native.load().bbq_group_context(self._group, rank)
+
+    def _not_sharded(self, sharded: bool):
+        if sharded and self._group:
+            raise BbqError(10, "a device-group format is already sharded over its GPUs: sharded=True does not apply")
+
+    def _one_gpu(self, member: str):
+        """Device-pointer, streaming, shard-bootstrap and debug members exist for one GPU only: on a device-group format
+        they would act on its first GPU's context alone, so they are refused."""
+        if self._group:
+            raise BbqError(10, f"{member} is not available on a device-group format")
 
     def getConfig(self) -> dict:
         return dict(self.config)
@@ -182,12 +267,17 @@ class BinaryQuantizationFormat:
         """sharded=True: this rank's rows of a corpus split over the communicator in rank order (bbq_index_build_sharded,
         collective); the rank may hold no rows.  Without a centroid every rank gets the reference-order centroid of the
         whole corpus, and its shard (base set) equals its rows of the whole-corpus build."""
+        self._not_sharded(sharded)
         if not sharded and (vectors is None or len(vectors) == 0):
             raise BbqError(3, "向量集合不能为空")
         m = _as_matrix(vectors if vectors is not None else [])
         h = C.c_void_p()
         cen = np.ascontiguousarray(centroid, np.float32) if centroid is not None else None
         L = _native.load()
+        if self._group:
+            _check(L.bbq_group_index_build(self._group, m.ctypes.data, m.shape[0], m.shape[1],
+                                           cen.ctypes.data if cen is not None else None, C.byref(h)), "build")
+            return {"quantizedVectors": GroupBinarizedByteVectorValues(self, h), "queryQuantizer": self}
         if sharded:
             dim = m.shape[1] if m.shape[0] else (cen.size if cen is not None else 0)
             _check(L.bbq_index_build_sharded(self._ctx, m.ctypes.data, m.shape[0], dim,
@@ -203,6 +293,8 @@ class BinaryQuantizationFormat:
                               sharded: bool = False):
         """Rows already in device memory (e.g. a torch tensor's data_ptr()).  sharded=True: as quantizeVectors
         (bbq_index_build_sharded_device, collective)."""
+        self._one_gpu("quantizeVectorsDevice")
+        self._not_sharded(sharded)
         h = C.c_void_p()
         cen = np.ascontiguousarray(centroid, np.float32) if centroid is not None else None
         L = _native.load()
@@ -215,6 +307,7 @@ class BinaryQuantizationFormat:
         """The reference centroid's running sum (f32[dim], updated in place and returned) continued over the rows that
         follow the corpus's first rowsBefore rows: host `rows`, or n device rows at d_rows_ptr
         (bbq_centroid_accumulate / _device).  rowsBefore == 0 starts the corpus."""
+        self._one_gpu("accumulateCentroid")
         if running.dtype != np.float32 or not running.flags.c_contiguous:
             raise BbqError(10, "running must be a contiguous float32 array")
         L = _native.load()
@@ -239,19 +332,21 @@ class BinaryQuantizationFormat:
 
     def reserveIndex(self, capacity: int, dim: int, centroid) -> BinarizedByteVectorValues:
         """Streaming build (bbq_index_reserve): explicit centroid, rows appended chunk by chunk."""
+        self._one_gpu("reserveIndex")
         cen = np.ascontiguousarray(centroid, np.float32)
         h = C.c_void_p()
         _check(_native.load().bbq_index_reserve(self._ctx, capacity, dim, cen.ctypes.data, C.byref(h)), "build")
         return BinarizedByteVectorValues(self, h)
 
     def appendRows(self, targetVectors: BinarizedByteVectorValues, rows=None, d_rows_ptr: int = 0, n: int = 0):
+        self._one_gpu("appendRows")
         L = _native.load()
         if rows is not None:
             m = _as_matrix(rows)
-            _check(L.bbq_index_append(targetVectors._h, m.ctypes.data, m.shape[0]), "build")
+            _check(L.bbq_index_append(_index(targetVectors), m.ctypes.data, m.shape[0]), "build")
         else:
-            _check(L.bbq_index_append_device(targetVectors._h, d_rows_ptr, n), "build")
-        targetVectors._n = int(L.bbq_index_size(targetVectors._h))
+            _check(L.bbq_index_append_device(_index(targetVectors), d_rows_ptr, n), "build")
+        targetVectors._n = int(L.bbq_index_size(_index(targetVectors)))
 
     def adoptQuantized(self, packed, corr4, centroid) -> BinarizedByteVectorValues:
         """Index quantised elsewhere (e.g. by the reference): bbq_index_from_quantized."""
@@ -259,6 +354,11 @@ class BinaryQuantizationFormat:
         corr4 = np.ascontiguousarray(corr4, np.float64)
         centroid = np.ascontiguousarray(centroid, np.float32)
         h = C.c_void_p()
+        if self._group:
+            _check(_native.load().bbq_group_index_from_quantized(self._group, packed.ctypes.data, corr4.ctypes.data,
+                                                                 centroid.ctypes.data, packed.shape[0], centroid.size,
+                                                                 C.byref(h)), "build")
+            return GroupBinarizedByteVectorValues(self, h)
         _check(_native.load().bbq_index_from_quantized(self._ctx, packed.ctypes.data, corr4.ctypes.data,
                                                        centroid.ctypes.data, packed.shape[0], centroid.size,
                                                        C.byref(h)), "build")
@@ -274,17 +374,25 @@ class BinaryQuantizationFormat:
         """Writes <prefix>.veb (vector data) and <prefix>.vemb (metadata + centroid): bbq_index_save.  sharded=True: one
         image of all row shards of the communicator, each rank writing its own rows (bbq_index_save_sharded,
         collective); the files equal those of one index holding the whole corpus."""
+        self._not_sharded(sharded)
         veb, vemb = self._image_paths(prefix)
         L = _native.load()
-        fn = L.bbq_index_save_sharded if sharded else L.bbq_index_save
+        if isinstance(targetVectors, GroupBinarizedByteVectorValues):
+            fn = L.bbq_group_index_save
+        else:
+            fn = L.bbq_index_save_sharded if sharded else L.bbq_index_save
         _check(fn(targetVectors._h, veb, vemb), "build")
 
     def loadIndex(self, prefix: str, sharded: bool = False) -> BinarizedByteVectorValues:
         """Reads an image written by saveIndex straight into device memory: bbq_index_load.  sharded=True: this rank's
         row range of the image (shard_bounds), with its base set (bbq_index_load_sharded, collective)."""
+        self._not_sharded(sharded)
         veb, vemb = self._image_paths(prefix)
         h = C.c_void_p()
         L = _native.load()
+        if self._group:
+            _check(L.bbq_group_index_load(self._group, veb, vemb, C.byref(h)), "build")
+            return GroupBinarizedByteVectorValues(self, h)
         fn = L.bbq_index_load_sharded if sharded else L.bbq_index_load
         _check(fn(self._ctx, veb, vemb, C.byref(h)), "build")
         return BinarizedByteVectorValues(self, h)
@@ -292,6 +400,7 @@ class BinaryQuantizationFormat:
     def loadIndexRows(self, prefix: str, first: int, count: int):
         """Rows [first, first + count) of an image as an index whose base is `first` (bbq_index_load_rows, not
         collective) -> (index, the five partial section checksums of the rows loaded)."""
+        self._one_gpu("loadIndexRows")
         veb, vemb = self._image_paths(prefix)
         h = C.c_void_p()
         part = (C.c_uint64 * 5)()
@@ -301,21 +410,24 @@ class BinaryQuantizationFormat:
     def writeIndexRows(self, shard: BinarizedByteVectorValues, prefix: str, totalRows: int):
         """This shard's rows at rows [base, base + size) of an image of totalRows rows (bbq_index_write_rows)
         -> the five partial section checksums of the rows written."""
+        self._one_gpu("writeIndexRows")
         veb, _ = self._image_paths(prefix)
         part = (C.c_uint64 * 5)()
-        _check(_native.load().bbq_index_write_rows(shard._h, veb, totalRows, part), "build")
+        _check(_native.load().bbq_index_write_rows(_index(shard), veb, totalRows, part), "build")
         return [int(x) for x in part]
 
     def writeIndexMeta(self, shard: BinarizedByteVectorValues, prefix: str, totalRows: int, checksums) -> None:
         """<prefix>.vemb for an image of totalRows rows whose sections have the given checksums (the sums mod 2^64 of
         every shard's partials) and this shard's centroid (bbq_index_write_meta)."""
+        self._one_gpu("writeIndexMeta")
         _, vemb = self._image_paths(prefix)
         sums = (C.c_uint64 * 5)(*[int(x) & 0xFFFFFFFFFFFFFFFF for x in checksums])
-        _check(_native.load().bbq_index_write_meta(shard._h, vemb, totalRows, sums), "build")
+        _check(_native.load().bbq_index_write_meta(_index(shard), vemb, totalRows, sums), "build")
 
     def setBase(self, targetVectors: BinarizedByteVectorValues, base: int) -> None:
         """Global row id of this shard's row 0 (bbq_index_set_base)."""
-        _check(_native.load().bbq_index_set_base(targetVectors._h, base))
+        self._one_gpu("setBase")
+        _check(_native.load().bbq_index_set_base(_index(targetVectors), base))
 
     # -- query side -------------------------------------------------------------------------------------
     def quantizeQueryVector(self, queryVector, centroid) -> dict:
@@ -326,8 +438,8 @@ class BinaryQuantizationFormat:
         q = np.ascontiguousarray(queryVector, np.float32)
         codes = np.empty(q.size, np.uint8)
         corr = np.empty(4, np.float64)
-        if isinstance(centroid, BinarizedByteVectorValues):
-            _check(_native.load().bbq_debug_quantize_query(centroid._h, q.ctypes.data, codes.ctypes.data,
+        if isinstance(centroid, (BinarizedByteVectorValues, GroupBinarizedByteVectorValues)):
+            _check(_native.load().bbq_debug_quantize_query(_index(centroid), q.ctypes.data, codes.ctypes.data,
                                                            corr.ctypes.data), "search")
         else:
             cen = np.ascontiguousarray(centroid, np.float32)
@@ -411,7 +523,11 @@ class BinaryQuantizationFormat:
         sc = np.empty((nq, max(k, 1)), np.float32)
         cnt = C.c_uint32(0)
         L = _native.load()
-        fn = L.bbq_search_sharded if sharded else L.bbq_search
+        self._not_sharded(sharded)
+        if isinstance(targetVectors, GroupBinarizedByteVectorValues):
+            fn = L.bbq_group_search
+        else:
+            fn = L.bbq_search_sharded if sharded else L.bbq_search
         _check(fn(targetVectors._h, qs.ctypes.data, nq, k, idx.ctypes.data, sc.ctypes.data, C.byref(cnt)), "search")
         assert sharded or cnt.value == (kk if nq else 0) or k == 0
         return idx[:, :cnt.value].copy(), sc[:, :cnt.value].copy()
@@ -422,11 +538,14 @@ class BinaryQuantizationFormat:
         m = _as_matrix(vectors)
         if m.shape[0] != targetVectors.size() or m.shape[1] != targetVectors.dimension():
             raise BbqError(4, "向量维度不匹配")
-        _check(_native.load().bbq_index_attach_rows(targetVectors._h, m.ctypes.data), "build")
+        L = _native.load()
+        fn = L.bbq_group_index_attach_rows if isinstance(targetVectors, GroupBinarizedByteVectorValues) else L.bbq_index_attach_rows
+        _check(fn(targetVectors._h, m.ctypes.data), "build")
 
     def attachOriginalVectorsDevice(self, targetVectors: BinarizedByteVectorValues, d_rows_ptr: int):
         """Same, rows already in device memory ([size, dimension] f32, e.g. a torch tensor's data_ptr())."""
-        _check(_native.load().bbq_index_attach_rows_device(targetVectors._h, d_rows_ptr), "build")
+        self._one_gpu("attachOriginalVectorsDevice")
+        _check(_native.load().bbq_index_attach_rows_device(_index(targetVectors), d_rows_ptr), "build")
 
     def searchOversampledBatch(self, queries, targetVectors: BinarizedByteVectorValues, k: int, oversampleFactor: int,
                                sharded: bool = False):
@@ -441,7 +560,11 @@ class BinaryQuantizationFormat:
         tsc = np.empty((nq, max(k, 1)), np.float64)
         cnt = C.c_uint32(0)
         L = _native.load()
-        fn = L.bbq_search_rerank_sharded if sharded else L.bbq_search_rerank
+        self._not_sharded(sharded)
+        if isinstance(targetVectors, GroupBinarizedByteVectorValues):
+            fn = L.bbq_group_search_rerank
+        else:
+            fn = L.bbq_search_rerank_sharded if sharded else L.bbq_search_rerank
         _check(fn(targetVectors._h, qs.ctypes.data, nq, k, oversampleFactor, idx.ctypes.data, qsc.ctypes.data,
                   tsc.ctypes.data, C.byref(cnt)), "search")
         n = cnt.value
@@ -450,28 +573,32 @@ class BinaryQuantizationFormat:
     def rerankOwnedDevice(self, targetVectors: BinarizedByteVectorValues, d_queries_ptr: int, nq: int,
                           d_cand_idx_ptr: int, m: int, d_true_bits_ptr: int, stream: int = 0):
         """bbq_rerank_owned_device: [nq][m] u64 = this shard's exact-score bits for the candidates it holds, else 0."""
-        _check(_native.load().bbq_rerank_owned_device(targetVectors._h, d_queries_ptr, nq, d_cand_idx_ptr, m,
+        self._one_gpu("rerankOwnedDevice")
+        _check(_native.load().bbq_rerank_owned_device(_index(targetVectors), d_queries_ptr, nq, d_cand_idx_ptr, m,
                                                       d_true_bits_ptr, stream or None), "search")
 
     # -- parity taps (tests) ------------------------------------------------------------------------------
     def debugQcDist(self, queryVector, targetVectors: BinarizedByteVectorValues) -> np.ndarray:
+        self._one_gpu("debugQcDist")
         q = np.ascontiguousarray(queryVector, np.float32)
         out = np.empty(targetVectors.size(), np.int32)
-        _check(_native.load().bbq_debug_qcdist(targetVectors._h, q.ctypes.data, out.ctypes.data), "search")
+        _check(_native.load().bbq_debug_qcdist(_index(targetVectors), q.ctypes.data, out.ctypes.data), "search")
         return out
 
     def debugQcDistBatch(self, queries, targetVectors: BinarizedByteVectorValues) -> np.ndarray:
         """The integer dots of the TENSOR-CORE scan (tcgen05 accumulators) for a query batch: int32 [nq, n]."""
+        self._one_gpu("debugQcDistBatch")
         qs = np.ascontiguousarray(queries, np.float32)
         out = np.empty((qs.shape[0], targetVectors.size()), np.int32)
-        _check(_native.load().bbq_debug_qcdist_batch(targetVectors._h, qs.ctypes.data, qs.shape[0], out.ctypes.data),
+        _check(_native.load().bbq_debug_qcdist_batch(_index(targetVectors), qs.ctypes.data, qs.shape[0], out.ctypes.data),
                "search")
         return out
 
     def debugScores(self, queryVector, targetVectors: BinarizedByteVectorValues) -> np.ndarray:
+        self._one_gpu("debugScores")
         q = np.ascontiguousarray(queryVector, np.float32)
         out = np.empty(targetVectors.size(), np.float32)
-        _check(_native.load().bbq_debug_scores(targetVectors._h, q.ctypes.data, out.ctypes.data), "search")
+        _check(_native.load().bbq_debug_scores(_index(targetVectors), q.ctypes.data, out.ctypes.data), "search")
         return out
 
     def stats(self) -> dict:
@@ -492,7 +619,8 @@ class BinaryQuantizationFormat:
     # -- device-resident entry points (plumbing for sharded search: torch tensors' data_ptr()) ------------
     def searchDevice(self, d_queries_ptr: int, nq: int, targetVectors: BinarizedByteVectorValues, k: int,
                      d_out_idx_ptr: int, d_out_score_ptr: int, stream: int = 0):
-        _check(_native.load().bbq_search_device(targetVectors._h, d_queries_ptr, nq, k, d_out_idx_ptr,
+        self._one_gpu("searchDevice")
+        _check(_native.load().bbq_search_device(_index(targetVectors), d_queries_ptr, nq, k, d_out_idx_ptr,
                                                 d_out_score_ptr, stream or None), "search")
 
     # -- sharded search: the exchange lives in the library (bbq_comm_*, one NCCL all-gather of 64-bit keys) -----
@@ -503,10 +631,12 @@ class BinaryQuantizationFormat:
         return bytes(buf)
 
     def commInit(self, comm_id: bytes, rank: int, world: int):
+        self._one_gpu("commInit")
         buf = (C.c_uint8 * 128).from_buffer_copy(comm_id)
         _check(_native.load().bbq_comm_init(self._ctx, buf, rank, world))
 
     def commDestroy(self):
+        self._one_gpu("commDestroy")
         _check(_native.load().bbq_comm_destroy(self._ctx))
 
     def commInfo(self) -> dict:
@@ -517,17 +647,20 @@ class BinaryQuantizationFormat:
     def searchShardedHost(self, h_queries_ptr: int, nq: int, targetVectors: BinarizedByteVectorValues, k: int,
                           h_out_idx_ptr: int, h_out_score_ptr: int) -> int:
         """bbq_search_sharded on raw HOST pointers (pinned or pageable); returns the per-query result count."""
+        self._one_gpu("searchShardedHost")
         cnt = C.c_uint32(0)
-        _check(_native.load().bbq_search_sharded(targetVectors._h, h_queries_ptr, nq, k, h_out_idx_ptr,
+        _check(_native.load().bbq_search_sharded(_index(targetVectors), h_queries_ptr, nq, k, h_out_idx_ptr,
                                                  h_out_score_ptr, C.byref(cnt)), "search")
         return cnt.value
 
     def searchShardedDevice(self, d_queries_ptr: int, nq: int, targetVectors: BinarizedByteVectorValues, k: int,
                             d_out_idx_ptr: int, d_out_score_ptr: int, stream: int = 0):
-        _check(_native.load().bbq_search_sharded_device(targetVectors._h, d_queries_ptr, nq, k, d_out_idx_ptr,
+        self._one_gpu("searchShardedDevice")
+        _check(_native.load().bbq_search_sharded_device(_index(targetVectors), d_queries_ptr, nq, k, d_out_idx_ptr,
                                                         d_out_score_ptr, stream or None), "search")
 
     def mergeTopKDevice(self, d_idx_ptr: int, d_score_ptr: int, lists: int, nq: int, k: int, d_out_idx_ptr: int,
                         d_out_score_ptr: int, stream: int = 0):
+        self._one_gpu("mergeTopKDevice")
         _check(_native.load().bbq_merge_topk_device(self._ctx, d_idx_ptr, d_score_ptr, lists, nq, k,
                                                     d_out_idx_ptr, d_out_score_ptr, stream or None), "search")

@@ -6,12 +6,15 @@ selection kernel, so the result is independent of the number of shards.  This fi
 the communicator id (bbq_comm_unique_id) and it is broadcast over whatever the host already has — here
 torch.distributed (gloo or nccl), in a Node host a pipe or an environment variable (INTEGRATION.md).
 The reference has no counterpart (it is single-process); the merge rule is its MinHeap contract made canonical
-(src/binaryQuantizationFormat.ts:383-411)."""
+(src/binaryQuantizationFormat.ts:383-411).
+One process can also drive every GPU itself: BinaryQuantizationFormat(config, devices=[...]) owns a device group
+(bbq_group_*), one worker thread per GPU running these same collective entries with the split of shard_bounds below;
+no communicator id, rank bookkeeping or corpus split is left to the host."""
 from __future__ import annotations
 
 import numpy as np
 
-from .format import BinarizedByteVectorValues, BinaryQuantizationFormat
+from .format import BinarizedByteVectorValues, BinaryQuantizationFormat, _index
 
 
 def shard_bounds(n_total: int, world: int, rank: int):
@@ -35,7 +38,7 @@ class ShardedSearcher:
         from .. import _native
         self.torch = torch
         self.fmt, self.shard, self.rank, self.world = fmt, shard, rank, world
-        st = _native.load().bbq_index_set_base(shard._h, int(base))
+        st = _native.load().bbq_index_set_base(_index(shard), int(base))
         if st != 0:
             raise RuntimeError(_native.load().bbq_last_error().decode())
         if world > 1:

@@ -14,7 +14,8 @@
  * There is NO CPU fallback: without a usable sm_100 device bbq_create fails with BBQ_ERR_NO_DEVICE.
  *
  * Threading: a bbq_ctx and its indexes may be used from one host thread at a time (the reference is
- * synchronous single-threaded JS, SURVEY §8b).  Different contexts are independent.
+ * synchronous single-threaded JS, SURVEY §8b).  Different contexts are independent.  A device group (bbq_group_*)
+ * drives every GPU of a box from one caller thread.
  */
 #ifndef BBQ_B200_H
 #define BBQ_B200_H
@@ -275,6 +276,62 @@ int bbq_search_sharded_device(bbq_index* index, const float* d_queries, uint32_t
  * ones make the copies asynchronous DMA).  A Node host wraps these in external ArrayBuffers. */
 void* bbq_host_alloc(size_t bytes);
 void bbq_host_free(void* p);
+
+/* -------- device groups: one process and one caller thread over the GPUs of a box ------------------------ */
+
+/* A device group owns one context, one NCCL communicator and one host worker thread per GPU.  Each group entry checks
+ * its arguments on the caller's thread (the same statuses and messages as the single-index entry, so no argument error
+ * reaches a collective), hands the collective entry above of every rank to that rank's worker, waits for all of them,
+ * and returns rank 0's results: bit for bit what the one-process-per-GPU path gives, which equals one index holding
+ * the whole corpus.  Only rank 0 writes into the caller's buffers.
+ *   Rows split: rank r holds rows [r*per, min(N, (r+1)*per)), per = ceil(N / n_devices) (host/sharded.py shard_bounds,
+ *   what bbq_index_load_sharded does), with its base set, so every id is global.  Shards may be empty (N < n_devices).
+ *   build = bbq_index_build_sharded of every rank's slice (the reference-order centroid chained across the GPUs; host
+ *   rows are validated by every worker on its slice first, and a NaN / Infinity reports bbq_index_build's status,
+ *   message and vector index in the whole corpus); from_quantized = bbq_index_from_quantized of every slice plus
+ *   bbq_index_set_base; load / save = bbq_index_load_sharded / bbq_index_save_sharded; attach_rows =
+ *   bbq_index_attach_rows of every slice (rows: all n rows, HOST); search = bbq_search_sharded; search_rerank =
+ *   bbq_search_rerank_sharded.  export routes each part of a row range to the shard that holds it (not collective);
+ *   size, dim and centroid answer from the group's metadata.
+ *   Errors: the lowest failing rank's status, message and bbq_last_error_pos reach the caller's thread.  A runtime
+ *   failure (status >= 100) on one rank while other ranks are still running 5 s later (the collective entries exchange
+ *   most failures, so peers normally return the same status at once): those ranks are taken to wait in a collective
+ *   the failed rank never joins.  The caller's thread then aborts every communicator (ncclCommAbort) and joins the
+ *   workers; the call returns the failed rank's status with "device group aborted after rank r failed: ...", the
+ *   group is failed, every later call returns BBQ_ERR_COMM with that message, and bbq_group_index_destroy /
+ *   bbq_group_destroy still work.  Before the communicators exist (creating the contexts) nothing is aborted: the
+ *   call waits for every worker and returns the lowest failing rank's own error.
+ *   Creation: every worker first creates its context (an empty, duplicated or negative device list is
+ *   BBQ_ERR_INVALID_ARG before any device is probed; without a device no worker starts: BBQ_ERR_NO_DEVICE); only when
+ *   all succeed do the workers create the communicators together.  n_devices == 1 creates no communicator: the
+ *   entries are then the single-GPU entries.  Whatever was created is released on failure, and every thread joined.
+ *   bbq_group_destroy: BBQ_ERR_INVALID_ARG while group indexes of the group are alive (the group stays usable);
+ *   otherwise ncclCommDestroy on every GPU, then every context, and the workers are joined.
+ *   bbq_group_context: rank r's context, for bbq_get_stats / bbq_set_profiling and non-collective members such as
+ *   bbq_quantize_query.  A collective entry called on it from outside the group returns BBQ_ERR_INVALID_ARG.
+ * Threading: a group and its indexes may be used from one host thread at a time, like a context. */
+typedef struct bbq_group bbq_group;
+typedef struct bbq_group_index bbq_group_index;
+int bbq_group_create(const bbq_config* config, const int32_t* devices, uint32_t n_devices, bbq_group** out);
+int bbq_group_destroy(bbq_group* g);
+int bbq_group_info(const bbq_group* g, uint32_t* n_devices, int32_t* devices /* n_devices entries, may be NULL */);
+bbq_ctx* bbq_group_context(bbq_group* g, uint32_t rank);
+int bbq_group_index_build(bbq_group* g, const float* rows, uint64_t n, uint32_t dim, const float* centroid,
+                          bbq_group_index** out);
+int bbq_group_index_from_quantized(bbq_group* g, const uint8_t* packed, const double* corr4, const float* centroid,
+                                   uint64_t n, uint32_t dim, bbq_group_index** out);
+int bbq_group_index_load(bbq_group* g, const char* veb_path, const char* vemb_path, bbq_group_index** out);
+int bbq_group_index_save(const bbq_group_index* gi, const char* veb_path, const char* vemb_path);
+uint64_t bbq_group_index_size(const bbq_group_index* gi);
+uint32_t bbq_group_index_dim(const bbq_group_index* gi);
+int bbq_group_index_centroid(const bbq_group_index* gi, float* out_centroid, double* out_centroid_dp);
+int bbq_group_index_export(const bbq_group_index* gi, uint64_t first, uint64_t count, uint8_t* packed, double* corr4);
+int bbq_group_index_attach_rows(bbq_group_index* gi, const float* rows);
+int bbq_group_search(bbq_group_index* gi, const float* queries, uint32_t nq, int64_t k, int32_t* out_idx,
+                     float* out_score, uint32_t* out_count);
+int bbq_group_search_rerank(bbq_group_index* gi, const float* queries, uint32_t nq, uint32_t k, uint32_t factor,
+                            int32_t* out_idx, float* out_qscore, double* out_true, uint32_t* out_count);
+void bbq_group_index_destroy(bbq_group_index* gi);
 
 /* -------- oversampled search + exact re-rank (SURVEY §8f rank 2) ---------------------------------------- */
 
