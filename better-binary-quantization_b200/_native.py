@@ -121,7 +121,6 @@ SYMBOLS = {
     "bbq_get_stats": (C.c_int, [_vp, C.POINTER(BbqStats)]),
     "bbq_set_profiling": (C.c_int, [_vp, C.c_int]),
     "bbq_reset_profiling": (C.c_int, [_vp]),
-    "bbq_debug_trace": (C.c_int, [_vp, _vp, C.c_uint32]),
 }
 
 _lib = None

@@ -86,16 +86,8 @@ struct bbq_ctx {
   DevBuf T, stage, cacc, chain, norms;  // chain: the centroid's running sum, dim words + one status word
   // query scratch
   DevBuf qrows, qT, qcodes, qcorr, planes, qterms, tau, dump, cand, cand_cnt, lists_a, lists_b,
-      out_idx, out_score, dots, images, qscreen, tau_bits, trace, rr_true, rr_idx, rr_q, rr_t, cenv, qoff, qenv;
-  int64_t sample_tiles_dyn = 128;  // BBQ_SAMPLE_TILES: sample size when the running threshold is on
-  int k1s_ctas = 4;         // BBQ_K1S_CTAS: persistent CTAs per SM of the streaming scan (huge = one tile per CTA)
-  int csa = 1;              // BBQ_CSA=0: plain popcount accumulation in the streaming scan (A/B, tests)
+      out_idx, out_score, dots, images, qscreen, tau_bits, rr_true, rr_idx, rr_q, rr_t, cenv, qoff, qenv;
   int popc_form = 0;        // BBQ_POPC_FORM=tile forces the shared-memory tile form of the popcount scan (tests)
-  int mma_ntile_cap = 0;    // BBQ_MMA_NTILE: cap on the queries resident per pass (tuning experiments)
-  int mma_layout = -1;      // BBQ_MMA_LAYOUT: -1 by accumulator columns (mma_plan), 0 wide-batch roles, 1 narrow-batch roles
-  int mma_issuers = 0;      // BBQ_MMA_ISSUERS: 0 by layout (mma_plan: 2 wide, 3 narrow), else 1..3 MMA issuing threads
-  int mma_narrow_max = 96;  // BBQ_MMA_NARROW_MAX: widest resident block (accumulator columns) that takes the narrow-batch roles
-  uint32_t mma_debug = 0;   // BBQ_MMA_DEBUG: timing-attribution knobs of the tensor-core scan (results become wrong)
   bool dynamic_tau = true;  // BBQ_DYNTAU=0 keeps the sampled threshold fixed during the tensor-core scan (tests)
   int query_quantizer = 0;  // BBQ_QQUANT: thread / warp / cta force one form of K4 (tests, A/B); default by batch size
   // query screening armed by an entry point for the batch that starts at validate_base: the next K4 launches do it
@@ -107,7 +99,7 @@ struct bbq_ctx {
   // A narrow batch is launch-latency bound (a single query: ~10 stream operations around 60-90 us of kernels), and
   // its whole device sequence — screening, K4, planes / B images, threshold sample, scan, selection, status read-back —
   // depends only on (index, batch size, k): bbq_search captures it into a CUDA graph the second time the same key
-  // arrives and replays it from then on (BBQ_GRAPH=0 turns that off).
+  // arrives and replays it from then on (batches of up to GRAPH_MAX_NQ queries).
   struct SearchGraphKey {
     uint64_t ix = 0, n = 0, base = 0; const void* codes = nullptr; const void* rscreen = nullptr;
     uint32_t nq = 0, k = 0; uint64_t scratch_gen = 0;
@@ -124,8 +116,6 @@ struct bbq_ctx {
     uint32_t last_path = 0, last_engine = 0;
     uint64_t replays = 0;
   } sgraph;
-  int graph_max_nq = 16;    // BBQ_GRAPH: 0 off, else the widest batch whose sequence is captured
-  int qquant_cta_max = -1;  // BBQ_QQUANT_CTA_MAX: largest batch quantised one CTA per query (-1: 2 x SM count)
   int scan_engine = 0;  // BBQ_SCAN: 0 auto, 1 popcount kernel only, 2 tensor-core kernel whenever it can run
   uint32_t* h_flag = nullptr;  // pinned: [0..nq) candidate counts, [nq] overflow flag, then 2 words: first invalid query
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;  // ordering between the context's stream and a caller's stream (StreamBridge)
@@ -226,6 +216,7 @@ struct bbq_index {
 
 static constexpr int64_t BUILD_CHUNK = 32768;   // rows per build chunk (transposed scratch = dim*chunk*4 B)
 static constexpr uint32_t QUERY_BATCH = 4096;   // queries per internal pass (12-bit query field of a parked hit)
+static constexpr uint32_t GRAPH_MAX_NQ = 16;    // widest batch whose device sequence bbq_search captures (bbq_ctx::sgraph)
 static constexpr int64_t SAMPLE_TILES = 128;    // threshold sample = 128 tiles = 16384 rows ...
 static constexpr int64_t SAMPLE_TILES_MAX = 2048;  // ... grown with k*n up to 262144 rows (see search_filtered)
 static constexpr uint32_t CAND_CAP = SELECT_MAX;
@@ -286,19 +277,9 @@ extern "C" int bbq_create(const bbq_config* config, bbq_ctx** out_ctx) {
   CU(cudaEventCreateWithFlags(&c->ev_in, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&c->ev_out, cudaEventDisableTiming));
   if (const char* e = getenv("BBQ_FORCE_PATH")) c->force_path = atoi(e);
-  if (const char* e = getenv("BBQ_SAMPLE_TILES")) c->sample_tiles_dyn = std::max(1, std::min(128, atoi(e)));
-  if (const char* e = getenv("BBQ_CSA")) c->csa = atoi(e);
-  if (const char* e = getenv("BBQ_K1S_CTAS")) c->k1s_ctas = std::max(1, atoi(e));
   if (const char* e = getenv("BBQ_POPC_FORM")) c->popc_form = !strcmp(e, "tile") ? 1 : 0;
-  if (const char* e = getenv("BBQ_MMA_NTILE")) c->mma_ntile_cap = atoi(e);
-  if (const char* e = getenv("BBQ_MMA_LAYOUT")) c->mma_layout = atoi(e);
-  if (const char* e = getenv("BBQ_MMA_NARROW_MAX")) c->mma_narrow_max = atoi(e);
-  if (const char* e = getenv("BBQ_MMA_ISSUERS")) c->mma_issuers = std::max(0, std::min(3, atoi(e)));
-  if (const char* e = getenv("BBQ_MMA_DEBUG")) c->mma_debug = (uint32_t)atoi(e);
   if (const char* e = getenv("BBQ_DYNTAU")) c->dynamic_tau = atoi(e) != 0;
   if (const char* e = getenv("BBQ_QQUANT")) c->query_quantizer = !strcmp(e, "thread") ? 1 : !strcmp(e, "warp") ? 2 : !strcmp(e, "cta") ? 3 : 0;
-  if (const char* e = getenv("BBQ_QQUANT_CTA_MAX")) c->qquant_cta_max = atoi(e);
-  if (const char* e = getenv("BBQ_GRAPH")) c->graph_max_nq = std::max(0, atoi(e));
   if (const char* e = getenv("BBQ_SCAN")) c->scan_engine = !strcmp(e, "popc") ? 1 : !strcmp(e, "mma") ? 2 : 0;
   *out_ctx = c;
   return BBQ_OK;
@@ -350,14 +331,6 @@ extern "C" int bbq_get_stats(bbq_ctx* c, bbq_stats* out) {
   c->ev_pending.clear();
   *out = c->stats;
   out->kernel_launches = c->launches;
-  return BBQ_OK;
-}
-extern "C" int bbq_debug_trace(bbq_ctx* c, long long* out, uint32_t count) {
-  if (!c || !out) return fail(BBQ_ERR_NULL, "null");
-  if (!c->trace.p) return fail(BBQ_ERR_INVALID_ARG, "no trace recorded (BBQ_MMA_DEBUG bit 32)");
-  CU(cudaSetDevice(c->device));
-  CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(out, c->trace.p, std::min<size_t>(count, 4 * 4096) * sizeof(long long), cudaMemcpyDeviceToHost));
   return BBQ_OK;
 }
 extern "C" int bbq_set_profiling(bbq_ctx* c, int enabled) {
@@ -793,24 +766,22 @@ extern "C" int bbq_index_export(const bbq_index* ix, uint64_t first, uint64_t co
 // ------------------------------------------------------------------------------------------------
 // search
 // ------------------------------------------------------------------------------------------------
+static constexpr unsigned K1S_CTAS_PER_SM = 4;  // persistent CTAs per SM of the streaming scan (its __launch_bounds__)
 template <int MODE>
 static int launch_scan_nb(bbq_ctx* c, int nb, bool stream_form, dim3 grid, size_t smem, cudaStream_t st,
                           const ScanParams& p) {
-#define BBQ_STREAM_LAUNCH(NB, MODE, W)                                                                             \
-  if (NB == 4 && c->csa) LAUNCH(c, (k_scan_stream<NB, MODE, W, NB == 4>), dim3(sgrid), TILE_ROWS, 0, st, p);       \
-  else LAUNCH(c, (k_scan_stream<NB, MODE, W, false>), dim3(sgrid), TILE_ROWS, 0, st, p)
 #define BBQ_SCAN_CASE(NB)                                                                                          \
   case NB:                                                                                                         \
     if (stream_form) {                                                                                             \
-      const unsigned sgrid = std::min<unsigned>(grid.x, (unsigned)c->sm_count * (unsigned)c->k1s_ctas);                             \
+      const unsigned sgrid = std::min<unsigned>(grid.x, (unsigned)c->sm_count * K1S_CTAS_PER_SM);                  \
       switch (p.row_bytes >> 4) {                                                                                  \
-        case 1: BBQ_STREAM_LAUNCH(NB, MODE, 1); break;                                                            \
-        case 2: BBQ_STREAM_LAUNCH(NB, MODE, 2); break;                                                            \
-        case 3: BBQ_STREAM_LAUNCH(NB, MODE, 3); break;                                                            \
-        case 4: BBQ_STREAM_LAUNCH(NB, MODE, 4); break;                                                            \
-        case 6: BBQ_STREAM_LAUNCH(NB, MODE, 6); break;                                                            \
-        case 8: BBQ_STREAM_LAUNCH(NB, MODE, 8); break;                                                            \
-        case 12: BBQ_STREAM_LAUNCH(NB, MODE, 12); break;                                                            \
+        case 1: LAUNCH(c, (k_scan_stream<NB, MODE, 1>), dim3(sgrid), TILE_ROWS, 0, st, p); break;                  \
+        case 2: LAUNCH(c, (k_scan_stream<NB, MODE, 2>), dim3(sgrid), TILE_ROWS, 0, st, p); break;                  \
+        case 3: LAUNCH(c, (k_scan_stream<NB, MODE, 3>), dim3(sgrid), TILE_ROWS, 0, st, p); break;                  \
+        case 4: LAUNCH(c, (k_scan_stream<NB, MODE, 4>), dim3(sgrid), TILE_ROWS, 0, st, p); break;                  \
+        case 6: LAUNCH(c, (k_scan_stream<NB, MODE, 6>), dim3(sgrid), TILE_ROWS, 0, st, p); break;                  \
+        case 8: LAUNCH(c, (k_scan_stream<NB, MODE, 8>), dim3(sgrid), TILE_ROWS, 0, st, p); break;                  \
+        case 12: LAUNCH(c, (k_scan_stream<NB, MODE, 12>), dim3(sgrid), TILE_ROWS, 0, st, p); break;                \
         default: return fail(BBQ_ERR_UNSUPPORTED, "no streaming scan for this row size");                          \
       }                                                                                                            \
     } else {                                                                                                       \
@@ -837,7 +808,6 @@ static int launch_scan_nb(bbq_ctx* c, int nb, bool stream_form, dim3 grid, size_
       return fail(BBQ_ERR_QUERY_BITS, "queryBits must be in 1..8");
   }
 #undef BBQ_SCAN_CASE
-#undef BBQ_STREAM_LAUNCH
   return BBQ_OK;
 }
 
@@ -899,8 +869,7 @@ static int quantize_rows(bbq_ctx* c, const float* d_queries, int nq, int dim, in
                           (size_t)((dim + 3) & ~3) * sizeof(float);
   // 0 = by batch size: one CTA per query for a narrow batch (K4 is the longest kernel of a single-query search and
   // the CTA form runs each pass at the latency of the add chain), one warp per query otherwise
-  const int cta_max = c->qquant_cta_max >= 0 ? c->qquant_cta_max : 2 * c->sm_count;
-  const int form = c->query_quantizer != 0 ? c->query_quantizer : (nq <= cta_max ? 3 : 2);
+  const int form = c->query_quantizer != 0 ? c->query_quantizer : (nq <= 2 * c->sm_count ? 3 : 2);
   // query screening (NaN / Infinity): armed by the entry point, done by K4 itself while it stages the query
   unsigned long long* bad = nullptr;
   int q_base = 0;
@@ -967,7 +936,6 @@ static bool mma_plan(const bbq_index* ix, int nq, MmaPlan* out) {
   const size_t budget = 227 * 1024 - 1024 - (HIT_RING * sizeof(uint64_t) + 64);
   int n_cap = (int)(budget / ((size_t)pl.kbytes + 64)) / 16 * 16;
   n_cap = std::min(n_cap, MMA_N_MAX);
-  if (c->mma_ntile_cap > 0) n_cap = std::min(n_cap, c->mma_ntile_cap / 16 * 16);
   if (n_cap < 16) return false;
   // 1-4 queries: the streaming popcount scan (HBM/latency bound, ~43 us per query and 1M rows).  From 5 queries on the
   // tensor-core scan wins: one pass over 1M x 1024 costs 0.145 ms whatever the block size (operand-feed bound), the
@@ -981,8 +949,9 @@ static bool mma_plan(const bbq_index* ix, int nq, MmaPlan* out) {
   // 16 columns 0.136 -> 0.109, 64: 0.146 -> 0.127, 96: 0.151 -> 0.137, 128: 0.157 -> 0.155 (EUCLIDEAN: 0.175 -> 0.185), 208: 0.213 ->
   // 0.218).  A narrow batch is bound by the ISSUE of its tcgen05 operations (32 MMAs + 12 commits per 128-row tile whatever
   // the width, ~100-150 cycles each for the issuing thread), so the narrow layout also runs three issuing threads.
-  pl.layout = c->mma_layout >= 0 ? (c->mma_layout ? 1 : 0) : (pl.n_tile <= c->mma_narrow_max ? 1 : 0);
-  pl.nissuers = c->mma_issuers > 0 ? c->mma_issuers : (pl.layout == 1 ? 3 : 2);
+  constexpr int MMA_NARROW_MAX = 96;  // widest resident block (accumulator columns) that takes the narrow layout
+  pl.layout = pl.n_tile <= MMA_NARROW_MAX ? 1 : 0;
+  pl.nissuers = pl.layout == 1 ? 3 : 2;
   pl.smem = (size_t)pl.n_tile * pl.kbytes + (size_t)pl.n_tile * (sizeof(QScreen) + sizeof(bbqn::QueryTerms)) + 26 * 8 + sizeof(HitCtx) + HIT_RING * sizeof(uint64_t) + 16 + 16;
   *out = pl;
   return true;
@@ -1017,17 +986,17 @@ static int prepare_mma_operands(bbq_index* ix, int nq, const MmaPlan& pl, cudaSt
   return BBQ_OK;
 }
 
-template <int MODE, int LAYOUT, bool DBG>
+template <int MODE, int LAYOUT>
 static int launch_mma_sim(bbq_ctx* c, int sim, int cpq, unsigned grid, size_t smem, cudaStream_t st, const MmaParams& p) {
-#define BBQ_MMA_CASE(S)                                                                                                       \
-  case S:                                                                                                                     \
-    if (cpq == 1) {                                                                                                           \
-      CU(cudaFuncSetAttribute(k_scan_mma<MODE, S, 1, LAYOUT, DBG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-      LAUNCH(c, (k_scan_mma<MODE, S, 1, LAYOUT, DBG>), grid, MmaLayout<LAYOUT>::THREADS, smem, st, p);                       \
-    } else {                                                                                                                  \
-      CU(cudaFuncSetAttribute(k_scan_mma<MODE, S, 2, LAYOUT, DBG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-      LAUNCH(c, (k_scan_mma<MODE, S, 2, LAYOUT, DBG>), grid, MmaLayout<LAYOUT>::THREADS, smem, st, p);                       \
-    }                                                                                                                         \
+#define BBQ_MMA_CASE(S)                                                                                                  \
+  case S:                                                                                                                \
+    if (cpq == 1) {                                                                                                      \
+      CU(cudaFuncSetAttribute(k_scan_mma<MODE, S, 1, LAYOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+      LAUNCH(c, (k_scan_mma<MODE, S, 1, LAYOUT>), grid, MmaLayout<LAYOUT>::THREADS, smem, st, p);                       \
+    } else {                                                                                                             \
+      CU(cudaFuncSetAttribute(k_scan_mma<MODE, S, 2, LAYOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+      LAUNCH(c, (k_scan_mma<MODE, S, 2, LAYOUT>), grid, MmaLayout<LAYOUT>::THREADS, smem, st, p);                       \
+    }                                                                                                                    \
     break;
   switch (sim) {
     BBQ_MMA_CASE(0)
@@ -1061,14 +1030,6 @@ static int launch_scan_mma(bbq_index* ix, int mode, int nq, uint32_t k, const Mm
   p.tau_bits = c->tau_bits.as<uint32_t>();
   p.bounds = ix->bounds;
   p.k = c->dynamic_tau ? k : 0xFFFFFFFFu;
-  p.debug = c->mma_debug;
-  p.trace = nullptr;
-  if (c->mma_debug & (32u | 256u)) {
-    const bool fresh = c->trace.p == nullptr;
-    TRY(c->trace.reserve(4 * 4096 * sizeof(long long)));
-    if (fresh) CU(cudaMemsetAsync(c->trace.p, 0, 4 * 4096 * sizeof(long long), st));
-    p.trace = c->trace.as<long long>();
-  }
   p.qterms = c->qterms.as<bbqn::QueryTerms>();
   p.nq = nq;
   p.n_tile = pl.n_tile;
@@ -1097,15 +1058,10 @@ static int launch_scan_mma(bbq_index* ix, int mode, int nq, uint32_t k, const Mm
   if (mode != SCAN_DUMP) c->stats.mma_layout = (uint32_t)pl.layout;
   c->stats.mma_passes = (uint32_t)pl.passes;
   const unsigned grid = (unsigned)std::min<int64_t>(ntiles, c->sm_count);
-  // (the dump — threshold sample, parity taps — always runs the wide-batch roles: it is a few hundred tiles,
-  // and without the attribution knobs; the filtered scan carries them only when BBQ_MMA_DEBUG asks for one)
-  if (mode == SCAN_DUMP) return launch_mma_sim<SCAN_DUMP, 0, false>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
-  if (c->mma_debug != 0) {
-    if (pl.layout == 1) return launch_mma_sim<SCAN_FILTER, 1, true>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
-    return launch_mma_sim<SCAN_FILTER, 0, true>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
-  }
-  if (pl.layout == 1) return launch_mma_sim<SCAN_FILTER, 1, false>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
-  return launch_mma_sim<SCAN_FILTER, 0, false>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
+  // (the dump — threshold sample, parity taps — always runs the wide-batch roles: it is a few hundred tiles)
+  if (mode == SCAN_DUMP) return launch_mma_sim<SCAN_DUMP, 0>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
+  if (pl.layout == 1) return launch_mma_sim<SCAN_FILTER, 1>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
+  return launch_mma_sim<SCAN_FILTER, 0>(c, p.sim, pl.cpq, grid, pl.smem, st, p);
 }
 
 static ScanParams base_scan_params(bbq_index* ix, int nq) {
@@ -1247,7 +1203,7 @@ static int search_filtered(bbq_index* ix, int nq, uint32_t k, int32_t* d_out_idx
   // sample grows with k * n until that expectation is a quarter of a candidate list (otherwise a large k or a large
   // shard would overflow the lists on perfectly ordinary data and fall back to the exact chunked path every time).
   const bool running = use_mma && c->dynamic_tau && k <= RETIGHTEN_KMAX;
-  int64_t want_tiles = running ? c->sample_tiles_dyn : SAMPLE_TILES;
+  int64_t want_tiles = SAMPLE_TILES;
   if (!running) {
     const int64_t need_rows = (int64_t)std::min<double>(4.0 * (double)k * (double)n / (double)CAND_CAP, 1e12);
     want_tiles = std::max(want_tiles, std::min<int64_t>(SAMPLE_TILES_MAX, (need_rows + TILE_ROWS - 1) / TILE_ROWS));
@@ -1458,7 +1414,7 @@ extern "C" int bbq_search(bbq_index* ix, const float* queries, uint32_t nq, int6
     TRY(st_search);
     return screen.read_back(c->stream);
   };
-  const bool graph_ok = c->graph_max_nq > 0 && nq <= (uint32_t)c->graph_max_nq && !c->profiling && c->mma_debug == 0;
+  const bool graph_ok = nq <= GRAPH_MAX_NQ && !c->profiling;
   bbq_ctx::SearchGraphKey key;
   key.ix = ix->serial; key.n = ix->n; key.base = ix->base; key.codes = ix->codes; key.rscreen = ix->rscreen;
   key.nq = nq; key.k = kk; key.scratch_gen = g_scratch_gen;

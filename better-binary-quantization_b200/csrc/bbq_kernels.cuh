@@ -867,7 +867,7 @@ __device__ __forceinline__ int csa_dot4(const uint4 x, const uint4 p0, const uin
 // per unit) and the exact f64 epilogue then runs with one row per lane.
 // Same integers, same scores, same outputs as k_scan; tiles/dump layout identical.
 // ------------------------------------------------------------------------------------------------
-template <int NB, int MODE, int W4, bool CSA>
+template <int NB, int MODE, int W4>
 __global__ void __launch_bounds__(TILE_ROWS, 4) k_scan_stream(const ScanParams p) {
   constexpr int w4 = W4;                  // 16-byte chunks per row (compile-time: 1..16)
   constexpr int R = 32 / w4;              // rows per load instruction
@@ -945,7 +945,7 @@ __global__ void __launch_bounds__(TILE_ROWS, 4) k_scan_stream(const ScanParams p
       int part[iters];
 #pragma unroll
       for (int it = 0; it < iters; it++) {
-        if (NB == 4 && CSA) {
+        if (NB == 4) {
           part[it] = csa_dot4(x[it], pl[0], pl[1 % NB], pl[2 % NB], pl[3 % NB]);
         } else {
           int acc = 0;

@@ -32,32 +32,19 @@
 
 namespace bbqk {
 
-#ifndef BBQ_MMA_EPI_WARPS
-#define BBQ_MMA_EPI_WARPS 8
-#endif
-#ifndef BBQ_MMA_EXP_GROUPS
-#define BBQ_MMA_EXP_GROUPS 1
-#endif
-#ifndef BBQ_MMA_LDW
-#define BBQ_MMA_LDW 16
-#endif
-constexpr int MMA_LDW = BBQ_MMA_LDW;                // accumulator columns per epilogue TMEM load (16 or 32)
-static_assert(MMA_LDW == 16 || MMA_LDW == 32, "tcgen05.ld .x16 or .x32");
-// Role layout of the 16 (or 20) warps of a CTA: warp 0 B loader, 1-2 MMA issuers (2 also allocates TMEM), 3 drainer,
+// Role layout of the 16 warps of a CTA: warp 0 B loader, 1-2 MMA issuers (2 also allocates TMEM), 3 drainer,
 // 4.. expansion groups of 4 warps (one warp per TMEM lane quarter, alternating hand-offs), then the epilogue (one or two
 // warps per TMEM lane quarter, alternating accumulator chunks).  Two layouts are compiled into the library:
-//   0 "wide batch"  : 8 epilogue warps + 1 expansion group (the build options above) — the per-pair screen is the load;
+//   0 "wide batch"  : 8 epilogue warps + 1 expansion group — the per-pair screen is the load;
 //   1 "narrow batch": 4 epilogue warps + 2 expansion groups, same 512 threads / 128 registers — with few resident
 //                     queries the epilogue has almost nothing to do and the serial operand feed of ONE group is the bound.
 // mma_plan picks by the number of accumulator columns (measured crossover, profiles/r02_k2_narrow_layout.txt).
 template <int L>
 struct MmaLayout {
-  static constexpr int EPI_WARPS = L == 0 ? BBQ_MMA_EPI_WARPS : 4;
-  static constexpr int EXP_GROUPS = L == 0 ? BBQ_MMA_EXP_GROUPS : 2;
+  static constexpr int EPI_WARPS = L == 0 ? 8 : 4;
+  static constexpr int EXP_GROUPS = L == 0 ? 1 : 2;
   static constexpr int EPI_WARP0 = 4 + 4 * EXP_GROUPS;
   static constexpr int THREADS = (EPI_WARP0 + EPI_WARPS) * 32;
-  static_assert(EPI_WARPS == 4 || EPI_WARPS == 8, "one or two epilogue warps per TMEM lane quarter");
-  static_assert(EXP_GROUPS == 1 || EXP_GROUPS == 2, "one or two expansion groups");
 };
 constexpr int MMA_N_MAX = 224;        // 2 accumulators + >= 2 A stages must fit the 512 TMEM columns
 constexpr int MMA_CHUNK_DIMS = 128;   // dims per A stage (32 TMEM columns)
@@ -179,14 +166,6 @@ __device__ __forceinline__ void tc_st32(uint32_t taddr, const uint32_t (&r)[32])
       "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
       : "memory");
 }
-__device__ __forceinline__ void tc_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16};" ::"r"(taddr),
-      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
 __device__ __forceinline__ void tc_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tc_ld16(uint32_t taddr, int (&r)[16]) {
   asm volatile(
@@ -197,19 +176,6 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, int (&r)[16]) {
       : "r"(taddr)
       : "memory");
 }
-__device__ __forceinline__ void tc_ld32(uint32_t taddr, int (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-}
-__device__ __forceinline__ void tc_ldw(uint32_t taddr, int (&r)[16]) { tc_ld16(taddr, r); }
-__device__ __forceinline__ void tc_ldw(uint32_t taddr, int (&r)[32]) { tc_ld32(taddr, r); }
 __device__ __forceinline__ int tc_ld1(uint32_t taddr) {
   int r;
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(r) : "r"(taddr) : "memory");
@@ -544,8 +510,6 @@ struct MmaParams {
   uint32_t* tau_bits;      // [passes * n_tile] ordered-key form of tau, atomicMax'ed
   const IndexBounds* bounds;
   uint32_t k;              // top-k size (dynamic tightening needs k <= RETIGHTEN_KMAX)
-  long long* trace;        // BBQ_MMA_DEBUG bit 32: clock64 stamps of CTA 0's hand-offs (tools/mma_trace.py)
-  uint32_t debug;          // profiling knobs (BBQ_MMA_DEBUG): 1 = epilogue skips the screen, 2 = hits are ignored, 4 = no TMEM loads, 32 = record the hand-off timeline
   const float4* rscreen;   // [n] per-row screen constants (k_index_bounds)
   const int32_t* qoff;     // [passes * n_tile] per-query offsets of the first-level screen (nullptr in SCAN_DUMP)
   const QEnv* qenv;        // [passes] first-level envelope of each resident query block
@@ -747,10 +711,9 @@ __device__ void mma_drain_ring(const HitCtx* cx, uint64_t* ring, const uint32_t*
 // CH tcgen05.st in flight before the single wait::st); hand-off h belongs to group h % G.  Every group prefetches its
 // own chunks PF deep across tile boundaries, and group 0 asks L2 for each row four tiles ahead (the 16-byte loads
 // themselves come too late to hide an HBM round trip under a busy SM).
-template <int G, int CH, bool DBG>
+template <int G, int CH>
 __device__ __forceinline__ void mma_expansion(const MmaParams& p, uint64_t* a_full, uint64_t* a_empty, uint32_t tmem_base,
                                               uint32_t a_col, int nstage, int nchunks, int warp, int lane) {
-  const uint32_t dbg = DBG ? p.debug : 0u;     // the production instantiation carries none of the attribution knobs
   const int grp = (warp - 4) >> 2;
   const int r = ((warp - 4) & 3) * 32 + lane;  // row within the tile == TMEM lane
   const uint32_t lane_addr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16);
@@ -772,7 +735,7 @@ __device__ __forceinline__ void mma_expansion(const MmaParams& p, uint64_t* a_fu
   };
   auto pf_set_tile = [&]() {
     pf_ptr = reinterpret_cast<const uint4*>(row_ptr(pf_tile));
-    if (grp == 0 && !(dbg & 128u)) {
+    if (grp == 0) {
       const uint8_t* far = row_ptr(pf_tile + L2_AHEAD);
       if (far != nullptr)
         for (int b = 0; b < p.row_bytes; b += 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(far + b));
@@ -820,7 +783,6 @@ __device__ __forceinline__ void mma_expansion(const MmaParams& p, uint64_t* a_fu
     }
   };
   for (int k = 0; k < CH * grp; k++) stage_inc(stage, sphase);
-  int exp_ev = 0;
   for (int pass = 0; pass < p.passes; pass++) {
     uint4 q[PF];
     pf_tile = 0;
@@ -835,47 +797,29 @@ __device__ __forceinline__ void mma_expansion(const MmaParams& p, uint64_t* a_fu
       for (int i = 0; i < PF; i += CH) {
         const int64_t h = h0 + (i / CH) * G;  // this group's hand-off
         if (h < hands) {
-          const bool tr = (dbg & 32u) && blockIdx.x == 0 && warp == 4 && lane == 0 && pass == 0 && exp_ev < 1000;
-          long long x0 = tr ? clock64() : 0;
           uint32_t e[2][32];
           uint32_t sid[CH];
           uint32_t st_ = stage, ph_ = sphase;
           const int nval = (int)min((int64_t)CH, total - CH * h);  // chunks of this hand-off that exist (the stream may end short)
-          long long t_exp = 0, t_wait = 0, t_st = 0;  // (timeline only)
 #pragma unroll
           for (int c = 0; c < CH; c++) {
-            const long long ya = tr ? clock64() : 0;
             expand(q[i + c], e[c & 1]);  // (a zero chunk past the end of the stream: loaded, never stored)
             q[i + c] = load_next();
             sid[c] = st_;
-            const long long yb = tr ? clock64() : 0;
             if (c < nval) {
               mbar_wait_relaxed(a_empty + st_, ph_ ^ 1u);
               tc_fence_after();
-              const long long yc = tr ? clock64() : 0;
               tc_st32(lane_addr + a_col + st_ * 32u, e[c & 1]);
-              if (tr) {
-                t_wait += yc - yb;
-                t_st += clock64() - yc;
-              }
             }
-            if (tr) t_exp += yb - ya;
             stage_inc(st_, ph_);
           }
-          long long x3 = tr ? clock64() : 0;
           tc_wait_st();
-          long long x4 = tr ? clock64() : 0;
           tc_fence_before();
           __syncwarp();
           if (lane == 0) {  // one arrival per expansion warp and stage
 #pragma unroll
             for (int c = 0; c < CH; c++)
               if (c < nval) mbar_arrive(a_full + sid[c]);
-          }
-          if (tr) {
-            long long* d = p.trace + 1 * 4096 + exp_ev * 8;
-            d[0] = x0; d[1] = t_exp; d[2] = t_wait; d[3] = t_st; d[4] = x4 - x3; d[5] = clock64() - x4; d[6] = x3 - x0;
-            exp_ev++;
           }
           for (int k = 0; k < CH * G; k++) stage_inc(stage, sphase);  // on to this group's next hand-off
         }
@@ -902,12 +846,8 @@ __device__ __forceinline__ void mma_expansion(const MmaParams& p, uint64_t* a_fu
 
 // CPQ = accumulator columns per query: 1, or 2 when the query code is split into nibbles (k_query_tiles); then the
 // epilogue works on val = 16 * D_hi + D_lo = 8 * dot and every per-query table is indexed by column / 2.
-// DBG = false is the production instantiation: every BBQ_MMA_DEBUG knob (timeline stamps, attribution switches,
-// first-level statistics) compiles away — the kernel is register- and layout-sensitive enough that merely CARRYING an
-// unused code path moved it by 12 % (profiles/r02_k2_paired_store_experiment.txt).
-template <int MODE, int SIM, int CPQ, int LAYOUT, bool DBG>
+template <int MODE, int SIM, int CPQ, int LAYOUT>
 __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(const __grid_constant__ MmaParams p) {
-  const uint32_t dbg = DBG ? p.debug : 0u;
   constexpr int MMA_EPI_WARPS = MmaLayout<LAYOUT>::EPI_WARPS, MMA_EXP_GROUPS = MmaLayout<LAYOUT>::EXP_GROUPS,
                 MMA_EPI_WARP0 = MmaLayout<LAYOUT>::EPI_WARP0, MMA_THREADS = MmaLayout<LAYOUT>::THREADS;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -920,7 +860,7 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
   float2* qw_s = reinterpret_cast<float2*>(qpb_s + p.n_tile / 2);
   bbqn::QueryTerms* qt_s = reinterpret_cast<bbqn::QueryTerms*>(qw_s + p.n_tile / 2);  // DUMP mode only
   int32_t* qoff_s = reinterpret_cast<int32_t*>(qt_s + p.n_tile);   // [n_tile] this pass's first-level offsets (16 B aligned)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(qoff_s + p.n_tile + 16);  // (+16: a 32-column load may straddle the end)
+  uint64_t* bars = reinterpret_cast<uint64_t*>(qoff_s + p.n_tile + 16);  // (+16: never-passing offsets past the block)
   uint64_t* a_full = bars;            // [8]
   uint64_t* a_empty = bars + 8;       // [8]
   uint64_t* acc_full = bars + 16;     // [2]
@@ -997,7 +937,6 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
   const int NI = max(1, min(p.nissuers, min(nchunks, 3)));
   uint32_t gchunk = 0;  // running chunk count of this CTA: stage = gchunk % nstage, phase = (gchunk / nstage) & 1
   uint32_t tcount_i = 0;
-  int mma_ev = 0;
   auto issue_pass = [&](int pass, int me) {  // whole warp; me = 0 issues the tile's first (overwriting) MMA
     const uint32_t idesc = make_idesc_i8(128, p.n_tile);
     const uint32_t lbo = (uint32_t)p.n_tile * 16u;
@@ -1012,11 +951,8 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
       for (int kc = me; kc < nchunks; kc += NI) {
         const uint32_t g = gchunk + (uint32_t)kc;
         const uint32_t stage = g % (uint32_t)nstage, sphase = (g / (uint32_t)nstage) & 1u;
-        const bool tr = (dbg & 32u) && blockIdx.x == 0 && lane == 0 && pass == 0 && me == 0;
-        long long t0 = tr ? clock64() : 0;
         mbar_wait(a_full + stage, sphase);
         tc_fence_after();
-        long long t1 = tr ? clock64() : 0;
         if (lane == 0) {
 #pragma unroll
           for (int j = 0; j < 4; j++) {
@@ -1026,12 +962,6 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
             if (kc == 0 && j == 0 && NI > 1) tc_commit(tile_go + buf);
           }
           tc_commit(a_empty + stage);  // frees the A stage once these MMAs have read it
-          if (tr && mma_ev < 1000) {
-            p.trace[0 * 4096 + mma_ev * 4 + 0] = t0;
-            p.trace[0 * 4096 + mma_ev * 4 + 1] = t1;
-            p.trace[0 * 4096 + mma_ev * 4 + 2] = clock64();
-            mma_ev++;
-          }
         }
         __syncwarp();
       }
@@ -1072,14 +1002,14 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
     // medium batches, wide rows) it hands over FOUR at a time — the tcgen05.wait::st round trip, not the ALU work,
     // bounds the feed, and four stores in flight amortise it twice as well; two groups alternate pairs of chunks when 8
     // stages exist, single chunks otherwise.
-    if (MMA_EXP_GROUPS == 2 && nstage >= 8 && !(dbg & 1024u))
-      mma_expansion<2, 2, DBG>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
+    if (MMA_EXP_GROUPS == 2 && nstage >= 8)
+      mma_expansion<2, 2>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
     else if (MMA_EXP_GROUPS == 2)
-      mma_expansion<2, 1, DBG>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
-    else if (nstage >= 8 && !(dbg & 512u))
-      mma_expansion<1, 4, DBG>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
+      mma_expansion<2, 1>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
+    else if (nstage >= 8)
+      mma_expansion<1, 4>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
     else
-      mma_expansion<1, 2, DBG>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
+      mma_expansion<1, 2>(p, a_full, a_empty, tmem_base, a_col, nstage, nchunks, warp, lane);
   } else if (warp >= MMA_EPI_WARP0) {
     // ===== epilogue: first-level integer screen on the accumulators, second level + parking for what passes =====
     const int ew = warp - MMA_EPI_WARP0;           // 0 .. MMA_EPI_WARPS-1
@@ -1090,7 +1020,6 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
     const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16);
     const int et = threadIdx.x - MMA_EPI_WARP0 * 32;  // 0 .. MMA_EPI_WARPS*32-1 within the epilogue group
     uint32_t tcount = 0;
-    unsigned long long dbg_tested = 0ull, dbg_passed = 0ull, dbg_warps = 0ull;  // BBQ_MMA_DEBUG bit 256: first-level statistics
     for (int pass = 0; pass < p.passes; pass++) {
       // per-pass query constants -> shared memory (epilogue warps only: named barrier 1)
       asm volatile("bar.sync 1, %0;" ::"n"(MMA_EPI_WARPS * 32) : "memory");
@@ -1155,7 +1084,7 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
           const float Sl = S - H - fmaf(A, 1.9073486328125e-06f, 1.0f);
           T = (Sl > -1.0e9f && Sl < 1.0e9f) ? (int)floorf(Sl) : INT_MIN;  // NaN / out of range: everything passes on
           if (!valid) T = INT_MAX;
-          if (always || MODE != SCAN_FILTER || p.qenv == nullptr || (dbg & 64u)) T = INT_MIN;
+          if (always || MODE != SCAN_FILTER || p.qenv == nullptr) T = INT_MIN;
         }
         const uint64_t rv2 = f2_pack(rv, rv), x1f2 = f2_pack(x1f, x1f), gv2 = f2_pack(gv, gv), iv2 = f2_pack(iv, iv);
         // f64 correctives: issued now, consumed only by the dump
@@ -1182,17 +1111,16 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
         if (refresh2 && p.qoff != nullptr) fo1 = __ldcg(p.qoff + q0q + et + ET);
         // software pipeline over this warp's 16-column chunks: the next chunk's TMEM load is in flight while the
         // current one is reduced; the chunk just read is re-armed for the tile two positions ahead
-        constexpr int W = MMA_LDW;
+        constexpr int W = 16;  // accumulator columns per TMEM load (tcgen05.ld .x16)
         int acc[W], nxt[W];
         int c0 = sub * W;
         if (c0 < nv) {
-          tc_ldw(d_addr + (uint32_t)c0, acc);
+          tc_ld16(d_addr + (uint32_t)c0, acc);
           tc_wait_ld();
         }
-        if (dbg & 4u) c0 = nv;
         auto chunk = [&](int (&cur)[W], int (&nx)[W], int cc) -> bool {
           const int c1 = cc + NSUB * W;
-          if (c1 < nv) tc_ldw(d_addr + (uint32_t)c1, nx);
+          if (c1 < nv) tc_ld16(d_addr + (uint32_t)c1, nx);
           // per QUERY from here on: val = 8 * dot (split codes: 16 * D_hi + D_lo), qc = the chunk's first query slot
           constexpr int NVC = W / CPQ;
           int val[NVC];
@@ -1234,15 +1162,9 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
               }
               const int m = max(max(mm[0], mm[1]), max(mm[2], mm[3]));
               go = m >= T;
-              if (dbg & 256u) {
-                dbg_tested++;
-                dbg_passed += go ? 1ull : 0ull;
-                const bool any_go = __any_sync(0xffffffffu, go);  // (every lane votes: no short-circuit around it)
-                dbg_warps += (lane == 0 && any_go) ? 1ull : 0ull;
-              }
             }
             uint32_t mask = 0u;
-            if (go && !(dbg & 1u)) {
+            if (go) {
 #pragma unroll
               for (int j = 0; j < NVC / 2; j++) {  // two queries per step
                 const int pj = (qc >> 1) + j;
@@ -1270,16 +1192,11 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
             // lower test NaN, and fminf returns the (+inf) window test instead
             if (!valid) mask = 0u;
             mask &= vmask;
-            if (dbg & 2u) mask = 0u;
             auto v_at = [&](int j) { return j < NVC ? val[j < NVC ? j : 0] : 0; };
             if ((mask & 0xFFFFu) != 0u)  // park the hits for the drainer warp
               mma_park_hits(ring_s, ring_ctl_s + 0, ring_ctl_s + 1, mask & 0xFFFFu, (uint32_t)row, q0q + qc, v_at(0), v_at(1),
                             v_at(2), v_at(3), v_at(4), v_at(5), v_at(6), v_at(7), v_at(8), v_at(9), v_at(10), v_at(11),
                             v_at(12), v_at(13), v_at(14), v_at(15));
-            if (NVC == 32 && (mask >> 16) != 0u)
-              mma_park_hits(ring_s, ring_ctl_s + 0, ring_ctl_s + 1, mask >> 16, (uint32_t)row, q0q + qc + 16, v_at(16),
-                            v_at(17), v_at(18), v_at(19), v_at(20), v_at(21), v_at(22), v_at(23), v_at(24), v_at(25),
-                            v_at(26), v_at(27), v_at(28), v_at(29), v_at(30), v_at(31));
           }
           if (c1 >= nv) return false;
           tc_wait_ld();
@@ -1305,11 +1222,6 @@ __global__ void __launch_bounds__(MmaLayout<LAYOUT>::THREADS, 1) k_scan_mma(cons
         mbar_arrive(acc_empty + buf);
         tcount++;
       }
-    }
-    if (dbg & 256u) {
-      atomicAdd(reinterpret_cast<unsigned long long*>(p.trace) + 3 * 4096 + 0, dbg_tested);
-      atomicAdd(reinterpret_cast<unsigned long long*>(p.trace) + 3 * 4096 + 1, dbg_passed);
-      atomicAdd(reinterpret_cast<unsigned long long*>(p.trace) + 3 * 4096 + 2, dbg_warps);
     }
     __syncwarp();
     if (lane == 0) atomicAdd(ring_ctl_s + 2, 1u);  // this epilogue warp will park nothing more

@@ -416,8 +416,6 @@ int bbq_get_stats(bbq_ctx* ctx, bbq_stats* out);
 /* Off by default.  When on, search calls bracket their kernel groups with CUDA events (recorded on the launch
  * stream); bbq_get_stats synchronises them and accumulates.  bbq_reset_profiling zeroes the accumulators. */
 int bbq_set_profiling(bbq_ctx* ctx, int enabled);
-/* Timeline of the tensor-core scan's hand-offs (clock64 stamps of CTA 0; only recorded with BBQ_MMA_DEBUG bit 32). */
-int bbq_debug_trace(bbq_ctx* ctx, long long* out, uint32_t count);
 int bbq_reset_profiling(bbq_ctx* ctx);
 
 #ifdef __cplusplus

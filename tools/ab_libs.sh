@@ -11,8 +11,8 @@ for rep in ${REPS:-1 2}; do for lib in "$@"; do
   fi
   for w in ${WL:-c3 c4}; do
     echo -n "$(basename $lib) $w: "
-    BBQ_MMA_DEBUG=${DEBUG:-0} timeout -s KILL ${TMO:-300} python bench.py --workload $w --datagen device --no-cpu --no-secondary --steps ${STEPS:-5} ${EXTRA:-} 2>/dev/null | tail -1 | \
-      python -c "import sys,json; d=json.loads(sys.stdin.read()); r=d['roofline']; print('QPS', round(d['value']), 'ms/step', round(d['ms_per_step'],3), 'scan launch ms', round(r['avg_scan_launch_ms'],4), 'passes', r.get('passes_over_shard'), 'frac', round(r['frac'],3))"
+    timeout -s KILL ${TMO:-300} python bench.py --workload $w --datagen device --no-cpu --no-secondary --steps ${STEPS:-5} ${EXTRA:-} 2>/dev/null | tail -1 | \
+      python -c "import sys,json; d=json.loads(sys.stdin.read()); r=d['roofline']; print('QPS', round(d['value']), 'ms/step', round(d['ms_per_step'],3), 'e2e ms/step', round(d['e2e']['ms_per_step'],4), 'scan launch ms', round(r['avg_scan_launch_ms'],4), 'passes', r.get('passes_over_shard'), 'frac', round(r['frac'],3))"
   done
 done; done
 cp "$keep" better-binary-quantization_b200/libbbq_b200.so

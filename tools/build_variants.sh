@@ -1,19 +1,14 @@
 #!/usr/bin/env bash
-# Builds variants of libbbq_b200.so for same-box A/B runs (tools/ab_libs.sh): role layouts of the tensor-core scan
-# and, with REF=<commit>, the library as of an earlier commit.  Outputs build/variants/*.so (they travel with gpurun).
+# Builds libbbq_b200.so as of an earlier commit for same-box A/B runs (tools/ab_libs.sh): REF=<commit> tools/build_variants.sh
+# Output: build/variants/ref_<commit>.so (build/ is ignored by git).
 set -e
 cd "$(dirname "$0")/.."
+: "${REF:?set REF=<commit> to build the library as of that commit}"
 mkdir -p build/variants
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo --fmad=false -std=c++17 -Xcompiler -fPIC -shared"
-for v in ${VARIANTS:-e8g1 e4g2 e8g2}; do
-  e=${v:1:1}; g=${v:3:1}; w=${v:5:2}; w=${w:-16}
-  $NVCC $FLAGS -DBBQ_MMA_EPI_WARPS=$e -DBBQ_MMA_EXP_GROUPS=$g -DBBQ_MMA_LDW=$w -o build/variants/$v.so better-binary-quantization_b200/csrc/bbq_api.cu &
-done
-if [ -n "${REF:-}" ]; then
-  rm -rf /tmp/bbq_ref_src && mkdir -p /tmp/bbq_ref_src
-  git archive "$REF" better-binary-quantization_b200/csrc include | tar -x -C /tmp/bbq_ref_src
-  $NVCC $FLAGS -o build/variants/ref_${REF:0:7}.so /tmp/bbq_ref_src/better-binary-quantization_b200/csrc/bbq_api.cu &
-fi
-wait
+src=$(mktemp -d)
+trap 'rm -rf "$src"' EXIT
+git archive "$REF" better-binary-quantization_b200/csrc include | tar -x -C "$src"
+$NVCC $FLAGS -o build/variants/ref_${REF:0:7}.so "$src"/better-binary-quantization_b200/csrc/bbq_api.cu
 ls -la build/variants/
